@@ -30,6 +30,15 @@ struct CudaError : std::runtime_error { using std::runtime_error::runtime_error;
 
 static int env_int(const char* name, int dflt) { const char* v = getenv(name); return v && *v ? atoi(v) : dflt; }
 
+// One call's guide packing and host-side result assembly run under the next call's kernels, and two sweeps never share -- and
+// thrash -- the L2-resident slices; the PAM scan of gsx_enumerate_genome takes the same turn for its chromosome upload.
+// GSX_DEVICE_LOCK=0 turns it off.
+std::unique_lock<std::mutex> gsx::device_turn(int device) {
+    static std::mutex device_mu[64];
+    if (!env_int("GSX_DEVICE_LOCK", 1)) return std::unique_lock<std::mutex>();
+    return std::unique_lock<std::mutex>(device_mu[device & 63]);
+}
+
 extern "C" const char* gsx_last_error(void) { return g_err.c_str(); }
 extern "C" const char* gsx_version(void) { return "2.0.0"; }
 extern "C" void gsx_free(void* p) { free(p); }
@@ -846,11 +855,8 @@ static void run_device_job(DeviceJob* job) {
         auto grow_queue = [&]() { B.free_one(d_queue); d_queue = nullptr; queue_cap *= 4; if (queue_cap >= (1ull << 32)) throw std::runtime_error("seed queue keeps overflowing"); };
 
         // Calls from several host threads (the reference's own worker threads, or gsx_enumerate_start) take turns on a device from the
-        // first search launch to the last result copy: one call's guide packing and host-side result assembly then run under the
-        // next call's kernels, and two sweeps never share -- and thrash -- the L2-resident slices.  GSX_DEVICE_LOCK=0 turns it off.
-        static std::mutex device_mu[64];
-        std::unique_lock<std::mutex> device_turn;
-        if (env_int("GSX_DEVICE_LOCK", 1)) device_turn = std::unique_lock<std::mutex>(device_mu[di.device & 63]);
+        // first search launch to the last result copy (gsx::device_turn).
+        std::unique_lock<std::mutex> turn = gsx::device_turn(di.device);
         CK(cudaEventRecord(ev[0], s));
         // ---- threshold prefilter (process.hpp:66-76): mismatch-only counting search, guide dropped if > 1 site -----
         if (p.threshold > 0) {
@@ -1163,7 +1169,7 @@ static void run_device_job(DeviceJob* job) {
         // the turn on the device ends with the copies: a result transfer running under the NEXT call's sweep slows both several
         // times over (170 MB streaming through the L2 that holds the sweep's slices: profiles/r02b_session_3100mb_sweep_lean.jsonl,
         // m3_lean_v11_pipe2); what overlaps between pipelined calls is the host work -- guide packing before, result assembly after
-        if (device_turn.owns_lock()) device_turn.unlock();
+        if (turn.owns_lock()) turn.unlock();
         float ms;
         CK(cudaEventElapsedTime(&ms, ev[0], ev[1])); job->ctr.ms_search = ms;
         CK(cudaEventElapsedTime(&ms, ev[1], ev[2])); job->ctr.ms_arrange = ms;

@@ -4,6 +4,7 @@
 #include "../../include/gsx.h"
 #include "gsx_host.h"
 #include "gsx_core.h"
+#include "gsx_sites.h"
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -11,6 +12,8 @@
 #include <cstring>
 #include <condition_variable>
 #include <deque>
+#include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -508,15 +511,59 @@ extern "C" int gsx_internal_format_rate(const gsx_index* ix, const gsx_result* r
     return GSX_OK;
 }
 
-// Whole-file driver.  Four things overlap: the GPU enumerates batch k+1 while the host packs the guides of batch k+2 (two-slot
-// gsx_enumerate_start / _wait), a formatter thread turns batch k into text on the host cores, and a writer thread copies the text of
-// batch k-1 into the output file on several threads; batches go out in file order.  The reference's counterpart is N worker threads
-// behind one mutex-guarded ofstream (process.hpp:119-126).
-extern "C" int gsx_enumerate_file(const gsx_index* ix, const char* kmers_csv, const char* out_path, const gsx_params* p,
-                                  int format_sam, int complete, size_t batch_guides, size_t* n_guides, gsx_counters* counters) {
-    if (!ix || !kmers_csv || !out_path || !p) return GSX_ERR_ARG;
-    GuideTable t; std::string err;
-    if (!read_guides_csv(kmers_csv, t, err)) { fprintf(stderr, "gsx: %s\n", err.c_str()); return gsx_set_error(GSX_ERR_IO, err); }
+// ---- whole-file driver -------------------------------------------------------------------------------------------------------
+// The guides come from a batch source: the parsed guides CSV (gsx_enumerate_file) or the PAM sites of a genome (gsx_enumerate_genome).
+// A batch owns what its rows point to that the source does not keep (`arena`); it lives until the formatter has released it.
+namespace {
+struct GuideBatch {
+    std::vector<gsx_guide> g; std::vector<gsx_guide_row> rows;
+    std::string arena;
+};
+struct BatchSource {
+    virtual ~BatchSource() = default;
+    // the next at most `max` guides in output order into b; false when there are none left.  Throws gsx::SiteError.
+    virtual bool next(size_t max, GuideBatch& b) = 0;
+    virtual std::string timing() const { return std::string(); }        // appended to the GSX_FILE_TIMING line
+};
+
+struct TableSource : BatchSource {
+    const GuideTable& t; size_t at = 0;
+    explicit TableSource(const GuideTable& tt) : t(tt) {}
+    bool next(size_t max, GuideBatch& b) override {
+        const size_t b1 = std::min(t.size(), at + max);
+        if (at >= b1) return false;
+        b.g.resize(b1 - at); b.rows.resize(b1 - at);
+        for (size_t i = at; i < b1; i++) { b.g[i - at] = {t.seq[i], t.pam[i]}; b.rows[i - at] = {t.id[i], t.seq[i], t.pam[i], (int)t.positive[i]}; }
+        at = b1;
+        return true;
+    }
+};
+
+// Guides per call: the per-device default (or GSX_FILE_BATCH) times the index's devices, fewer with bulges.  n: the guides of the whole
+// job when they are known in advance (n_known: a CSV), which lets a short job use smaller batches.
+size_t file_batch_guides(const gsx_index* ix, const gsx_params* p, uint32_t qlen, bool n_known, size_t n) {
+    // a batch large enough for the slice-major kernels, small enough that its hits fit the arenas: a guide with bulges has
+    // thousands of edited forms and about ten hits per form
+    const char* e = getenv("GSX_FILE_BATCH");
+    size_t batch_guides = e && *e ? (size_t)atoll(e) : 200000;                                 // per device
+    if (p->rna_bulges || p->dna_bulges) {
+        const uint64_t forms = std::max<uint64_t>(1, bulge_variant_count(std::min<uint32_t>(qlen, 31), p->rna_bulges, p->dna_bulges));
+        batch_guides = (size_t)std::min<uint64_t>(batch_guides, std::max<uint64_t>(64, (4u << 20) / forms));
+    }
+    batch_guides *= (size_t)std::max(1, gsx_index_n_devices(ix));                             // (guides are sharded over the index's devices)
+    // a file of only a few such batches: smaller ones, so that formatting and writing batch k still overlap the search of batch
+    // k+1 (not below 50 k guides per device: the slice-major kernels lose a fifth of their rate there)
+    if (n_known && !(e && *e) && !(p->rna_bulges || p->dna_bulges) && n < 4 * batch_guides)
+        batch_guides = std::max<size_t>((n + 3) / 4, (size_t)50000 * (size_t)std::max(1, gsx_index_n_devices(ix)));
+    return batch_guides ? batch_guides : 1;
+}
+
+// Four things overlap: the GPU enumerates batch k+1 while the host packs the guides of batch k+2 (two-slot gsx_enumerate_start /
+// _wait), a formatter thread turns batch k into text on the host cores, and a writer thread copies the text of batch k-1 into the
+// output file on several threads; batches go out in file order.  The reference's counterpart is N worker threads behind one
+// mutex-guarded ofstream (process.hpp:119-126).
+int run_file_job(const gsx_index* ix, BatchSource& src, const char* out_path, const gsx_params* p, int format_sam, int complete,
+                 size_t batch_guides, size_t* n_guides, gsx_counters* counters) {
     OutFile out;
     if (!out.open(out_path)) { fprintf(stderr, "gsx: cannot write %s\n", out_path); return gsx_set_error(GSX_ERR_IO, std::string("cannot write ") + out_path); }
     {
@@ -526,24 +573,8 @@ extern "C" int gsx_enumerate_file(const gsx_index* ix, const char* kmers_csv, co
         if (!out.append(hdr)) { out.close_file(); return gsx_set_error(GSX_ERR_IO, std::string("cannot write ") + out_path); }
     }
     gsx_params pp = *p; pp.sam_scoring = format_sam ? 1 : 0;
-    const size_t n = t.size();
-    if (batch_guides == 0) {
-        // a batch large enough for the slice-major kernels, small enough that its hits fit the arenas: a guide with bulges has
-        // thousands of edited forms and about ten hits per form
-        const char* e = getenv("GSX_FILE_BATCH");
-        batch_guides = e && *e ? (size_t)atoll(e) : 200000;                                   // per device
-        if (p->rna_bulges || p->dna_bulges) {
-            const uint64_t forms = std::max<uint64_t>(1, bulge_variant_count(n ? (uint32_t)std::min<size_t>(strlen(t.seq[0]), 31) : 20, p->rna_bulges, p->dna_bulges));
-            batch_guides = (size_t)std::min<uint64_t>(batch_guides, std::max<uint64_t>(64, (4u << 20) / forms));
-        }
-        batch_guides *= (size_t)std::max(1, gsx_index_n_devices(ix));                         // (guides are sharded over the index's devices)
-        // a file of only a few such batches: smaller ones, so that formatting and writing batch k still overlap the search of batch
-        // k+1 (not below 50 k guides per device: the slice-major kernels lose a fifth of their rate there)
-        if (!(e && *e) && !(p->rna_bulges || p->dna_bulges) && n < 4 * batch_guides)
-            batch_guides = std::max<size_t>((n + 3) / 4, (size_t)50000 * (size_t)std::max(1, gsx_index_n_devices(ix)));
-        if (batch_guides == 0) batch_guides = 1;
-    }
-    struct Item { gsx_result* r; size_t b0, b1; };
+    size_t n = 0;                                                                              // guides submitted
+    struct Item { gsx_result* r; std::unique_ptr<GuideBatch> b; };
     struct Text { std::vector<std::string> parts; };
     std::mutex mu; std::condition_variable cv;
     std::deque<Item> queue; bool done = false; int wrc = GSX_OK;
@@ -569,16 +600,13 @@ extern "C" int gsx_enumerate_file(const gsx_index* ix, const char* kmers_csv, co
         }
     });
     std::thread formatter([&] {
-        std::vector<gsx_guide_row> rows;
         for (;;) {
             Item it;
-            { std::unique_lock<std::mutex> lk(mu); cv.wait(lk, [&] { return !queue.empty() || done; }); if (queue.empty()) break; it = queue.front(); }
+            { std::unique_lock<std::mutex> lk(mu); cv.wait(lk, [&] { return !queue.empty() || done; }); if (queue.empty()) break; it = std::move(queue.front()); }
             Text tx;
             const auto tf = now();
             if (wrc == GSX_OK) {
-                rows.resize(it.b1 - it.b0);
-                for (size_t i = it.b0; i < it.b1; i++) rows[i - it.b0] = {t.id[i], t.seq[i], t.pam[i], (int)t.positive[i]};
-                format_rows_parts(ix, it.r, rows.data(), 0, rows.size(), &pp, format_sam, complete, tx.parts);
+                format_rows_parts(ix, it.r, it.b->rows.data(), 0, it.b->rows.size(), &pp, format_sam, complete, tx.parts);
                 gsx_counters c; gsx_result_counters(it.r, &c);
                 total.nodes += c.nodes; total.lookups += c.lookups; total.matches += c.matches; total.hits += c.hits; total.lf_steps += c.lf_steps; total.spills += c.spills; total.launches += c.launches;
                 total.ms_search += c.ms_search; total.ms_arrange += c.ms_arrange; total.ms_locate += c.ms_locate; total.ms_score += c.ms_score;
@@ -587,6 +615,7 @@ extern "C" int gsx_enumerate_file(const gsx_index* ix, const char* kmers_csv, co
             s_format += since(tf);
             const auto tr = now();
             gsx_result_free(it.r);
+            it.b.reset();
             s_free += since(tr);
             {
                 std::unique_lock<std::mutex> lk(mu);
@@ -607,8 +636,9 @@ extern "C" int gsx_enumerate_file(const gsx_index* ix, const char* kmers_csv, co
     // format_csv_guide: 22, 12 in succinct mode)
     const uint32_t want = format_sam ? (kWantDistance | kWantCounted | kWantAbsPos | kWantChr | kWantPos1)
                                      : (kWantDistance | kWantCounted | kWantChr | kWantPos1 | kWantStrand | (complete ? kWantBulges | kWantMatchString : 0u));
-    // two batches in flight: the guides of batch k+1 are packed (and its small uploads issued) while batch k runs on the device
-    struct Slot { std::vector<gsx_guide> g; gsx_pending* pd = nullptr; size_t b0 = 0, b1 = 0; };
+    // two batches in flight: the guides of batch k+1 are taken from the source (and its small uploads issued) while batch k runs on the
+    // device
+    struct Slot { std::unique_ptr<GuideBatch> b; gsx_pending* pd = nullptr; };
     Slot slots[2]; int n_pending = 0, head = 0;
     auto finish_one = [&]() {
         Slot& sl = slots[head]; head ^= 1; n_pending--;
@@ -616,24 +646,27 @@ extern "C" int gsx_enumerate_file(const gsx_index* ix, const char* kmers_csv, co
         const auto tc = now();
         const int rc1 = gsx_enumerate_wait(sl.pd, &r); sl.pd = nullptr;
         s_wait_call += since(tc);
-        if (rc1) { if (rc == GSX_OK) { rc = rc1; rc_msg = gsx_last_error(); } return; }
-        if (rc != GSX_OK) { gsx_result_free(r); return; }
+        if (rc1) { if (rc == GSX_OK) { rc = rc1; rc_msg = gsx_last_error(); } sl.b.reset(); return; }
+        if (rc != GSX_OK) { gsx_result_free(r); sl.b.reset(); return; }
         std::unique_lock<std::mutex> lk(mu);
         const auto tq = now();
         cv.wait(lk, [&] { return queue.size() < 2; });
         s_wait_queue += since(tq);
-        queue.push_back({r, sl.b0, sl.b1});
+        queue.push_back({r, std::move(sl.b)});
         lk.unlock(); cv.notify_all();
     };
-    for (size_t b0 = 0; b0 < n && rc == GSX_OK; b0 += batch_guides) {
+    while (rc == GSX_OK) {
         if (n_pending == 2) finish_one();
         if (rc != GSX_OK) break;
         Slot& sl = slots[(head + n_pending) & 1];
-        sl.b0 = b0; sl.b1 = std::min(n, b0 + batch_guides);
-        sl.g.resize(sl.b1 - sl.b0);
-        for (size_t i = sl.b0; i < sl.b1; i++) sl.g[i - sl.b0] = {t.seq[i], t.pam[i]};
-        const int rc1 = gsx_internal_enumerate_start_want(ix, sl.g.data(), sl.g.size(), &pp, want, &sl.pd);
-        if (rc1) { rc = rc1; rc_msg = gsx_last_error(); break; }
+        sl.b.reset(new GuideBatch());
+        try {
+            if (!src.next(batch_guides, *sl.b)) { sl.b.reset(); break; }
+        } catch (const gsx::SiteError& f) { rc = f.code; rc_msg = f.msg; sl.b.reset(); break; }
+        catch (const std::bad_alloc&) { rc = GSX_ERR_NOMEM; rc_msg = "out of host memory"; sl.b.reset(); break; }
+        n += sl.b->g.size();
+        const int rc1 = gsx_internal_enumerate_start_want(ix, sl.b->g.data(), sl.b->g.size(), &pp, want, &sl.pd);
+        if (rc1) { rc = rc1; rc_msg = gsx_last_error(); sl.b.reset(); break; }
         n_pending++;
     }
     while (n_pending) finish_one();
@@ -642,13 +675,177 @@ extern "C" int gsx_enumerate_file(const gsx_index* ix, const char* kmers_csv, co
     formatter.join(); writer.join();
     if (timing)
         fprintf(stderr, "gsx file job: %.3f s wall, %zu guides in batches of %zu; formatter busy %.3f s (+ %.3f s releasing results, %.3f s waiting for the writer), "
-                "writer busy %.3f s; submitter waited %.3f s for calls and %.3f s for the formatter; calls: device %.3f s, d2h %.3f s, h2d %.3f s, prepare %.3f s, call walls %.3f s\n",
+                "writer busy %.3f s; submitter waited %.3f s for calls and %.3f s for the formatter; calls: device %.3f s, d2h %.3f s, h2d %.3f s, prepare %.3f s, call walls %.3f s%s\n",
                 since(t_job), n, batch_guides, s_format, s_free, s_fwait_writer, s_write, s_wait_call, s_wait_queue, total.ms_total_device / 1e3, total.ms_d2h / 1e3,
-                total.ms_h2d / 1e3, total.ms_prepare / 1e3, total.ms_wall / 1e3);
+                total.ms_h2d / 1e3, total.ms_prepare / 1e3, total.ms_wall / 1e3, src.timing().c_str());
     if (!out.close_file() && wrc == GSX_OK) wrc = GSX_ERR_IO;
     if (rc) return gsx_set_error(rc, rc_msg);
     if (wrc) return gsx_set_error(wrc, std::string("cannot write ") + out_path);
     if (n_guides) *n_guides = n;
     if (counters) *counters = total;
     return GSX_OK;
+}
+}  // namespace
+
+extern "C" int gsx_enumerate_file(const gsx_index* ix, const char* kmers_csv, const char* out_path, const gsx_params* p,
+                                  int format_sam, int complete, size_t batch_guides, size_t* n_guides, gsx_counters* counters) {
+    if (!ix || !kmers_csv || !out_path || !p) return GSX_ERR_ARG;
+    GuideTable t; std::string err;
+    if (!read_guides_csv(kmers_csv, t, err)) { fprintf(stderr, "gsx: %s\n", err.c_str()); return gsx_set_error(GSX_ERR_IO, err); }
+    if (batch_guides == 0) batch_guides = file_batch_guides(ix, p, t.size() ? (uint32_t)std::min<size_t>(strlen(t.seq[0]), 31) : 20, true, t.size());
+    TableSource src(t);
+    return run_file_job(ix, src, out_path, p, format_sam, complete, batch_guides, n_guides, counters);
+}
+
+// ---- genome in, guides enumerated: gsx_generate_kmers -> (BED selection) -> gsx_enumerate_file without the CSV in between --------
+namespace {
+// The sites of one chromosome at a time from the producer (gsx_sites.h), turned into rows by the generator's own row logic; a
+// batch may span chromosomes, so its strings are copied into the batch's arena.
+struct GenomeSource : BatchSource {
+    gsx::FastaReader rd; gsx::SiteScanner S;
+    const std::string pam, prefix; const uint64_t min_len;
+    const std::map<std::string, std::vector<std::pair<uint64_t, uint64_t>>>* regions;      // null: every site
+    std::string name, seq; std::vector<gsx::StartRange> ranges;
+    size_t list = 0, at = 0; bool have_chr = false;
+    GenomeSource(FILE* in, const std::string& pam_, uint32_t k, bool start, int device, const std::string& prefix_, uint64_t min_len_,
+                 const std::map<std::string, std::vector<std::pair<uint64_t, uint64_t>>>* regions_)
+        : rd(in), S(pam_, k, start, device), pam(pam_), prefix(prefix_), min_len(min_len_), regions(regions_) {}
+    bool load() {                                                                              // the next chromosome with sites to offer
+        for (;;) {
+            if (!rd.next(name, &seq, nullptr)) return false;
+            if (seq.size() < min_len || seq.empty()) continue;
+            if (regions) {
+                const auto it = regions->find(name);
+                ranges = it == regions->end() ? std::vector<gsx::StartRange>() : gsx::merge_regions(it->second, S.k());
+                if (ranges.empty()) continue;
+            }
+            S.scan(seq, regions ? &ranges : nullptr);
+            list = 0; at = 0; have_chr = true;
+            return true;
+        }
+    }
+    bool next(size_t max, GuideBatch& b) override {
+        std::vector<size_t> off; std::vector<uint8_t> fwd;                                     // id at off[i], k-mer behind it
+        while (off.size() < max) {
+            if (!have_chr || list == S.n_lists()) { have_chr = false; seq.clear(); if (!load()) break; continue; }
+            const std::vector<uint32_t>& v = S.sites(list);
+            if (at == v.size()) { list++; at = 0; continue; }
+            const bool f = S.forward(list);
+            const size_t m = std::min(v.size() - at, max - off.size());
+            for (size_t q = at; q < at + m; q++) {
+                char num[16]; const int nl = (int)(put_u64_at(num, S.pos1(list, v[q])) - num);
+                off.push_back(b.arena.size()); fwd.push_back(f);
+                gsx::append_site_id(b.arena, prefix, name, num, nl, f); b.arena += '\0';
+                gsx::append_site_kmer(b.arena, seq, S.kmer_start(list, v[q]), S.k(), f); b.arena += '\0';
+            }
+            at += m;
+        }
+        if (off.empty()) return false;
+        b.g.resize(off.size()); b.rows.resize(off.size());
+        for (size_t i = 0; i < off.size(); i++) {
+            const char* id = b.arena.data() + off[i]; const char* kmer = id + strlen(id) + 1;
+            b.g[i] = {kmer, pam.c_str()}; b.rows[i] = {id, kmer, pam.c_str(), (int)fwd[i]};
+        }
+        return true;
+    }
+    std::string timing() const override {
+        char t[160]; snprintf(t, sizeof t, "; PAM scan %.3f s over %zu chromosome(s) (+ %.3f s waiting for the device)", S.seconds, S.chromosomes, S.wait_seconds);
+        return t;
+    }
+};
+
+// BED intervals (0-based, half-open) per chromosome, checked against the index's chromosome table
+bool read_bed(const char* path, const std::map<std::string, uint64_t>& chr_len, std::map<std::string, std::vector<std::pair<uint64_t, uint64_t>>>& out,
+              int& code, std::string& err) {
+    FILE* f = fopen(path, "rb");
+    if (!f) { code = GSX_ERR_IO; err = std::string("cannot open regions file ") + path; return false; }
+    std::string line; char chunk[1 << 16]; size_t lineno = 0; bool ok = true;
+    auto parse_u64 = [](const std::string& s, uint64_t& v) {
+        if (s.empty() || s.size() > 19) return false;
+        v = 0; for (char c : s) { if (c < '0' || c > '9') return false; v = v * 10 + (uint64_t)(c - '0'); }
+        return true;
+    };
+    auto handle = [&](std::string l) {
+        lineno++;
+        while (!l.empty() && (l.back() == '\n' || l.back() == '\r')) l.pop_back();
+        std::vector<std::string> w;
+        for (size_t b = 0; b < l.size();) {
+            while (b < l.size() && (l[b] == ' ' || l[b] == '\t')) b++;
+            size_t e = b; while (e < l.size() && l[e] != ' ' && l[e] != '\t') e++;
+            if (e > b) w.push_back(l.substr(b, e - b));
+            b = e;
+        }
+        if (w.empty() || l[0] == '#' || l.compare(0, 5, "track") == 0 || l.compare(0, 7, "browser") == 0) return true;
+        code = GSX_ERR_ARG;
+        const std::string where = std::string("regions file ") + path + " line " + std::to_string(lineno);
+        uint64_t s = 0, e = 0;
+        if (w.size() < 3 || !parse_u64(w[1], s) || !parse_u64(w[2], e)) { err = where + ": expected \"chrom start end\""; return false; }
+        const auto it = chr_len.find(w[0]);
+        if (it == chr_len.end()) { err = where + ": chromosome \"" + w[0] + "\" is not in the index"; return false; }
+        if (s > e) { err = where + ": start " + w[1] + " is past end " + w[2]; return false; }
+        if (e > it->second) { err = where + ": end " + w[2] + " is past the end of " + w[0] + " (" + std::to_string(it->second) + " bases)"; return false; }
+        out[w[0]].emplace_back(s, e);
+        return true;
+    };
+    while (ok && fgets(chunk, sizeof chunk, f)) {
+        line += chunk;
+        if (line.back() == '\n') { ok = handle(line); line.clear(); }
+    }
+    if (ok && !line.empty()) ok = handle(line);
+    fclose(f);
+    return ok;
+}
+}  // namespace
+
+extern "C" int gsx_enumerate_genome(const gsx_index* ix, const char* fasta_path, const char* pam_c, uint32_t k, uint64_t min_chr_length,
+                                    const char* prefix_c, const char* regions_bed, const char* out_path, const gsx_params* p,
+                                    int format_sam, int complete, size_t batch_guides, size_t* n_guides, gsx_counters* counters) {
+    if (!ix || !fasta_path || !pam_c || !out_path || !p) return gsx_set_error(GSX_ERR_ARG, "null argument");
+    if (n_guides) *n_guides = 0;
+    // everything is checked before the first device work: options, then the FASTA against the index, then the regions
+    const std::string pam(pam_c), prefix(prefix_c ? prefix_c : "");
+    if (k < 1 || k > 32) return gsx_set_error(GSX_ERR_ARG, "kmer_length " + std::to_string(k) + " is outside 1..32");
+    if (pam.empty() || pam.size() > 8) return gsx_set_error(GSX_ERR_ARG, "PAM \"" + pam + "\" must have 1..8 characters");
+    for (char c : pam)
+        if (!(c == 'A' || c == 'C' || c == 'G' || c == 'T' || c == 'N'))
+            return gsx_set_error(GSX_ERR_ARG, "PAM \"" + pam + "\" has the character '" + std::string(1, c) + "': PAM characters must be A, C, G, T or N");
+    std::string longest = pam;
+    for (uint32_t i = 0; i < p->n_alt_pams; i++) if (p->alt_pams && p->alt_pams[i] && strlen(p->alt_pams[i]) > longest.size()) longest = p->alt_pams[i];
+    if (k + longest.size() + p->dna_bulges > 32)
+        return gsx_set_error(GSX_ERR_ARG, "k-mer length " + std::to_string(k) + " + PAM \"" + longest + "\" + " + std::to_string(p->dna_bulges) +
+                                              " DNA bulge(s) is longer than 32 characters");
+    if (ix->dev.empty()) return gsx_set_error(GSX_ERR_NO_DEVICE, "index is not resident on any device");
+    std::map<std::string, uint64_t> chr_len;
+    for (size_t i = 0; i < ix->host.chr_names.size(); i++) chr_len[ix->host.chr_names[i]] = ix->host.chr_lens[i];
+    FILE* in = fopen(fasta_path, "rb");
+    if (!in) return gsx_set_error(GSX_ERR_IO, std::string("cannot open ") + fasta_path);
+    {
+        gsx::FastaReader rd(in);
+        std::string name; uint64_t len = 0;
+        while (rd.next(name, nullptr, &len)) {
+            if (len < min_chr_length || len == 0) continue;
+            const auto it = chr_len.find(name);
+            if (it == chr_len.end()) { fclose(in); return gsx_set_error(GSX_ERR_ARG, "FASTA record \"" + name + "\" (" + std::to_string(len) + " bases) is not a chromosome of the index"); }
+            if (it->second != len) {
+                fclose(in);
+                return gsx_set_error(GSX_ERR_ARG, "FASTA record \"" + name + "\" has " + std::to_string(len) + " bases, the index's chromosome of that name " +
+                                                      std::to_string(it->second) + ": index and FASTA are of different assemblies");
+            }
+        }
+        rewind(in);
+    }
+    std::map<std::string, std::vector<std::pair<uint64_t, uint64_t>>> regions;
+    if (regions_bed) {
+        int code = GSX_OK; std::string err;
+        if (!read_bed(regions_bed, chr_len, regions, code, err)) { fclose(in); return gsx_set_error(code, err); }
+    }
+    if (batch_guides == 0) batch_guides = file_batch_guides(ix, p, k, false, 0);
+    int rc;
+    try {
+        GenomeSource src(in, pam, k, p->start != 0, ix->dev[0].device, prefix, min_chr_length, regions_bed ? &regions : nullptr);
+        rc = run_file_job(ix, src, out_path, p, format_sam, complete, batch_guides, n_guides, counters);
+    } catch (const gsx::SiteError& f) { rc = gsx_set_error(f.code, f.msg); }
+    catch (const std::bad_alloc&) { rc = gsx_set_error(GSX_ERR_NOMEM, "out of host memory"); }
+    fclose(in);
+    return rc;
 }

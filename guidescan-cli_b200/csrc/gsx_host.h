@@ -71,6 +71,10 @@ struct DeviceIndex {
     uint64_t bytes = 0;
 };
 
+// a device's turn (gsx_api.cpp): held by a call from its first search launch to its last result copy, and by the PAM scan of the
+// genome driver (gsx_sites.h) from its chromosome upload to its last site list; an empty lock when GSX_DEVICE_LOCK=0
+std::unique_lock<std::mutex> device_turn(int device);
+
 // GPU suffix sorting (gsx_build.cu): text (bytes, no sentinel) -> HostStrand with samples every 2^sa_shift rows
 bool build_strand_gpu(int device, const uint8_t* text, uint64_t len, uint32_t sa_shift, HostStrand& out, std::string& err);
 

@@ -62,7 +62,7 @@ EXPORTS = ["gsx_params_default", "gsx_index_open", "gsx_index_build", "gsx_index
            "gsx_index_n_chromosomes", "gsx_index_chromosome_name", "gsx_index_chromosome_length", "gsx_index_device_bytes",
            "gsx_index_n_devices", "gsx_index_save_reference_format", "gsx_index_open_seconds", "gsx_index_device_checksum", "gsx_enumerate_start", "gsx_enumerate_wait", "gsx_index_rank", "gsx_index_locate", "gsx_index_export_bwt", "gsx_index_export_sa_samples", "gsx_enumerate", "gsx_result_view_get",
            "gsx_result_counters", "gsx_result_match_sequence", "gsx_result_free", "gsx_format_rows", "gsx_format_header",
-           "gsx_enumerate_file", "gsx_guides_csv_open", "gsx_guides_csv_row", "gsx_guides_csv_close", "gsx_generate_kmers", "gsx_free", "gsx_last_error", "gsx_version", "gsx_device_count"]
+           "gsx_enumerate_file", "gsx_guides_csv_open", "gsx_guides_csv_row", "gsx_guides_csv_close", "gsx_generate_kmers", "gsx_enumerate_genome", "gsx_free", "gsx_last_error", "gsx_version", "gsx_device_count"]
 
 _L.gsx_last_error.restype = C.c_char_p
 _L.gsx_version.restype = C.c_char_p
@@ -108,6 +108,8 @@ _L.gsx_guides_csv_close.argtypes = [C.c_void_p]
 _L.gsx_guides_csv_close.restype = None
 _L.gsx_generate_kmers.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, C.c_uint32, C.c_uint64, C.c_char_p, C.c_int, C.c_int,
                                   C.POINTER(C.c_uint64)]
+_L.gsx_enumerate_genome.argtypes = [C.c_void_p, C.c_char_p, C.c_char_p, C.c_uint32, C.c_uint64, C.c_char_p, C.c_char_p, C.c_char_p,
+                                    C.POINTER(Params), C.c_int, C.c_int, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(Counters)]
 
 
 class GsxError(RuntimeError):
@@ -354,6 +356,16 @@ class Index:
         n, c = C.c_size_t(), Counters()
         _ck(_L.gsx_enumerate_file(self.h, kmers_csv.encode(), out_path.encode(), C.byref(params), int(fmt == "sam"),
                                   int(mode == "complete"), batch_guides, C.byref(n), C.byref(c)), "gsx_enumerate_file")
+        return n.value, c.as_dict()
+
+    def enumerate_genome(self, fasta: str, out_path: str, params, pam="NGG", kmer_length=20, min_chr_length=0, prefix="",
+                         regions=None, fmt="csv", mode="complete", batch_guides=0):
+        """generate_kmers(fasta, ..., start=params.start) -> rows inside the BED file `regions` (None: all) -> enumerate_file, in
+        one pass without the guides CSV.  Returns (guides, counters)."""
+        n, c = C.c_size_t(), Counters()
+        _ck(_L.gsx_enumerate_genome(self.h, fasta.encode(), pam.encode(), kmer_length, min_chr_length, prefix.encode(),
+                                    regions.encode() if regions else None, out_path.encode(), C.byref(params), int(fmt == "sam"),
+                                    int(mode == "complete"), batch_guides, C.byref(n), C.byref(c)), "gsx_enumerate_genome")
         return n.value, c.as_dict()
 
 

@@ -3,6 +3,7 @@
 // Text formatting, file I/O and option parsing are host C++; all arithmetic of the hot path runs on the device.
 #include "../../include/gsx.h"
 #include <algorithm>
+#include <cerrno>
 #include <chrono>
 #include <fcntl.h>
 #include <sys/stat.h>
@@ -32,12 +33,76 @@ static void usage() {
             "      --format TEXT:{csv,sam}     File format for output.\n"
             "      --mode TEXT:{succinct,complete}  Information to output.\n"
             "      -f,--kmers-file FILE        REQUIRED  File containing kmers to build gRNA database over\n"
+            "                                  (unless --genome is given; the two are mutually exclusive)\n"
             "      -o,--output TEXT            REQUIRED  Output file.\n"
             "      --gpus INT=1                Number of GPUs to shard the guides over (extension): devices 0 .. INT-1.\n"
-            "      --devices LIST              The same with explicit device ordinals, e.g. 0,2,3 (extension).\n");
+            "      --devices LIST              The same with explicit device ordinals, e.g. 0,2,3 (extension).\n"
+            "      --genome GENOME.fa          Generate the guides from this FASTA (as `kmers` does, PAM position from --start) and\n"
+            "                                  enumerate them in one pass, without a kmers file (extension).  With --genome:\n"
+            "        --pam TEXT=NGG            PAM pattern (A, C, G, T, N).\n"
+            "        --kmer-length UINT=20     Guide length, 1..32 (with the PAM and DNA bulges at most 32).\n"
+            "        --min-chr-length UINT=0   Skip FASTA records shorter than this.\n"
+            "        --prefix TEXT             Prefix of every guide id.\n"
+            "        --regions BED             Keep only guides whose k bases lie inside one BED interval (0-based, half-open).\n"
+            "  kmers [OPTIONS] GENOME.fa\n"
+            "      Writes the kmers file `enumerate -f` reads: every k-mer next to a PAM on either strand (the original's\n"
+            "      scripts/generate_kmers.py; the PAM scan runs on the GPU).\n"
+            "      -o,--output FILE            REQUIRED  Output CSV.\n"
+            "      --pam TEXT=NGG              PAM pattern (A, C, G, T, N).\n"
+            "      --kmer-length UINT=20       Length of the k-mers.\n"
+            "      --min-chr-length UINT=0     Skip FASTA records shorter than this.\n"
+            "      --prefix TEXT               Prefix of every k-mer id.\n"
+            "      --start                     The PAM precedes the k-mer.\n"
+            "      --device INT=0              GPU that runs the scan.\n");
 }
 
 static std::string lower(std::string s) { std::transform(s.begin(), s.end(), s.begin(), ::tolower); return s; }
+
+// a non-negative decimal option value; anything else ends the program with the CLI's usage status
+static unsigned long long uint_arg(const char* name, const char* v) {
+    char* end = nullptr;
+    errno = 0;
+    const unsigned long long x = strtoull(v, &end, 10);
+    if (!*v || *end || errno || v[0] == '-') { fprintf(stderr, "%s: %s is not a non-negative integer\n", name, v); exit(105); }
+    return x;
+}
+
+// PAM characters of the generator (scripts/generate_kmers.py expands N only)
+static bool pam_ok(const std::string& pam) {
+    if (pam.empty() || pam.size() > 8) return false;
+    for (char c : pam) if (!(c == 'A' || c == 'C' || c == 'G' || c == 'T' || c == 'N')) return false;
+    return true;
+}
+
+static int do_kmers(int argc, char** argv) {
+    std::string fasta, output, pam = "NGG", prefix;
+    unsigned long long k = 20, min_len = 0, device = 0; bool start = false;
+    for (int i = 0; i < argc; i++) {
+        std::string a = argv[i];
+        auto need = [&](const char* name) -> const char* { if (i + 1 >= argc) { fprintf(stderr, "%s: 1 required\n", name); exit(106); } return argv[++i]; };
+        if (a == "-o" || a == "--output") output = need("--output");
+        else if (a == "--pam") pam = need("--pam");
+        else if (a == "--kmer-length") k = uint_arg("--kmer-length", need("--kmer-length"));
+        else if (a == "--min-chr-length") min_len = uint_arg("--min-chr-length", need("--min-chr-length"));
+        else if (a == "--prefix") prefix = need("--prefix");
+        else if (a == "--start") start = true;
+        else if (a == "--device") device = uint_arg("--device", need("--device"));
+        else if (a == "-h" || a == "--help") { usage(); return 0; }
+        else if (!a.empty() && a[0] == '-') { fprintf(stderr, "The following argument was not expected: %s\n", a.c_str()); return 109; }
+        else fasta = a;
+    }
+    if (fasta.empty()) { fprintf(stderr, "genome is required\n"); return 106; }
+    if (output.empty()) { fprintf(stderr, "--output is required\n"); return 106; }
+    if (k < 1 || k > 64) { fprintf(stderr, "--kmer-length: %llu not in 1..64\n", k); return 105; }
+    if (!pam_ok(pam)) { fprintf(stderr, "--pam: %s must be 1..8 characters of A, C, G, T, N\n", pam.c_str()); return 105; }
+    uint64_t n = 0;
+    const auto t0 = std::chrono::steady_clock::now();
+    if (gsx_generate_kmers(fasta.c_str(), output.c_str(), pam.c_str(), (uint32_t)k, min_len, prefix.c_str(), start, (int)device, &n)) {
+        fprintf(stderr, "ERROR: %s\n", gsx_last_error()); return 1;
+    }
+    printf("Wrote %llu kmer(s) to %s in %.3f s.\n", (unsigned long long)n, output.c_str(), std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count());
+    return 0;
+}
 
 static int do_index(int argc, char** argv) {
     std::string fasta, prefix; bool reference_format = false;
@@ -68,6 +133,8 @@ static int do_enumerate(int argc, char** argv) {
     gsx_params p; gsx_params_default(&p);
     std::string index, kmers, output, format = "csv", mode = "complete";
     std::vector<std::string> alts; int gpus = 1; std::vector<int> devs;
+    // --genome: the generator's options (`kmers`) and the regions; `generator` lists those given, which -f does not take
+    std::string genome, pam = "NGG", prefix, regions; unsigned long long k = 20, min_len = 0; std::vector<std::string> generator;
     for (int i = 0; i < argc; i++) {
         std::string a = argv[i];
         auto need = [&](const char* name) -> const char* { if (i + 1 >= argc) { fprintf(stderr, "%s: 1 required\n", name); exit(106); } return argv[++i]; };
@@ -85,6 +152,12 @@ static int do_enumerate(int argc, char** argv) {
         else if (a == "--mode") mode = lower(need("--mode"));
         else if (a == "-f" || a == "--kmers-file") kmers = need("--kmers-file");
         else if (a == "-o" || a == "--output") output = need("--output");
+        else if (a == "--genome") genome = need("--genome");
+        else if (a == "--pam") { pam = need("--pam"); generator.push_back(a); }
+        else if (a == "--kmer-length") { k = uint_arg("--kmer-length", need("--kmer-length")); generator.push_back(a); }
+        else if (a == "--min-chr-length") { min_len = uint_arg("--min-chr-length", need("--min-chr-length")); generator.push_back(a); }
+        else if (a == "--prefix") { prefix = need("--prefix"); generator.push_back(a); }
+        else if (a == "--regions") { regions = need("--regions"); generator.push_back(a); }
         else if (a == "--gpus") gpus = atoi(need("--gpus"));
         else if (a == "--devices") {
             std::string l = need("--devices");
@@ -95,10 +168,18 @@ static int do_enumerate(int argc, char** argv) {
         else index = a;
     }
     if (index.empty()) { fprintf(stderr, "index is required\n"); return 106; }
-    if (kmers.empty()) { fprintf(stderr, "--kmers-file is required\n"); return 106; }
+    if (!kmers.empty() && !genome.empty()) { fprintf(stderr, "--kmers-file excludes --genome: give one of them\n"); return 109; }
+    if (kmers.empty() && genome.empty()) { fprintf(stderr, "--kmers-file is required\n"); return 106; }
+    if (genome.empty() && !generator.empty()) { fprintf(stderr, "%s needs --genome\n", generator[0].c_str()); return 109; }
     if (output.empty()) { fprintf(stderr, "--output is required\n"); return 106; }
     if (format != "csv" && format != "sam") { fprintf(stderr, "--format: %s not in {csv,sam}\n", format.c_str()); return 105; }
     if (mode != "succinct" && mode != "complete") { fprintf(stderr, "--mode: %s not in {succinct,complete}\n", mode.c_str()); return 105; }
+    if (!genome.empty()) {                                    // (the library checks these too; here they fail before the index is opened)
+        if (k < 1 || k > 32) { fprintf(stderr, "--kmer-length: %llu not in 1..32\n", k); return 105; }
+        if (!pam_ok(pam)) { fprintf(stderr, "--pam: %s must be 1..8 characters of A, C, G, T, N\n", pam.c_str()); return 105; }
+        size_t longest = pam.size(); for (auto& x : alts) longest = std::max(longest, x.size());
+        if (k + longest + p.dna_bulges > 32) { fprintf(stderr, "--kmer-length %llu + PAM %zu + --dna-bulges %u is longer than 32\n", k, longest, p.dna_bulges); return 105; }
+    }
     std::vector<const char*> ap; for (auto& s : alts) ap.push_back(s.c_str());
     p.alt_pams = ap.data(); p.n_alt_pams = (uint32_t)ap.size();
     if (devs.empty()) for (int d = 0; d < std::max(1, gpus); d++) devs.push_back(d);
@@ -112,7 +193,9 @@ static int do_enumerate(int argc, char** argv) {
     }
     auto t0 = std::chrono::steady_clock::now();
     size_t n = 0; gsx_counters c;
-    rc = gsx_enumerate_file(ix, kmers.c_str(), output.c_str(), &p, format == "sam", mode == "complete", 0, &n, &c);
+    if (genome.empty()) rc = gsx_enumerate_file(ix, kmers.c_str(), output.c_str(), &p, format == "sam", mode == "complete", 0, &n, &c);
+    else rc = gsx_enumerate_genome(ix, genome.c_str(), pam.c_str(), (uint32_t)k, min_len, prefix.c_str(), regions.empty() ? nullptr : regions.c_str(),
+                                   output.c_str(), &p, format == "sam", mode == "complete", 0, &n, &c);
     if (rc) { fprintf(stderr, "%s\n", gsx_last_error()); gsx_index_close(ix); return 1; }
     double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     printf("Read in %zu kmer(s).\n", n);
@@ -129,6 +212,7 @@ int main(int argc, char** argv) {
     if (cmd == "-h" || cmd == "--help") { usage(); return 0; }
     if (cmd == "index") return do_index(argc - 2, argv + 2);
     if (cmd == "enumerate") return do_enumerate(argc - 2, argv + 2);
+    if (cmd == "kmers") return do_kmers(argc - 2, argv + 2);
     if (cmd == "download") { fprintf(stderr, "download: not part of the GPU hot path (no network); use the reference binary\n"); return 1; }
     usage();
     return 106;

@@ -206,6 +206,17 @@ void gsx_guides_csv_close(gsx_guide_table*);
  * scan and the ordered compaction run on `device`; text identical to the script's.  *n_kmers (may be NULL) = rows written. */
 int gsx_generate_kmers(const char* fasta_path, const char* out_csv_path, const char* pam, uint32_t kmer_length,
                        uint64_t min_chr_length, const char* prefix, int start, int device, uint64_t* n_kmers);
+/* Generation and enumeration in one pass, without the guides CSV: writes byte for byte what gsx_generate_kmers(fasta_path, csv,
+ * pam, kmer_length, min_chr_length, prefix, params->start) followed by gsx_enumerate_file(csv, out_path, ...) writes, for any
+ * batch size and device list.  regions_bed != NULL keeps only the generated rows whose k bases lie inside one interval of the BED
+ * file (0-based, half-open `chrom start end`; further columns, blank lines and `#` / `track` / `browser` lines are ignored); rows
+ * keep the generator's order.  The index must be built from the same assembly: every FASTA record of at least min_chr_length
+ * bases must be a chromosome of the index with the same length.  Options, FASTA and BED are checked before any device work
+ * (GSX_ERR_ARG names the offending item).  The PAM scan runs on the index's first device, one chromosome at a time, taking that
+ * device's turn like a call; host memory holds one chromosome, its sites and the batches in flight.  *n_guides = guides enumerated. */
+int gsx_enumerate_genome(const gsx_index*, const char* fasta_path, const char* pam, uint32_t kmer_length, uint64_t min_chr_length,
+                         const char* prefix, const char* regions_bed, const char* out_path, const gsx_params*, int format_sam,
+                         int complete, size_t batch_guides, size_t* n_guides, gsx_counters* counters);
 
 void gsx_free(void*);
 
