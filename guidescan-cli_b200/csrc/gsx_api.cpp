@@ -790,9 +790,74 @@ static void run_device_job(DeviceJob* job) {
         uint64_t n_launches = 0;
         uint32_t* d_xtab = nullptr; uint32_t xtab_M = ~0u, xtab_sb = 0, n_xtab = 0; SweepPlan xplan{};
         uint32_t* d_gtab = nullptr; size_t gtab_cap = 0;
+        // Two-part enumeration (sweep_split_kernel, GSX_SPLIT=0 turns it off): 20-nt guides, one PAM of the form N + two concrete
+        // characters, at most 3 mismatches, an index without N, no --start, no threshold pass, and a jump table deep enough to hold
+        // both capped halves (13 characters: the PAM and the proximal half of the PAM-first form; with fewer, that form would hand the
+        // tree search alignments with two proximal mismatches only for the re-anchoring to drop them).  Per guide and strand a quarter
+        // of the summary sectors of the plain sweep.
+        const uint32_t split_half = 10;
+        const bool split_ok = sweep_sb != 0 && !use_variants && p.threshold <= 0 && !p.start && prep.n_fast_pams == 1 && prep.plen == 3 &&
+                              (prep.pampack & 7u) == 4u && ((prep.pampack >> 3) & 7u) < 4u && ((prep.pampack >> 6) & 7u) < 4u &&
+                              prep.min_qlen == 2 * split_half && prep.max_qlen == 2 * split_half && p.mismatches <= kSplitMaxM && plain_index &&
+                              ftab_L >= prep.plen + split_half && n < (1u << 22) && env_int("GSX_SPLIT", 1) != 0;
+        // slices one character wider than the plain sweep's: a quarter of the patterns per guide, so four times the slice keeps the
+        // patterns per work unit up (3.1 Gb, 200 k guides, one B200: sweep 13.0 ms at sb = 4 against 15.9 at 5 and 15.7 at 3,
+        // profiles/r03a_split_ab_3100mb_200k.jsonl)
+        const uint32_t split_sb = split_ok && env_int("GSX_SPLIT_SB", 0) > 0 ? (uint32_t)env_int("GSX_SPLIT_SB", 0) : (sweep_sb > 1 ? sweep_sb - 1 : sweep_sb);
+        uint32_t* d_sxtab = nullptr; uint32_t n_sxtab = 0; SplitPlan splan{};
+        uint64_t* d_gq2 = nullptr; SeedNode* d_queue2 = nullptr; uint64_t queue2_cap = 0;
+        MatchRec* d_matches2 = nullptr; uint64_t matches2_cap = 0; uint32_t* d_nmatch2 = nullptr;
+        uint32_t* d_ctrs2 = split_ok ? B.alloc<uint32_t>(4, true, s) : nullptr;      // [0] form-1 seed count [1] task counter [2] form-1 match count
+        bool split_ran = false;
         // fast path launch over ng guides (m.gq): [sweep_kernel ->] search_fast_kernel.  d_ctrs: [3] seed queue count, [4] sweep work-unit counter
         uint32_t lean_qmin = prep.min_qlen, lean_qmax = prep.max_qlen;              // guide lengths of the batch the fast kernels see (edited guides: - R .. + D)
+        auto launch_split = [&](SearchArgs& m, uint32_t ng, cudaEvent_t ev_mid) {
+            const uint32_t sb = split_sb;
+            if (!d_sxtab) {
+                std::vector<uint32_t> xtab;
+                split_make_plan(ftab_L, sb, m.p.M, 2 * split_half, prep.plen, prep.pampack, split_half, splan, xtab);
+                if (xtab.size() > (size_t)kSplitXtabShared) throw std::runtime_error("two-part enumeration: xor table too long for this slice width");
+                n_sxtab = (uint32_t)xtab.size();
+                d_sxtab = B.alloc<uint32_t>(xtab.size());
+                CK(cudaMemcpyAsync(d_sxtab, xtab.data(), xtab.size() * 4, cudaMemcpyHostToDevice, s)); CK(cudaStreamSynchronize(s));
+                d_gq2 = B.alloc<uint64_t>(ng); d_nmatch2 = B.alloc<uint32_t>(ng + 1);
+                CK(launch_split_queries(m.gq, ng, prep.pampack, prep.plen, d_gq2, s)); n_launches++;
+            }
+            if (!d_queue) d_queue = B.alloc<SeedNode>(queue_cap);
+            if (queue2_cap != queue_cap) { if (d_queue2) B.free_one(d_queue2); d_queue2 = B.alloc<SeedNode>(queue_cap); queue2_cap = queue_cap; }
+            if (matches2_cap < m.p.match_cap) { if (d_matches2) B.free_one(d_matches2); d_matches2 = B.alloc<MatchRec>(m.p.match_cap); matches2_cap = m.p.match_cap; }
+            CK(cudaMemsetAsync(d_ctrs2, 0, 4 * sizeof(uint32_t), s));
+            SweepArgs w{};
+            w.plan.L = ftab_L; w.plan.sb = sb; w.plan.M = m.p.M; w.split = splan;
+            w.st[0] = m.st[0]; w.st[1] = m.st[1]; w.gq = m.gq; w.gq2 = d_gq2; w.skip = m.skip; w.n_guides = ng; w.xtab = d_sxtab; w.n_xtab = n_sxtab;
+            w.M = m.p.M; w.plen = m.plen; w.pampack = m.pampack;
+            w.queue = d_queue; w.queue_cap = (uint32_t)queue_cap; w.queue_count = d_ctrs + 3; w.item_counter = d_ctrs + 4;
+            w.queue2 = d_queue2; w.queue2_count = d_ctrs2 + 0;
+            w.error_flag = d_ctrs + 2; w.stats = d_stats;
+            if (gtab_cap < 2 * (size_t)ng) { if (d_gtab) B.free_one(d_gtab); d_gtab = B.alloc<uint32_t>((size_t)ng * 40); gtab_cap = 2 * (size_t)ng; }
+            w.gtab = d_gtab;
+            CK(launch_sweep_guides(w, s)); n_launches++;                          // rows 0 .. ng-1: form 0
+            SweepArgs w1 = w; w1.gq = d_gq2; w1.plen = 0; w1.pampack = 0; w1.gtab = d_gtab + (size_t)ng * 20;
+            CK(launch_sweep_guides(w1, s)); n_launches++;                         // rows ng .. 2ng-1: form 1
+            CK(launch_sweep_split(w, env_int("GSX_SPLIT_CTAS", 6), di.sm_count, s)); n_launches++;
+            if (ev_mid) CK(cudaEventRecord(ev_mid, s));
+            m.seeds = d_queue; m.n_seeds = d_ctrs + 3; m.seed_cap = (uint32_t)queue_cap; m.combos = nullptr; m.n_combos = 0;
+            CK(launch_search_fast(m, variant_f, di.sm_count, s)); n_launches++;
+            // form 1: the tree search of its seeds with the PAM-first query (all of it protospacer), into an arena of its own
+            SearchArgs m1 = m;
+            m1.gq = d_gq2; m1.plen = 0; m1.pampack = 0; m1.seeds = d_queue2; m1.n_seeds = d_ctrs2 + 0;
+            m1.task_counter = d_ctrs2 + 1; m1.match_count = d_ctrs2 + 2; m1.matches = d_matches2; m1.guide_nmatch = d_nmatch2;
+            CK(launch_search_fast(m1, variant_f, di.sm_count, s)); n_launches++;
+            ReanchorArgs r{};
+            r.st[0] = m.st[0]; r.st[1] = m.st[1]; r.in = d_matches2; r.n_in = d_ctrs2 + 2; r.in_cap = m.p.match_cap;
+            r.gq = m.gq; r.gq2 = d_gq2; r.pampack = prep.pampack; r.plen = prep.plen;
+            r.out = m.matches; r.out_count = m.match_count; r.out_cap = m.p.match_cap; r.guide_nmatch = m.guide_nmatch; r.error_flag = m.error_flag;
+            r.stats = d_stats;
+            CK(launch_reanchor(r, s)); n_launches++;
+            split_ran = true;
+        };
         auto launch_fast = [&](SearchArgs& m, uint32_t ng, uint32_t sb, cudaEvent_t ev_mid) {
+            if (sb && split_ok && !m.p.counting && !m.fmask) { launch_split(m, ng, ev_mid); return; }
             if (sb) {
                 SweepArgs w{};
                 if (xtab_M != m.p.M || xtab_sb != sb) {
@@ -1062,6 +1127,7 @@ static void run_device_job(DeviceJob* job) {
             uint32_t h[4]; read_ctrs(h, 4, d_ctrs); n_launches++;
             B.free_one(d_spill);
             if (h[2] & GSX_KERR_WATCHDOG) throw std::runtime_error("search kernel watchdog tripped");
+            if (h[2] & GSX_KERR_REANCHOR) throw std::runtime_error("two-part search: a PAM-first match has no interval in the other index");
             if (h[2] & (GSX_KERR_MATCH_OVERFLOW | GSX_KERR_SPILL_OVERFLOW | GSX_KERR_QUEUE_OVERFLOW)) {
                 B.free_one(d_matches);
                 if (h[2] & GSX_KERR_QUEUE_OVERFLOW) grow_queue();
@@ -1071,6 +1137,7 @@ static void run_device_job(DeviceJob* job) {
                 continue;
             }
             n_matches = h[1]; n_seeds_used = use_sweep ? h[3] : 0;
+            if (split_ran) { uint32_t h1; read_ctrs(&h1, 1, d_ctrs2); n_seeds_used += h1; n_launches++; }
             break;
         }
         }

@@ -816,6 +816,62 @@ GSX_HD uint32_t sweep_pattern(const SweepPlan& pl, const uint32_t* xtab, uint32_
     return (beta << low_bits) | (((uint32_t)q & ((1u << low_bits) - 1u)) ^ (w & 0x0FFFFFFFu));
 }
 
+// ---- two-part enumeration (sweep_split_kernel) ------------------------------------------------------------------------------
+// The strand indexes are over a text and its reverse complement, so the alignment a backward search of the consumed string
+// u_0 .. u_{T-1} finds in one index is the one a backward search of c_k = complement(u_{T-1-k}) finds in the other: the same
+// site read PAM-first.  split_query turns a distal-first query (q: protospacer, then pampack) into that PAM-first form: the PAM's
+// characters complemented in reverse order (a wildcard becomes A: the plan lets that character take all four symbols), then the
+// protospacer complemented from its PAM-proximal end.  The narrow key of such a match has T digits, all of the protospacer kind.
+GSX_HD uint64_t split_query(uint64_t q, uint32_t pampack, uint32_t plen) {
+    const uint32_t qlen = (uint32_t)(q >> 58), T = qlen + plen;
+    uint64_t v = (uint64_t)T << 58;
+    for (uint32_t k = 0; k < T; k++) {
+        uint32_t c;
+        if (k < plen) { const uint32_t pc = (pampack >> (3u * (plen - 1u - k))) & 7u; c = pc < 4u ? 3u - pc : 0u; }
+        else c = 3u - ((uint32_t)(q >> (2u * (qlen - 1u - (k - plen)))) & 3u);
+        v |= (uint64_t)c << (2u * k);
+    }
+    return v;
+}
+// A form-1 match (key over the PAM-first characters, found with query q2) as the distal-first consumed string u[0 .. T-1] (2-bit
+// codes) of the same site; returns the mismatches of u among the first `head` protospacer characters of q
+GSX_HD uint32_t split_unfold(uint64_t key, uint64_t q2, uint32_t T, uint64_t q, uint32_t head, uint32_t u[kMaxQ]) {
+    for (uint32_t k = T; k-- > 0;) {
+        const uint32_t d = (uint32_t)(key % 5ull); key /= 5ull;
+        const uint32_t c = d == 0u ? ((uint32_t)(q2 >> (2u * k)) & 3u) : d - 1u;
+        u[T - 1u - k] = 3u - c;
+    }
+    uint32_t mm = 0;
+    for (uint32_t j = 0; j < head; j++) mm += u[j] != (((uint32_t)(q >> (2u * j))) & 3u) ? 1u : 0u;
+    return mm;
+}
+// the narrow key and the mismatches the distal-first search gives the consumed string u (protospacer digits against q, then PAM digits)
+GSX_HD uint64_t split_key(const uint32_t* u, uint64_t q, uint32_t plen, uint32_t& mm) {
+    const uint32_t qlen = (uint32_t)(q >> 58);
+    uint64_t key = 0; mm = 0;
+    for (uint32_t j = 0; j < qlen + plen; j++) {
+        uint32_t d;
+        if (j < qlen) { d = u[j] == ((uint32_t)(q >> (2u * j)) & 3u) ? 0u : 1u + u[j]; mm += d ? 1u : 0u; }
+        else d = u[j] < 3u ? u[j] : 4u;
+        key = key * 5ull + d;
+    }
+    return key;
+}
+// table characters (2 bits each, low bit set) of form 0 / 1 by class; the split is after the guide's first `half` characters
+//   form 0 (distal-first, qlen characters then the PAM): characters 0 .. half-1 capped, the rest cost budget
+//   form 1 (PAM-first): the PAM's concrete characters never substituted, its wildcards free, the next qlen - half characters capped
+GSX_HD void split_classes(uint32_t form, uint32_t L, uint32_t qlen, uint32_t plen, uint32_t pampack, uint32_t half,
+                          uint32_t& cost, uint32_t& cap, uint32_t& exact, uint32_t& freec) {
+    cost = cap = exact = freec = 0;
+    for (uint32_t k = 0; k < L && k < 16u; k++) {
+        const uint32_t bit = 1u << (2u * k);
+        if (form == 0u) { cost |= bit; if (k < half) cap |= bit; continue; }
+        if (k < plen) { if (((pampack >> (3u * (plen - 1u - k))) & 7u) == 4u) freec |= bit; else exact |= bit; continue; }
+        cost |= bit;
+        if (k < plen + (qlen - half)) cap |= bit;
+    }
+}
+
 // ---- several alternative PAMs in one pass (specialised kernels, optional) ----------------------------------------------
 // The reference searches the PAMs of a guide one after the other into the same std::set (process.hpp:51-56, index.hpp:210-212),
 // so the result is the union of the per-PAM match sets.  One pass finds the same union: search with the FILTER PAM -- the

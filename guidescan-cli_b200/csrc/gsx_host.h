@@ -143,6 +143,9 @@ std::vector<uint64_t> ftab_combos(uint32_t n_pos, uint32_t M);
 // slice-major enumeration plan (gsx_core.h sweep_pattern): the xor table of every way to substitute at most M of the
 // characters outside the slice, listed per pass and budget
 void sweep_make_plan(uint32_t L, uint32_t sb, uint32_t M, SweepPlan& plan, std::vector<uint32_t>& xtab);
+// the same for the two-part enumeration of guides of qlen characters and a PAM of plen (gsx_types.h SplitPlan, gsx_core.h split_classes)
+void split_make_plan(uint32_t L, uint32_t sb, uint32_t M, uint32_t qlen, uint32_t plen, uint32_t pampack, uint32_t half, SplitPlan& plan,
+                     std::vector<uint32_t>& xtab);
 // one bit per 64-row block that holds a row whose BWT symbol is not A/C/G/T (gsx_core.h exc_before)
 std::vector<uint32_t> build_exc_map(const HostStrand& h);
 // bulges as edited guides (gsx_core.h variant_op): every op list within the budgets; their number

@@ -11,6 +11,7 @@
 #include <cstdio>
 #include <cstring>
 #include <fstream>
+#include <functional>
 #include <sstream>
 #include <thread>
 
@@ -362,6 +363,37 @@ void sweep_make_plan(uint32_t L, uint32_t sb, uint32_t M, SweepPlan& plan, std::
     for (uint32_t z = 0; z < 2; z++)
         for (uint32_t B = 0; B <= M; B++)
             for (uint32_t t = 0; t < plan.xcnt[z][B]; t++) if ((xtab[plan.xoff[z][B] + t] & 15u) == 0u) plan.xlines[z][B]++;
+}
+
+void split_make_plan(uint32_t L, uint32_t sb, uint32_t M, uint32_t qlen, uint32_t plen, uint32_t pampack, uint32_t half, SplitPlan& plan,
+                     std::vector<uint32_t>& xtab) {
+    memset(&plan, 0, sizeof plan);
+    xtab.clear();
+    const uint32_t n_pos = L - sb, top_mask = (1u << (2u * sb)) - 1u;
+    for (uint32_t f = 0; f < 2; f++) {
+        uint32_t cost, cap, exact, freec;
+        split_classes(f, L, qlen, plen, pampack, half, cost, cap, exact, freec);
+        plan.cost_top[f] = (cost >> (2u * n_pos)) & top_mask;
+        plan.cap_top[f] = (cap >> (2u * n_pos)) & top_mask;
+        plan.exact_top[f] = (exact >> (2u * n_pos)) & top_mask;
+        for (uint32_t c = 0; c < 2; c++)
+            for (uint32_t B = 0; B <= M; B++) {
+                plan.xoff[f][c][B] = (uint32_t)xtab.size();
+                // every xor value over characters 0 .. n_pos-1 with at most B substitutions that cost budget, at most c of them capped
+                std::function<void(uint32_t, uint32_t, uint32_t, uint32_t)> walk = [&](uint32_t k, uint32_t x, uint32_t used, uint32_t capped) {
+                    if (k == n_pos) { xtab.push_back(x | (used << 28)); return; }
+                    const uint32_t bit = 1u << (2u * k);
+                    if (exact & bit) { walk(k + 1, x, used, capped); return; }
+                    if (freec & bit) { for (uint32_t s = 0; s < 4; s++) walk(k + 1, x | (s << (2u * k)), used, capped); return; }
+                    walk(k + 1, x, used, capped);
+                    const uint32_t cp = (cap & bit) ? 1u : 0u;
+                    if (used < B && capped + cp <= c)
+                        for (uint32_t s = 1; s < 4; s++) walk(k + 1, x | (s << (2u * k)), used + 1u, capped + cp);
+                };
+                walk(0, 0, 0, 0);
+                plan.xcnt[f][c][B] = (uint32_t)xtab.size() - plan.xoff[f][c][B];
+            }
+    }
 }
 
 // ---- native cache format (<prefix>.gsx): a flat dump of the HBM layout ----------------------------------------

@@ -1408,6 +1408,212 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) sweep_lean_kernel(SweepArgs 
     if (lane == 0) { atomicAdd(a.stats + 0, n_nodes); atomicAdd(a.stats + 1, n_nodes + n_two + st.lines); atomicAdd(a.stats + 5, (unsigned long long)st.sectors); }
 }
 
+// ---------------------------------------------------------------------------------------------------------
+// sweep_split_kernel: the two-part enumeration (gsx_types.h SplitPlan).  An alignment with at most 3 mismatches has at most one of
+// them among the guide's ten PAM-distal characters -- form 0, the guide read distal-first as above, capped to one substitution over
+// those ten: 2 185 patterns per guide and strand at L = 14 -- or at most one among the ten PAM-proximal ones -- form 1, the same
+// site read PAM-first in the other strand's index: the PAM's concrete characters fixed, its wildcard free, one substitution over the
+// proximal half: 496 patterns.  Together a quarter of the 10 690 patterns of the plain enumeration.  A work unit = (index i, slice,
+// 32 guides) runs form 0 of task (g, i) and form 1 of task (g, 1 - i), both against index i's slice.  With a few patterns per guide
+// in a slice, the unit's patterns of both forms are ONE flat (guide, pattern) list, each lane judging its pattern with its own
+// guide's row of the guide table (rows n .. 2n-1: form 1).  Seeds of form 1 go to a queue of their own: search_fast_kernel
+// finishes them with the PAM-first query, and reanchor_kernel turns their matches into the records of the distal-first search.
+// ---------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ void split_emit(const SweepArgs& a, uint32_t lane, bool emit, bool form1, uint32_t idx, uint32_t tlm, const FtabEntry* tab) {
+#pragma unroll
+    for (int f = 0; f < 2; f++) {
+        const bool e = emit && (form1 == (f == 1));
+        const uint32_t emask = __ballot_sync(0xffffffffu, e);
+        if (!emask) continue;
+        uint32_t* cnt = f ? a.queue2_count : a.queue_count;
+        SeedNode* queue = f ? a.queue2 : a.queue;
+        uint32_t qbase = 0; const int leader = __ffs(emask) - 1;
+        if ((int)lane == leader) qbase = atomicAdd(cnt, (uint32_t)__popc(emask));
+        qbase = __shfl_sync(0xffffffffu, qbase, leader);
+        if (e) {
+            const uint32_t slot = qbase + __popc(emask & ((1u << lane) - 1u));
+            if (slot < a.queue_cap) {
+                const uint2 v = __ldg(reinterpret_cast<const uint2*>(tab + idx));
+                SeedNode sn; sn.sp = v.x; sn.ep = v.x + v.y - 1u; sn.idx = idx; sn.tlm = (tlm & 0x07FFFFFFu) | (a.plan.L << 27);
+                queue[slot] = sn;
+            } else atomicOr(a.error_flag, GSX_KERR_QUEUE_OVERFLOW);
+        }
+    }
+}
+// up to 32 parked nodes of either form: rows 16..31 of their intervals (as lean_drain)
+template <int NB>
+__device__ __forceinline__ void split_drain(const SweepArgs& a, ParkBuf& pk, uint32_t lane, LeanStats& st) {
+    const uint32_t n = pk.count < 32u ? pk.count : 32u;
+    const bool mine = lane < n;
+    uint32_t word = 0, tl = 0;
+    if (mine) { word = pk.idx[pk.count - n + lane]; tl = pk.tl[pk.count - n + lane]; }
+    __syncwarp();
+    pk.count -= n; st.sectors += n;
+    const uint32_t idx = word & 0x0FFFFFFFu, budget = word >> 28, row = tl >> 1;
+    const bool s1 = (tl & 1u) != 0u, form1 = row >= a.n_guides;
+    uint32_t alive = 0, w0;
+    if (mine) alive = lean_row_eval<NB, false>(a.gtab + (size_t)row * GT_WORDS, s1 ? a.st[1].sum1 : a.st[0].sum1, s1 ? a.st[1].sum2 : a.st[0].sum2,
+                                               idx, budget, 1u, true, w0);
+    const uint32_t g = row - (form1 ? a.n_guides : 0u);
+    split_emit(a, lane, alive != 0u, form1, idx, ((g << 1) | (tl & 1u)) | ((a.M - budget) << 24) | (budget << 27),
+               reinterpret_cast<const FtabEntry*>(s1 ? a.st[1].ftab : a.st[0].ftab));
+}
+
+template <int WARPS, int MINB, int NB>
+__global__ void __launch_bounds__(WARPS * 32, MINB) sweep_split_kernel(SweepArgs a) {
+    __shared__ SplitPlan s_sp;
+    __shared__ uint32_t s_park[WARPS][2][PK_SLOTS];
+    __shared__ uint32_t s_off[WARPS][32], s_n0[WARPS][32], s_l0[WARPS][32], s_l1[WARPS][32];
+    __shared__ uint32_t s_xtab[kSplitXtabShared];
+    for (int i = threadIdx.x; i < (int)(sizeof(SplitPlan) / 4); i += blockDim.x)
+        reinterpret_cast<uint32_t*>(&s_sp)[i] = reinterpret_cast<const uint32_t*>(&a.split)[i];
+    for (uint32_t i = threadIdx.x; i < (uint32_t)kSplitXtabShared; i += blockDim.x) s_xtab[i] = i < a.n_xtab ? a.xtab[i] : 0u;
+    __syncthreads();
+    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5, FULL = 0xffffffffu;
+    ParkBuf pk; pk.idx = s_park[warp][0]; pk.tl = s_park[warp][1]; pk.count = 0;
+    const uint32_t L = a.plan.L, sb = a.plan.sb, M = a.M, n = a.n_guides;
+    const uint32_t low = 2u * (L - sb), top_mask = (1u << (2u * sb)) - 1u;
+    const uint32_t n_slices = 1u << (2u * sb), n_gb = (n + 31u) >> 5;
+    const uint32_t items_per_strand = n_slices * n_gb, n_items = 2u * items_per_strand;      // (the host keeps this below 2^32)
+    LeanStats st = {0, 0, 0, 0};
+    for (;;) {
+        uint32_t item = 0;
+        if (lane == 0) item = atomicAdd(a.item_counter, 1u);
+        item = __shfl_sync(FULL, item, 0);
+        if (item >= n_items) break;
+        const uint32_t strand = item >= items_per_strand ? 1u : 0u;
+        const uint32_t rem = item - (strand ? items_per_strand : 0u);
+        const uint32_t beta = rem / n_gb, gb = rem - beta * n_gb;
+        const uint32_t g = gb * 32u + lane;
+        const bool valid = g < n && !(a.skip && a.skip[g]);
+        // this lane's guide: how many patterns of each form fall into the slice, and which list of the xor table they are
+        uint32_t cnt0 = 0, cnt1 = 0, l0 = 0, l1 = 0;
+        if (valid) {
+#pragma unroll
+            for (uint32_t f = 0; f < 2u; f++) {
+                const uint64_t q = __ldg((f ? a.gq2 : a.gq) + g);
+                const uint32_t x = ((uint32_t)(q >> low) & top_mask) ^ beta, d = (x | (x >> 1)) & 0x55555555u;
+                const uint32_t h = __popc(d & s_sp.cost_top[f]), cp = __popc(d & s_sp.cap_top[f]);
+                if (!(d & s_sp.exact_top[f]) && h <= M && cp <= 1u) {
+                    const uint32_t Bf = M - h, c = 1u - cp;
+                    const uint32_t w = s_sp.xoff[f][c][Bf] | (Bf << 16), k = s_sp.xcnt[f][c][Bf];
+                    if (f) { cnt1 = k; l1 = w; } else { cnt0 = k; l0 = w; }
+                }
+            }
+        }
+        const uint32_t mine = cnt0 + cnt1;
+        uint32_t incl = mine;
+#pragma unroll
+        for (uint32_t o = 1; o < 32u; o <<= 1) { const uint32_t v = __shfl_up_sync(FULL, incl, o); if (lane >= o) incl += v; }
+        const uint32_t total = __shfl_sync(FULL, incl, 31);
+        if (total == 0u) continue;
+        __syncwarp();
+        s_off[warp][lane] = incl - mine; s_n0[warp][lane] = cnt0; s_l0[warp][lane] = l0; s_l1[warp][lane] = l1;
+        __syncwarp();
+        st.sectors += total;
+        const unsigned char* sum0 = strand ? a.st[1].sum0 : a.st[0].sum0;
+        const unsigned char* sum2 = strand ? a.st[1].sum2 : a.st[0].sum2;
+        const FtabEntry* tab = reinterpret_cast<const FtabEntry*>(strand ? a.st[1].ftab : a.st[0].ftab);
+        const uint32_t hi_bits = beta << low;
+        for (uint32_t f0 = 0; f0 < total; f0 += 32u) {
+            while (pk.count >= 32u) split_drain<NB>(a, pk, lane, st);
+            const uint32_t fi = f0 + lane;
+            const bool live = fi < total;
+            uint32_t k = 0;                                                           // the lane whose list holds pattern fi: last k with off[k] <= fi
+#pragma unroll
+            for (uint32_t step = 16; step; step >>= 1) if (s_off[warp][k + step] <= fi) k += step;
+            uint32_t t = fi - s_off[warp][k];
+            const uint32_t n0 = s_n0[warp][k];
+            const bool form1 = t >= n0;
+            if (form1) t -= n0;
+            const uint32_t lw = form1 ? s_l1[warp][k] : s_l0[warp][k];
+            const uint32_t xw = live ? s_xtab[(lw & 0xFFFFu) + t] : 0u;
+            const uint32_t go = gb * 32u + k, row = live ? go + (form1 ? n : 0u) : 0u;
+            const uint32_t* rowp = a.gtab + (size_t)row * GT_WORDS;
+            const uint32_t idx = hi_bits | (__ldg(rowp + GT_QLOW) ^ (xw & 0x0FFFFFFFu));
+            const uint32_t budget = live ? (lw >> 16) - (xw >> 28) : 0u;
+            st.lines += __popc(__ballot_sync(FULL, live && (xw & 15u) == 0u));
+            uint32_t w0;
+            const uint32_t alive = lean_row_eval<NB, false>(rowp, sum0, sum2, idx, budget, 0u, live, w0);
+            // (w0 == 0 for lanes without a pattern and for empty table entries; the flags are only ever set on non-empty ones)
+            const bool emit = (alive | (w0 & SUM_WIDE32)) != 0u;                     // (more than 32 rows: not summarised, the tree search takes it)
+            const bool park = !emit && (w0 & SUM_WIDE16) != 0u;
+            st.nodes += (w0 & 0xFFFFu) ? 1u : 0u;
+            st.two += (w0 & SUM_TWO_BLOCKS) ? 1u : 0u;
+            split_emit(a, lane, emit, form1, idx, ((go << 1) | strand) | ((M - budget) << 24) | (budget << 27), tab);
+            lean_park(pk, lane, park, idx | (budget << 28), (row << 1) | strand);
+        }
+    }
+    while (pk.count) split_drain<NB>(a, pk, lane, st);
+    unsigned long long n_nodes = st.nodes, n_two = st.two;
+    for (int o = 16; o; o >>= 1) { n_nodes += __shfl_xor_sync(FULL, n_nodes, o); n_two += __shfl_xor_sync(FULL, n_two, o); }
+    if (lane == 0) { atomicAdd(a.stats + 0, n_nodes); atomicAdd(a.stats + 1, n_nodes + n_two + st.lines); atomicAdd(a.stats + 5, (unsigned long long)st.sectors); }
+}
+
+__global__ void split_queries_kernel(const uint64_t* __restrict__ gq, uint32_t n, uint32_t pampack, uint32_t plen, uint64_t* __restrict__ gq2) {
+    for (uint32_t g = blockIdx.x * blockDim.x + threadIdx.x; g < n; g += gridDim.x * blockDim.x) gq2[g] = split_query(gq[g], pampack, plen);
+}
+
+// one form-1 match: back to the distal-first consumed string of the same site; dropped when it has fewer than two mismatches among the
+// guide's first ten characters (form 0 found it); else its interval in the other index by an exact backward search (jump table, then
+// one occurrence lookup per interval end and character) and the record the distal-first search emits for it
+__global__ void reanchor_kernel(ReanchorArgs r) {
+    const uint32_t n_in = min(*r.n_in, r.in_cap);
+    unsigned long long lookups = 0;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_in; i += gridDim.x * blockDim.x) {
+        const MatchRec m = r.in[i];
+        const uint32_t g = m.task >> 1, s = (m.task & 1u) ^ 1u;
+        const uint64_t q = __ldg(r.gq + g), q2 = __ldg(r.gq2 + g);
+        const uint32_t qlen = (uint32_t)(q >> 58), T = qlen + r.plen, half = qlen / 2u;
+        uint32_t u[kMaxQ];
+        if (split_unfold(m.key_lo, q2, T, q, half, u) < 2u) continue;
+        uint32_t mm;
+        const uint64_t key = split_key(u, q, r.plen, mm);
+        const DevStrand& st = r.st[s];
+        const uint32_t L = st.ftab_L;
+        uint32_t e = 0;
+        for (uint32_t j = 0; j < L; j++) e |= u[j] << (2u * j);
+        const uint2 v = __ldg(reinterpret_cast<const uint2*>(reinterpret_cast<const FtabEntry*>(st.ftab) + e));
+        uint32_t sp = v.x, e1 = v.x + v.y;
+        lookups += 1u + 2u * (T - L);
+        for (uint32_t j = L; j < T && sp < e1; j++) {
+            const OccBlock* b0 = block_ptr(st, sp >> 6); const OccBlock* b1 = block_ptr(st, e1 >> 6);
+            uint32_t os[4], oe[4];
+            block_occ(st, b0->cnt, b0->hi, b0->lo, sp, os); block_occ(st, b1->cnt, b1->hi, b1->lo, e1, oe);
+            sp = st.C[u[j]] + os[u[j]]; e1 = st.C[u[j]] + oe[u[j]];
+        }
+        if (e1 - sp != m.width || sp >= e1) { atomicOr(r.error_flag, GSX_KERR_REANCHOR); continue; }
+        const uint32_t slot = atomicAdd(r.out_count, 1u);
+        if (slot < r.out_cap) {
+            MatchRec o; o.key_hi = 0; o.key_lo = key; o.task = (g << 1) | s; o.sp = sp; o.width = m.width; o.info = mm | (T << 24);
+            r.out[slot] = o;
+            atomicAdd(r.guide_nmatch + g, 1u);
+        } else atomicOr(r.error_flag, GSX_KERR_MATCH_OVERFLOW);
+    }
+    if (lookups) atomicAdd(r.stats + 7, lookups);
+}
+
+cudaError_t launch_split_queries(const uint64_t* gq, uint32_t n, uint32_t pampack, uint32_t plen, uint64_t* gq2, cudaStream_t s) {
+    split_queries_kernel<<<grid_for_n(n, 256, 148 * 8), 256, 0, s>>>(gq, n, pampack, plen, gq2);
+    return cudaGetLastError();
+}
+cudaError_t launch_sweep_split(const SweepArgs& a, int ctas_per_sm, int sm_count, cudaStream_t s) {
+    if (a.M > kSplitMaxM || a.n_xtab > (uint32_t)kSplitXtabShared) return cudaErrorInvalidValue;
+    const dim3 block(8 * 32);
+    switch (ctas_per_sm) {
+    case 4: sweep_split_kernel<8, 4, 4><<<sm_count * 4, block, 0, s>>>(a); break;
+    case 5: sweep_split_kernel<8, 5, 4><<<sm_count * 5, block, 0, s>>>(a); break;
+    case 6: sweep_split_kernel<8, 6, 4><<<sm_count * 6, block, 0, s>>>(a); break;
+    case 8: sweep_split_kernel<8, 8, 4><<<sm_count * 8, block, 0, s>>>(a); break;
+    default: return cudaErrorInvalidValue;
+    }
+    return cudaGetLastError();
+}
+cudaError_t launch_reanchor(const ReanchorArgs& r, cudaStream_t s) {
+    reanchor_kernel<<<148 * 4, 256, 0, s>>>(r);
+    return cudaGetLastError();
+}
+
 cudaError_t launch_sweep_guides(const SweepArgs& a, cudaStream_t s) {
     sweep_guides_kernel<<<grid_for_n(a.n_guides, 256, 148 * 8), 256, 0, s>>>(a, a.gtab);
     return cudaGetLastError();

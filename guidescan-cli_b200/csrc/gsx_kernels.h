@@ -10,7 +10,8 @@ enum : uint32_t {
     GSX_KERR_MATCH_OVERFLOW = 1,   // match arena too small: host retries with a larger one
     GSX_KERR_SPILL_OVERFLOW = 2,   // a warp's global spill stack is full: host retries with a larger one
     GSX_KERR_WATCHDOG = 4,         // iteration cap hit (never expected)
-    GSX_KERR_QUEUE_OVERFLOW = 8    // seed queue of the sweep kernel too small: host retries with a larger one
+    GSX_KERR_QUEUE_OVERFLOW = 8,   // seed queue of the sweep kernel too small: host retries with a larger one
+    GSX_KERR_REANCHOR = 16         // a form-1 match of a two-part search has no interval in the other index (never expected)
 };
 
 // level-L node that survived the sweep kernel's filter: the DFS kernel continues from it
@@ -73,6 +74,21 @@ struct SweepArgs {
     uint32_t* queue_count; uint32_t* item_counter; uint32_t* error_flag;
     unsigned long long* stats;         // [0] nodes [1] lookups (reference unit) [5] summary sectors loaded
     const uint32_t* fmask;             // as SearchArgs::fmask (nullptr = off)
+    // two-part enumeration (sweep_split_kernel): gtab holds 2 * n_guides rows, form 0 (gq) then form 1 (gq2); seeds of form 1 go to queue2
+    const uint64_t* gq2;
+    SeedNode* queue2; uint32_t* queue2_count;
+    SplitPlan split;
+};
+
+// the form-1 matches of a two-part search (sweep_split_kernel) -> the records the distal-first search emits for the same alignments
+struct ReanchorArgs {
+    DevStrand st[2];
+    const MatchRec* in; const uint32_t* n_in; uint32_t in_cap;     // form-1 matches (task = guide * 2 + the index they were found in)
+    const uint64_t* gq; const uint64_t* gq2;
+    uint32_t pampack, plen;
+    MatchRec* out; uint32_t* out_count; uint32_t out_cap;
+    uint32_t* guide_nmatch; uint32_t* error_flag;
+    unsigned long long* stats;         // [7] += jump-table and occurrence lookups
 };
 
 struct LocateArgs {
@@ -118,6 +134,11 @@ int search_fast_grid_warps(int variant, int sm_count);
 cudaError_t launch_search_fast(const SearchArgs& a, int variant, int sm_count, cudaStream_t s);
 cudaError_t launch_sweep_guides(const SweepArgs& a, cudaStream_t s);      // per-guide filter masks (before launch_sweep)
 cudaError_t launch_sweep(const SweepArgs& a, int variant, int sm_count, cudaStream_t s);
+// two-part enumeration: PAM-first queries of the guides (gsx_core.h split_query), the sweep over both forms, the re-anchoring
+cudaError_t launch_split_queries(const uint64_t* gq, uint32_t n, uint32_t pampack, uint32_t plen, uint64_t* gq2, cudaStream_t s);
+constexpr int kSplitXtabShared = 1024;          // words of shared memory sweep_split_kernel keeps for its xor table
+cudaError_t launch_sweep_split(const SweepArgs& a, int ctas_per_sm, int sm_count, cudaStream_t s);
+cudaError_t launch_reanchor(const ReanchorArgs& r, cudaStream_t s);
 // bulges as edited guides (gsx_core.h variant_rewrite)
 cudaError_t launch_variant_expand(const GuideRec* guides, uint32_t n_seg, uint32_t n_v, const uint32_t* seg, const uint32_t* descs,
                                   const uint32_t* doff, uint64_t* vq, uint32_t* vdesc, uint32_t* vguide, uint32_t* vfmask, cudaStream_t s);

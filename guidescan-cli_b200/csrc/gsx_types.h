@@ -120,6 +120,20 @@ struct SweepPlan {
     uint32_t xlines[2][kMaxDist + 1];   // how many of those patterns leave the first two characters alone (each opens a jump-table line: work counter)
 };
 
+// two-part enumeration of the sweep (sweep_split_kernel, gsx_core.h split_query): every alignment with at most 3 mismatches has at
+// most one of them among the guide's ten PAM-distal characters (form 0: the guide read distal-first, as sweep_lean_kernel reads it)
+// or at most one among the ten PAM-proximal ones (form 1: the guide read PAM-first, searched in the other strand's index).  Per form
+// and table character a class: costs budget, never substituted, free (all four symbols at no cost), or costs budget and counts
+// against the cap of one substitution over the form's capped half.
+constexpr uint32_t kSplitMaxM = 3;
+struct SplitPlan {
+    // the slice characters (2 bits each, the low bit set) of each form that cost budget / count against the cap / are never substituted
+    uint32_t cost_top[2], cap_top[2], exact_top[2];
+    // xoff[f][c][B]: start, in the xor table, of the patterns of form f over the characters outside the slice with at most c (0 or 1)
+    // substitutions left under the cap and budget B; xcnt: their number.  Entry = xor value | budget used << 28 (sweep_pattern)
+    uint32_t xoff[2][2][kSplitMaxM + 1], xcnt[2][2][kSplitMaxM + 1];
+};
+
 // node meta word
 constexpr uint32_t META_LVL_MASK = 63u;           // bits 0..5   guide positions + PAM characters consumed
 constexpr uint32_t META_MM_SHIFT = 6;             // bits 6..8
