@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 #include <algorithm>
 #include <chrono>
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -659,11 +660,147 @@ static std::vector<Node> expand_roots(const gsx_index* ix, const Prepared& prep,
     return cur;
 }
 
+// ---- the search plan ----------------------------------------------------------------------------------------------------------
+static constexpr uint32_t kSplitHalf = 10;          // the two-part sweep cuts its 20-nt guides here
+static constexpr int kUnset = INT_MIN;              // a knob that is not set
+SearchPlan gsx::plan_search(const Prepared& prep, const gsx_params& p, const IndexShape& ix, uint32_t n) {
+    SearchPlan pl;
+    const uint32_t L = ix.ftab_L[0];
+    pl.variant_general[0] = env_int("GSX_SEARCH_VARIANT", 0); pl.variant_general[1] = env_int("GSX_SEARCH_VARIANT_WIDE", 0);
+    pl.variant_fast = env_int("GSX_FAST_VARIANT", ix.lines ? 1 : 0);
+    // fast path (search_fast_kernel) when the batch and the index allow it; GSX_FORCE_GENERAL=1 keeps the general kernel
+    // (an index whose only non-ACGT BWT row is the sentinel runs the plain kernels; genomes with N / IUPAC characters -- every
+    // real assembly -- run search_fast_kernel<..., EXC> behind the same sweep: 4.75 M guides/s against 80 k on the general kernel
+    // at 3.1 Gb with 300 runs of N, output identical to the CPU arm's, profiles/r02a_session_3100mb.jsonl; GSX_FAST_ON_N=0 turns it off)
+    pl.exc = !ix.plain && env_int("GSX_FAST_ON_N", 1) != 0 && pl.variant_fast == 1 && ix.exc_map;
+    pl.use_fast = (prep.fast_ok || prep.variant_ok) && !env_int("GSX_FORCE_GENERAL", 0) && n < (1u << 23) && (ix.plain || pl.exc);
+    // bulges: the search runs over the guides' edited forms (gsx_core.h variant_rewrite), in chunks, on the same kernels
+    pl.use_variants = pl.use_fast && prep.variant_ok;
+    // The specialised kernels read the packed guides (8 bytes each) only; the 80-byte records are needed from the locate stage
+    // on.  Their upload (pageable host memory: the call blocks the host) is issued on a second stream AFTER the first search
+    // launch, so that it runs under the search instead of in front of it.
+    pl.late_guides = pl.use_fast && !pl.use_variants;
+    const bool wide = prep.wide;
+    pl.search_warps = pl.use_fast ? search_fast_grid_warps(pl.variant_fast, ix.sm_count) : search_grid_warps(wide, pl.variant_general[wide], ix.sm_count);
+    pl.threshold_warps = pl.use_fast ? pl.search_warps : search_grid_warps(false, pl.variant_general[0], ix.sm_count);
+    if (pl.use_fast) {
+        // L2 residency hint: intervals wide enough that all such blocks of both strands fit the L2 budget
+        // (a level-d interval end costs one 128-byte line; lines touched down to level D ~ 2.7 * 4^D per strand)
+        const double l2_bytes = (double)env_int("GSX_L2_PIN_MB", 64) * 1e6;
+        const double w = l2_bytes > 0 ? (double)ix.rows * 2.0 * 2.7 * 128.0 / l2_bytes : 4.0e9;
+        pl.pin_width = w >= 4.0e9 ? 0xFFFFFFFFu : (uint32_t)std::max(256.0, w);
+    }
+    // slice-major front end (sweep_kernel) for large batches: needs the jump table and the look-ahead lines
+    pl.ftab_L = L; pl.sweep_variant_set = env_int("GSX_SWEEP_VARIANT", kUnset); pl.load_mode = (uint32_t)env_int("GSX_SWEEP_LOAD", 2);
+    if (pl.use_fast && L >= 6 && ix.ftab_L[1] == L && ix.sum0 && env_int("GSX_SWEEP", 1)) {
+        const double per_strand = 40.0 * std::pow(4.0, (double)L);                     // sum0 + the part of sum1 that is touched
+        const double target = (double)env_int("GSX_SWEEP_SLICE_MB", 12) * 1e6;
+        uint32_t sb = 1; while (sb < L - 3 && per_strand / std::pow(4.0, (double)sb) > target) sb++;
+        if (env_int("GSX_SWEEP_SB", 0) > 0) sb = (uint32_t)env_int("GSX_SWEEP_SB", 0);
+        pl.sweep_width = sb >= 1 && sb + 3 <= L ? sb : 0; pl.sweep_min = (uint32_t)env_int("GSX_SWEEP_MIN", 8192);
+    }
+    pl.search_sb = pl.use_variants ? 0u : pl.sweep_sb(n, prep.min_qlen, std::max<uint32_t>(p.mismatches, p.threshold > 0 ? (uint32_t)p.threshold : 0u));
+    if (p.threshold > 0) pl.threshold_sb = pl.sweep_sb(n, prep.min_qlen, (uint32_t)p.threshold);
+    pl.combos = pl.use_fast && L && !pl.search_sb; pl.threshold_combos = p.threshold > 0 && pl.use_fast && L && !pl.threshold_sb;
+    // Two-part enumeration (sweep_split_kernel, GSX_SPLIT=0 turns it off): 20-nt guides, one PAM of the form N + two concrete
+    // characters, at most 3 mismatches, an index without N, no --start, no threshold pass, and a jump table deep enough to hold
+    // both capped halves (13 characters: the PAM and the proximal half of the PAM-first form; with fewer, that form would hand the
+    // tree search alignments with two proximal mismatches only for the re-anchoring to drop them).  Per guide and strand a quarter
+    // of the summary sectors of the plain sweep.
+    pl.split = pl.search_sb != 0 && !pl.use_variants && p.threshold <= 0 && !p.start && prep.n_fast_pams == 1 && prep.plen == 3 &&
+               (prep.pampack & 7u) == 4u && ((prep.pampack >> 3) & 7u) < 4u && ((prep.pampack >> 6) & 7u) < 4u &&
+               prep.min_qlen == 2 * kSplitHalf && prep.max_qlen == 2 * kSplitHalf && p.mismatches <= kSplitMaxM && ix.plain &&
+               L >= prep.plen + kSplitHalf && n < (1u << 22) && env_int("GSX_SPLIT", 1) != 0;
+    if (pl.split) {
+        // slices one character wider than the plain sweep's: a quarter of the patterns per guide, so four times the slice keeps the
+        // patterns per work unit up (3.1 Gb, 200 k guides, one B200: sweep 13.0 ms at sb = 4 against 15.9 at 5 and 15.7 at 3,
+        // profiles/r03a_split_ab_3100mb_200k.jsonl)
+        pl.split_sb = env_int("GSX_SPLIT_SB", 0) > 0 ? (uint32_t)env_int("GSX_SPLIT_SB", 0) : (pl.search_sb > 1 ? pl.search_sb - 1 : pl.search_sb);
+        pl.split_ctas = env_int("GSX_SPLIT_CTAS", 6);
+    }
+    // alternative PAMs (process.hpp:51-56): the searches of the PAMs are independent and their matches are collected in
+    // the same per-guide sets, so each PAM gets its own pass over the same arenas; only the work counters start over
+    // Default (GSX_FUSED_PAMS=0 keeps one pass per PAM; m = 4 with NGG + NAG at 3.1 Gb: 232 k against 142 k guides/s, same text): the PAMs in
+    // ONE pass -- search with the filter PAM, keep the alignments whose PAM characters spell a real PAM (gsx_core.h fused_pam_ok)
+    pl.fuse_pams = prep.n_fast_pams > 1 && pl.variant_fast == 1 && env_int("GSX_FUSED_PAMS", 1) != 0;
+    if (!pl.use_fast) {
+        const int gw = search_grid_warps(wide, pl.variant_general[wide], ix.sm_count);
+        if (gw > 0 && (uint64_t)2 * n < (uint64_t)4 * gw) pl.expand_roots = (size_t)8 * gw;          // fewer tasks than the grid can keep busy
+    }
+    // seed queue of the sweep: 12 survivors per guide measured at m = 3 on 3.1 Gb (two orders of magnitude more at m = 4);
+    // sized with a wide margin, never beyond the 32-bit slot numbers the kernels use; an overflow is retried with 4x the room
+    const uint64_t queue_set = (uint64_t)std::max(env_int("GSX_QUEUE_CAP", 0), 0);
+    pl.queue_cap = queue_set ? queue_set : std::min<uint64_t>(std::max<uint64_t>((uint64_t)n * (p.mismatches >= 4 ? 1024 : 256), 1u << 20), 1ull << 30);
+    // Match arena: an overflow costs a second run of the whole search, so the first size has to be right.  Expected matches per
+    // guide on a genome without structure = 2 strands x rows x (substitution patterns within the budget) / 4^length x the fraction
+    // of sites a PAM list accepts: 11 at 3 mismatches / NGG on 3.1 Gb, 300 at 4 mismatches with NGG + NAG (the size round 1 got
+    // wrong: n x 48 -- every such call searched twice).  The job raises it to what earlier calls on the index needed.
+    pl.match_per_guide = wide ? 2048.0 : 48.0;
+    if (!wide) {
+        const double ql = (double)std::max<uint32_t>(prep.min_qlen, 1);
+        double patterns = 0, c = 1;                                           // sum over j <= M of C(q, j) 3^j
+        for (uint32_t j = 0; j <= p.mismatches && j <= prep.min_qlen; j++) { patterns += c; c = c * 3.0 * (ql - j) / (j + 1.0); }
+        double pam_frac = 0;
+        for (int ps = 0; ps < kMaxPamSets; ps++) {
+            double f = 0;
+            for (int k = 0; k < prep.pamsets[ps].n_pams; k++) { double g1 = 1; for (int j = 0; j < prep.pamsets[ps].plen[k]; j++) if (prep.pamsets[ps].sym[k][j] != SYM_N) g1 *= 0.25; f += g1; }
+            pam_frac = std::max(pam_frac, std::min(1.0, f));
+        }
+        const double expect = 2.0 * (double)ix.rows * patterns / std::pow(4.0, ql) * pam_frac;
+        pl.match_per_guide = std::max(pl.match_per_guide, 1.5 * expect + 8.0);
+    }
+    pl.match_cap_set = (uint64_t)std::max(env_int("GSX_MATCH_CAP", 0), 0);      // tests: force the retry path
+    const uint32_t spill_set = (uint32_t)std::max(env_int("GSX_SPILL_CAP", 0), 0);
+    pl.spill_cap = spill_set ? spill_set : (wide && !pl.use_variants) ? 8192 : 2048;
+    if (pl.use_variants) {
+        const uint32_t R = p.rna_bulges, D = p.dna_bulges;
+        pl.chunk = (uint32_t)std::min<int64_t>(std::max<int64_t>(env_int("GSX_VARIANT_CHUNK", 262144), 1), (1 << 22));
+        // the sweep skips patterns that substitute an inserted position (GSX_FORCED_SWEEP=0: it tests them and the rewrite drops their
+        // matches; 11 % fewer seeds, 1.4 % less search time at 3.1 Gb)
+        pl.fmask = env_int("GSX_FORCED_SWEEP", 1) != 0;
+        pl.edited_qmin = prep.min_qlen > R ? prep.min_qlen - R : 0; pl.edited_qmax = prep.max_qlen + D;
+        pl.chunk_queue_cap = queue_set ? queue_set : std::max<uint64_t>((uint64_t)pl.chunk * 256, 1u << 20);
+        pl.chunk_match_cap = std::max<uint64_t>((uint64_t)pl.chunk * 48, 1u << 18);
+        pl.edited_match_cap = std::max<uint64_t>(1u << 18, std::min<uint64_t>((uint64_t)n * bulge_variant_count(prep.max_qlen, R, D) * 12, 1u << 26));
+        if (pl.match_cap_set) pl.chunk_match_cap = pl.edited_match_cap = pl.match_cap_set;
+    }
+    // match ordering (GSX_ORDER: 0 warp per guide, 1 CTA per guide, 2 radix sort) and specificity (GSX_SPEC_WARP) by default follow
+    // the matches and hits per guide, known after the search
+    pl.order_probe = !env_int("GSX_ORDER", 0) && !env_int("GSX_ORDER_CTA", 0);
+    pl.order_mode = env_int("GSX_ORDER", env_int("GSX_ORDER_CTA", 0) ? 1 : kUnset); pl.spec_warp = env_int("GSX_SPEC_WARP", kUnset);
+    return pl;
+}
+
+uint32_t SearchPlan::sweep_sb(uint32_t ng, uint32_t min_qlen, uint32_t M) const {
+    if (!sweep_width || ng < sweep_min || min_qlen < ftab_L || M > 4) return 0;
+    return 2.0 * std::pow(4.0, (double)sweep_width) * ((ng + 31) / 32) * 8.0 >= 4.0e9 ? 0 : sweep_width;      // (32-bit work units)
+}
+
+// sweep_lean_kernel (variants 10-12) where its compiled loops cover the batch: at most 4 mismatches, every guide length of the
+// batch giving one of its plane layouts; sweep_kernel (variant 2) otherwise.  Measured at 3.1 Gb
+// (profiles/r02c_session_3100mb_sweep_lean3.jsonl): six CTAs per SM (variant 12) for plain batches of at most 3 mismatches --
+// 24.0 ms per 200 k guides against 36.6 for sweep_kernel --, five (variant 11) for 4 mismatches and for the edited guides of a
+// bulge search
+int SearchPlan::sweep_variant(uint32_t M, uint32_t qmin, uint32_t qmax, uint32_t plen, uint32_t pampack) const {
+    const int sv = sweep_variant_set != kUnset ? sweep_variant_set : (M <= 3 && !use_variants) ? 12 : 11;
+    bool lean = M <= 4;
+    for (uint32_t ql = qmin; lean && ql <= qmax; ql++) lean = sweep_shape_of(sweep_codes((uint64_t)ql << 58, ftab_L, plen, pampack)) >= 0;
+    return sv >= 10 && !lean ? 2 : sv;
+}
+
+static IndexShape shape_of(const DeviceIndex& di) {
+    const DevStrand &a = di.st[0].d, &b = di.st[1].d;
+    return IndexShape{a.n_exc == 1 && b.n_exc == 1 && a.n_nrows == 0 && b.n_nrows == 0, a.lines != nullptr, di.st[0].exc_map && di.st[1].exc_map,
+                      {a.ftab_L, b.ftab_L}, a.sum0 && b.sum0, a.n, di.sm_count};
+}
+
+// ---- the device job -----------------------------------------------------------------------------------------------------------
 // streams and events of one device job: released on every path out of run_device_job (errors included); in-flight copies are
 // waited for first, because the buffers they touch go back to the allocation pools right after
+enum JobEvent { kSearchBegin, kSearchEnd, kArrangeEnd, kLocateEnd, kScoreEnd, kCopyEnd, kSweepBegin, kSweepEnd, kJobEvents };
 struct JobStreams {
     cudaStream_t s = nullptr, s2 = nullptr;
-    cudaEvent_t ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}, ev_guides = nullptr;
+    cudaEvent_t ev[kJobEvents] = {}, ev_guides = nullptr;
     ~JobStreams() {
         if (s) cudaStreamSynchronize(s);
         if (s2) cudaStreamSynchronize(s2);
@@ -684,491 +821,386 @@ struct DeviceJob {
     uint32_t want = kWantAll;            // per-hit arrays to bring to the host (gsx_host.h)
 };
 
+// the sweep's state: xor table (of the last M and slice width), per-guide filter masks, seed queue
+struct SweepState {
+    uint32_t* xtab = nullptr; uint32_t xtab_M = ~0u, xtab_sb = 0, n_xtab = 0; SweepPlan plan{};
+    uint32_t* gtab = nullptr; size_t gtab_cap = 0; SeedNode* queue = nullptr; uint64_t queue_cap = 0;
+};
+// the two-part sweep's own state: its xor table, the PAM-first queries, their seed queue and match arena, and their counters
+struct SplitState {
+    uint32_t* xtab = nullptr; uint32_t n_xtab = 0; SplitPlan plan{};
+    uint64_t* gq2 = nullptr; uint32_t* nmatch2 = nullptr; SeedNode* queue2 = nullptr; uint64_t queue2_cap = 0;
+    MatchRec* matches2 = nullptr; uint64_t matches2_cap = 0; bool ran = false;
+    uint32_t* ctrs2 = nullptr;           // [0] form-1 seed count [1] task counter [2] form-1 match count
+};
+// a match arena search_until_fits grows: records, capacity, and the error when it would pass 2^31 records
+struct MatchArena { MatchRec* p; uint64_t cap; const char* too_many; };
+#define LAUNCH(call) do { CK(call); n_launches++; } while (0)
 
-static void run_device_job(DeviceJob* job) {
-    try {
-        const DeviceIndex& di = job->ix->dev[job->slot];
-        const Prepared& prep = *job->prep; const gsx_params& p = *job->p;
-        const uint32_t n = (uint32_t)(job->g1 - job->g0);
-        const uint32_t n_dist = p.mismatches + 1;
-        CK(cudaSetDevice(di.device));
-        DevBufs B(di.device);
-        Mailbox mbox;                                            // (declared before the streams: they are drained before it goes back to the free list)
-        JobStreams js;                                           // (declared after the buffer holder: destroyed -- synchronised -- before it)
+// One device job's state; run_device_job calls its stages in order.
+struct DeviceRun {
+    DeviceJob& job; const DeviceIndex& di; const Prepared& prep; const gsx_params& p;
+    const uint32_t n, n_dist;
+    const SearchPlan plan;
+    const uint64_t learn_key;            // index of learned_matches_per_guide: the option set
+    DevBufs B;
+    Mailbox mbox;                        // (declared before the streams: they are drained before it goes back to the free list)
+    JobStreams js;                       // (declared after the buffer holder: destroyed -- synchronised -- before it)
+    cudaStream_t &s = js.s, &s2 = js.s2;
+    // Calls from several host threads (the reference's own worker threads, or gsx_enumerate_start) take turns on a device from the
+    // first search launch to the last result copy (gsx::device_turn).
+    std::unique_lock<std::mutex> turn;
+    uint64_t n_launches = 0; bool guides_up = false;
+    GuideRec* d_guides = nullptr; PamSet* d_pamsets = nullptr; uint32_t* d_nmatch = nullptr; uint8_t* d_dropped = nullptr; unsigned long long* d_stats = nullptr;
+    uint32_t* d_ctrs = nullptr;          // [0] task counter [1] match count [2] error flag [3] seed queue count [4] sweep work units [5] final matches
+    SearchArgs a{};                      // what every search launch of the job starts from
+    SweepState sw; SplitState sp;
+    uint32_t qmin = 0, qmax = 0;         // guide lengths of the batch the fast kernels see (edited guides: - R .. + D)
+    MatchRec* d_matches = nullptr; uint32_t n_matches = 0, n_seeds = 0; bool use_sweep = false;
+    uint32_t *d_moff = nullptr, *d_sorted = nullptr, *d_sorted_off = nullptr, *d_nhits = nullptr, *d_hoff = nullptr, *d_cbd = nullptr;
+    uint32_t *d_hit_match = nullptr, *d_hit_row = nullptr, nh = 0;
+    LocateArgs L{}; SpecArgs S{}; unsigned long long stats[8] = {};
+
+    explicit DeviceRun(DeviceJob& j)
+        : job(j), di(j.ix->dev[j.slot]), prep(*j.prep), p(*j.p), n((uint32_t)(j.g1 - j.g0)), n_dist(j.p->mismatches + 1),
+          plan(plan_search(prep, p, shape_of(di), n)),
+          learn_key((uint64_t)p.mismatches | ((uint64_t)prep.n_fast_pams << 8) | ((uint64_t)p.rna_bulges << 16) | ((uint64_t)p.dna_bulges << 24) |
+                    ((uint64_t)prep.min_qlen << 32) | ((uint64_t)(prep.wide ? 1 : 0) << 40)), B(di.device) {}
+    // the first words of d_ctrs, read on the host without touching the copy engine
+    void read_ctrs(uint32_t* h, uint32_t n_words, const uint32_t* d_src) {
+        CK(launch_publish(d_src, n_words, mbox.p, s)); CK(cudaStreamSynchronize(s));
+        for (uint32_t i = 0; i < n_words; i++) h[i] = mbox.p[i];
+    }
+    void upload_guides(cudaStream_t st) {
+        if (guides_up) return;
+        const auto t0 = std::chrono::steady_clock::now();
+        CK(cudaMemcpyAsync(d_guides, prep.recs.data() + job.g0, (size_t)n * sizeof(GuideRec), cudaMemcpyHostToDevice, st));
+        CK(cudaEventRecord(js.ev_guides, st)); guides_up = true;
+        job.ctr.ms_h2d += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    }
+    // every way to substitute at most M of the jump table's characters but the last two (search_fast_kernel without a sweep)
+    void upload_combos(SearchArgs& m, uint32_t M) {
+        const std::vector<uint64_t> cb = ftab_combos(plan.ftab_L - 2, M);
+        uint64_t* d_cb = B.alloc<uint64_t>(cb.size());
+        CK(cudaMemcpyAsync(d_cb, cb.data(), cb.size() * 8, cudaMemcpyHostToDevice, s)); CK(cudaStreamSynchronize(s));
+        m.combos = d_cb; m.n_combos = (uint32_t)cb.size();
+    }
+    // streams, result arrays, the first uploads; false when the batch is empty.  Ends by taking the device's turn.
+    bool setup() {
         CK(cudaStreamCreate(&js.s)); CK(cudaStreamCreate(&js.s2));
         for (auto& e : js.ev) CK(cudaEventCreate(&e));
         CK(cudaEventCreateWithFlags(&js.ev_guides, cudaEventDisableTiming));
-        const cudaStream_t s = js.s, s2 = js.s2; cudaEvent_t* const ev = js.ev; const cudaEvent_t ev_guides = js.ev_guides;
-        // the first words of d_ctrs, read on the host without touching the copy engine
-        auto read_ctrs = [&](uint32_t* h, uint32_t n_words, const uint32_t* d_src) {
-            CK(launch_publish(d_src, n_words, mbox.p, s)); CK(cudaStreamSynchronize(s));
-            for (uint32_t i = 0; i < n_words; i++) h[i] = mbox.p[i];
-        };
-        HostArrays& H = job->out; H.n_guides = n;
+        HostArrays& H = job.out; H.n_guides = n;
         H.dropped = H.alloc<uint8_t>(n); H.n_hits_of = H.alloc<uint32_t>(n); H.hoff = H.alloc<uint32_t>(n + 1);
         H.specificity = H.alloc<float>(n); H.perfect = H.alloc<uint8_t>(n); H.cbd = H.alloc<uint32_t>((size_t)n * n_dist);
-        if (n == 0) { H.hoff[0] = 0; return; }
-
-        // fast path (search_fast_kernel) when the batch and the index allow it; GSX_FORCE_GENERAL=1 keeps the general kernel
-        // (an index whose only non-ACGT BWT row is the sentinel runs the plain kernels; genomes with N / IUPAC characters -- every
-        // real assembly -- run search_fast_kernel<..., EXC> behind the same sweep: 4.75 M guides/s against 80 k on the general kernel
-        // at 3.1 Gb with 300 runs of N, output identical to the CPU arm's, profiles/r02a_session_3100mb.jsonl; GSX_FAST_ON_N=0 turns it off)
-        const bool plain_index = di.st[0].d.n_exc == 1 && di.st[1].d.n_exc == 1 && di.st[0].d.n_nrows == 0 && di.st[1].d.n_nrows == 0;
-        const bool exc_index = !plain_index && env_int("GSX_FAST_ON_N", 1) != 0 && env_int("GSX_FAST_VARIANT", di.st[0].d.lines ? 1 : 0) == 1 &&
-                               di.st[0].exc_map && di.st[1].exc_map;
-        const bool use_fast = (prep.fast_ok || prep.variant_ok) && !env_int("GSX_FORCE_GENERAL", 0) && n < (1u << 23) && (plain_index || exc_index);
-        // bulges: the search runs over the guides' edited forms (gsx_core.h variant_rewrite), in chunks, on the same kernels
-        const bool use_variants = use_fast && prep.variant_ok;
-        // The specialised kernels read the packed guides (8 bytes each) only; the 80-byte records are needed from the locate stage
-        // on.  Their upload (pageable host memory: the call blocks the host) is issued on a second stream AFTER the first search
-        // launch, so that it runs under the search instead of in front of it.
-        const bool late_guides = use_fast && !use_variants && env_int("GSX_LATE_GUIDES", 1) != 0;
-        GuideRec* d_guides = B.alloc<GuideRec>(n);
-        PamSet* d_pamsets = B.alloc<PamSet>(kMaxPamSets);
-        bool guides_up = false;
-        auto upload_guides = [&](cudaStream_t st) {
-            if (guides_up) return;
-            const auto t0 = std::chrono::steady_clock::now();
-            CK(cudaMemcpyAsync(d_guides, prep.recs.data() + job->g0, (size_t)n * sizeof(GuideRec), cudaMemcpyHostToDevice, st));
-            CK(cudaEventRecord(ev_guides, st));
-            job->ctr.ms_h2d += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-            guides_up = true;
-        };
-        auto t_h2d0 = std::chrono::steady_clock::now();
+        if (n == 0) { H.hoff[0] = 0; return false; }
+        d_guides = B.alloc<GuideRec>(n); d_pamsets = B.alloc<PamSet>(kMaxPamSets);
+        const auto t_h2d0 = std::chrono::steady_clock::now();
         CK(cudaMemcpyAsync(d_pamsets, prep.pamsets, sizeof(prep.pamsets), cudaMemcpyHostToDevice, s));
-        job->ctr.ms_h2d = 0;
-        if (!late_guides) upload_guides(s);
-
-        uint32_t* d_nmatch = B.alloc<uint32_t>(n + 1, true, s);
-        uint8_t* d_dropped = B.alloc<uint8_t>(n, true, s);
-        uint32_t* d_ctrs = B.alloc<uint32_t>(8, true, s);            // [0] task counter [1] match count [2] error flag
-        unsigned long long* d_stats = B.alloc<unsigned long long>(8, true, s);
-        const int variant_n = env_int("GSX_SEARCH_VARIANT", 0), variant_w = env_int("GSX_SEARCH_VARIANT_WIDE", 0);
-
-        SearchArgs a{};
+        job.ctr.ms_h2d = 0;
+        if (!plan.late_guides) upload_guides(s);
+        d_nmatch = B.alloc<uint32_t>(n + 1, true, s); d_dropped = B.alloc<uint8_t>(n, true, s);
+        d_ctrs = B.alloc<uint32_t>(8, true, s); d_stats = B.alloc<unsigned long long>(8, true, s);
         a.st[0] = di.st[0].d; a.st[1] = di.st[1].d; a.guides = d_guides; a.pamsets = d_pamsets;
         a.task_counter = d_ctrs + 0; a.match_count = d_ctrs + 1; a.error_flag = d_ctrs + 2; a.stats = d_stats;
-        a.guide_nmatch = d_nmatch; a.max_iters = 1u << 28; a.max_pams = prep.max_pams;
-        a.p.n_tasks = 2 * n;
-        const int variant_f = env_int("GSX_FAST_VARIANT", di.st[0].d.lines ? 1 : 0);
-        if (use_fast) {
+        a.guide_nmatch = d_nmatch; a.max_iters = 1u << 28; a.max_pams = prep.max_pams; a.p.n_tasks = 2 * n;
+        if (plan.use_fast) {
             uint64_t* d_gq = B.alloc<uint64_t>(n);
-            CK(cudaMemcpyAsync(d_gq, prep.gq.data() + job->g0, (size_t)n * 8, cudaMemcpyHostToDevice, s));
-            if (late_guides) job->ctr.ms_h2d += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_h2d0).count();
+            CK(cudaMemcpyAsync(d_gq, prep.gq.data() + job.g0, (size_t)n * 8, cudaMemcpyHostToDevice, s));
+            if (plan.late_guides) job.ctr.ms_h2d += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_h2d0).count();
             a.gq = d_gq; a.pampack = prep.pampack; a.plen = prep.plen;
-            a.exc = exc_index ? 1u : 0u; a.exc_map[0] = (const uint32_t*)di.st[0].exc_map; a.exc_map[1] = (const uint32_t*)di.st[1].exc_map;
-            // L2 residency hint: intervals wide enough that all such blocks of both strands fit the L2 budget
-            // (a level-d interval end costs one 128-byte line; lines touched down to level D ~ 2.7 * 4^D per strand)
-            const double l2_bytes = (double)env_int("GSX_L2_PIN_MB", 64) * 1e6;
-            const double w = l2_bytes > 0 ? (double)di.st[0].d.n * 2.0 * 2.7 * 128.0 / l2_bytes : 4.0e9;
-            a.pin_width = w >= 4.0e9 ? 0xFFFFFFFFu : (uint32_t)std::max(256.0, w);
-            a.combos = nullptr; a.n_combos = 0;
+            a.exc = plan.exc ? 1u : 0u; a.exc_map[0] = (const uint32_t*)di.st[0].exc_map; a.exc_map[1] = (const uint32_t*)di.st[1].exc_map;
+            a.pin_width = plan.pin_width; a.combos = nullptr; a.n_combos = 0;
         }
-        // slice-major front end (sweep_kernel) for large batches: needs the jump table and the look-ahead lines
-        const uint32_t ftab_L = di.st[0].d.ftab_L;
-        // slice width (characters) for a batch of ng guides no shorter than min_qlen, 0 = no sweep
-        auto plan_sweep = [&](uint32_t ng, uint32_t min_qlen, uint32_t M) -> uint32_t {
-            bool ok = use_fast && ftab_L >= 6 && di.st[1].d.ftab_L == ftab_L && di.st[0].d.sum0 && di.st[1].d.sum0 && env_int("GSX_SWEEP", 1) &&
-                      ng >= (uint32_t)env_int("GSX_SWEEP_MIN", 8192) && min_qlen >= ftab_L && M <= 4;
-            if (!ok) return 0;
-            const double per_strand = 40.0 * std::pow(4.0, (double)ftab_L);                  // sum0 + the part of sum1 that is touched
-            const double target = (double)env_int("GSX_SWEEP_SLICE_MB", 12) * 1e6;
-            uint32_t sb = 1; while (sb < ftab_L - 3 && per_strand / std::pow(4.0, (double)sb) > target) sb++;
-            if (env_int("GSX_SWEEP_SB", 0) > 0) sb = (uint32_t)env_int("GSX_SWEEP_SB", 0);
-            if (sb < 1 || sb + 3 > ftab_L) return 0;
-            if (2.0 * std::pow(4.0, (double)sb) * ((ng + 31) / 32) * 8.0 >= 4.0e9) return 0;
-            return sb;
-        };
-        const uint32_t sweep_sb = use_variants ? 0u : plan_sweep(n, prep.min_qlen, std::max<uint32_t>(p.mismatches, p.threshold > 0 ? (uint32_t)p.threshold : 0u));
-        bool use_sweep = sweep_sb != 0;
-        // seed queue of the sweep: 12 survivors per guide measured at m = 3 on 3.1 Gb (two orders of magnitude more at m = 4);
-        // sized with a wide margin, never beyond the 32-bit slot numbers the kernels use; an overflow is retried with 4x the room
-        uint64_t queue_cap = std::max<uint64_t>((uint64_t)n * (p.mismatches >= 4 ? 1024 : 256), 1u << 20);
-        queue_cap = std::min<uint64_t>(queue_cap, 1ull << 30);
-        if (env_int("GSX_QUEUE_CAP", 0) > 0) queue_cap = (uint64_t)env_int("GSX_QUEUE_CAP", 0);
-        SeedNode* d_queue = nullptr;
-        uint64_t n_launches = 0;
-        uint32_t* d_xtab = nullptr; uint32_t xtab_M = ~0u, xtab_sb = 0, n_xtab = 0; SweepPlan xplan{};
-        uint32_t* d_gtab = nullptr; size_t gtab_cap = 0;
-        // Two-part enumeration (sweep_split_kernel, GSX_SPLIT=0 turns it off): 20-nt guides, one PAM of the form N + two concrete
-        // characters, at most 3 mismatches, an index without N, no --start, no threshold pass, and a jump table deep enough to hold
-        // both capped halves (13 characters: the PAM and the proximal half of the PAM-first form; with fewer, that form would hand the
-        // tree search alignments with two proximal mismatches only for the re-anchoring to drop them).  Per guide and strand a quarter
-        // of the summary sectors of the plain sweep.
-        const uint32_t split_half = 10;
-        const bool split_ok = sweep_sb != 0 && !use_variants && p.threshold <= 0 && !p.start && prep.n_fast_pams == 1 && prep.plen == 3 &&
-                              (prep.pampack & 7u) == 4u && ((prep.pampack >> 3) & 7u) < 4u && ((prep.pampack >> 6) & 7u) < 4u &&
-                              prep.min_qlen == 2 * split_half && prep.max_qlen == 2 * split_half && p.mismatches <= kSplitMaxM && plain_index &&
-                              ftab_L >= prep.plen + split_half && n < (1u << 22) && env_int("GSX_SPLIT", 1) != 0;
-        // slices one character wider than the plain sweep's: a quarter of the patterns per guide, so four times the slice keeps the
-        // patterns per work unit up (3.1 Gb, 200 k guides, one B200: sweep 13.0 ms at sb = 4 against 15.9 at 5 and 15.7 at 3,
-        // profiles/r03a_split_ab_3100mb_200k.jsonl)
-        const uint32_t split_sb = split_ok && env_int("GSX_SPLIT_SB", 0) > 0 ? (uint32_t)env_int("GSX_SPLIT_SB", 0) : (sweep_sb > 1 ? sweep_sb - 1 : sweep_sb);
-        uint32_t* d_sxtab = nullptr; uint32_t n_sxtab = 0; SplitPlan splan{};
-        uint64_t* d_gq2 = nullptr; SeedNode* d_queue2 = nullptr; uint64_t queue2_cap = 0;
-        MatchRec* d_matches2 = nullptr; uint64_t matches2_cap = 0; uint32_t* d_nmatch2 = nullptr;
-        uint32_t* d_ctrs2 = split_ok ? B.alloc<uint32_t>(4, true, s) : nullptr;      // [0] form-1 seed count [1] task counter [2] form-1 match count
-        bool split_ran = false;
-        // fast path launch over ng guides (m.gq): [sweep_kernel ->] search_fast_kernel.  d_ctrs: [3] seed queue count, [4] sweep work-unit counter
-        uint32_t lean_qmin = prep.min_qlen, lean_qmax = prep.max_qlen;              // guide lengths of the batch the fast kernels see (edited guides: - R .. + D)
-        auto launch_split = [&](SearchArgs& m, uint32_t ng, cudaEvent_t ev_mid) {
-            const uint32_t sb = split_sb;
-            if (!d_sxtab) {
-                std::vector<uint32_t> xtab;
-                split_make_plan(ftab_L, sb, m.p.M, 2 * split_half, prep.plen, prep.pampack, split_half, splan, xtab);
-                if (xtab.size() > (size_t)kSplitXtabShared) throw std::runtime_error("two-part enumeration: xor table too long for this slice width");
-                n_sxtab = (uint32_t)xtab.size();
-                d_sxtab = B.alloc<uint32_t>(xtab.size());
-                CK(cudaMemcpyAsync(d_sxtab, xtab.data(), xtab.size() * 4, cudaMemcpyHostToDevice, s)); CK(cudaStreamSynchronize(s));
-                d_gq2 = B.alloc<uint64_t>(ng); d_nmatch2 = B.alloc<uint32_t>(ng + 1);
-                CK(launch_split_queries(m.gq, ng, prep.pampack, prep.plen, d_gq2, s)); n_launches++;
-            }
-            if (!d_queue) d_queue = B.alloc<SeedNode>(queue_cap);
-            if (queue2_cap != queue_cap) { if (d_queue2) B.free_one(d_queue2); d_queue2 = B.alloc<SeedNode>(queue_cap); queue2_cap = queue_cap; }
-            if (matches2_cap < m.p.match_cap) { if (d_matches2) B.free_one(d_matches2); d_matches2 = B.alloc<MatchRec>(m.p.match_cap); matches2_cap = m.p.match_cap; }
-            CK(cudaMemsetAsync(d_ctrs2, 0, 4 * sizeof(uint32_t), s));
-            SweepArgs w{};
-            w.plan.L = ftab_L; w.plan.sb = sb; w.plan.M = m.p.M; w.split = splan;
-            w.st[0] = m.st[0]; w.st[1] = m.st[1]; w.gq = m.gq; w.gq2 = d_gq2; w.skip = m.skip; w.n_guides = ng; w.xtab = d_sxtab; w.n_xtab = n_sxtab;
-            w.M = m.p.M; w.plen = m.plen; w.pampack = m.pampack;
-            w.queue = d_queue; w.queue_cap = (uint32_t)queue_cap; w.queue_count = d_ctrs + 3; w.item_counter = d_ctrs + 4;
-            w.queue2 = d_queue2; w.queue2_count = d_ctrs2 + 0;
-            w.error_flag = d_ctrs + 2; w.stats = d_stats;
-            if (gtab_cap < 2 * (size_t)ng) { if (d_gtab) B.free_one(d_gtab); d_gtab = B.alloc<uint32_t>((size_t)ng * 40); gtab_cap = 2 * (size_t)ng; }
-            w.gtab = d_gtab;
-            CK(launch_sweep_guides(w, s)); n_launches++;                          // rows 0 .. ng-1: form 0
-            SweepArgs w1 = w; w1.gq = d_gq2; w1.plen = 0; w1.pampack = 0; w1.gtab = d_gtab + (size_t)ng * 20;
-            CK(launch_sweep_guides(w1, s)); n_launches++;                         // rows ng .. 2ng-1: form 1
-            CK(launch_sweep_split(w, env_int("GSX_SPLIT_CTAS", 6), di.sm_count, s)); n_launches++;
-            if (ev_mid) CK(cudaEventRecord(ev_mid, s));
-            m.seeds = d_queue; m.n_seeds = d_ctrs + 3; m.seed_cap = (uint32_t)queue_cap; m.combos = nullptr; m.n_combos = 0;
-            CK(launch_search_fast(m, variant_f, di.sm_count, s)); n_launches++;
-            // form 1: the tree search of its seeds with the PAM-first query (all of it protospacer), into an arena of its own
-            SearchArgs m1 = m;
-            m1.gq = d_gq2; m1.plen = 0; m1.pampack = 0; m1.seeds = d_queue2; m1.n_seeds = d_ctrs2 + 0;
-            m1.task_counter = d_ctrs2 + 1; m1.match_count = d_ctrs2 + 2; m1.matches = d_matches2; m1.guide_nmatch = d_nmatch2;
-            CK(launch_search_fast(m1, variant_f, di.sm_count, s)); n_launches++;
-            ReanchorArgs r{};
-            r.st[0] = m.st[0]; r.st[1] = m.st[1]; r.in = d_matches2; r.n_in = d_ctrs2 + 2; r.in_cap = m.p.match_cap;
-            r.gq = m.gq; r.gq2 = d_gq2; r.pampack = prep.pampack; r.plen = prep.plen;
-            r.out = m.matches; r.out_count = m.match_count; r.out_cap = m.p.match_cap; r.guide_nmatch = m.guide_nmatch; r.error_flag = m.error_flag;
-            r.stats = d_stats;
-            CK(launch_reanchor(r, s)); n_launches++;
-            split_ran = true;
-        };
-        auto launch_fast = [&](SearchArgs& m, uint32_t ng, uint32_t sb, cudaEvent_t ev_mid) {
-            if (sb && split_ok && !m.p.counting && !m.fmask) { launch_split(m, ng, ev_mid); return; }
-            if (sb) {
-                SweepArgs w{};
-                if (xtab_M != m.p.M || xtab_sb != sb) {
-                    std::vector<uint32_t> xtab;
-                    sweep_make_plan(ftab_L, sb, m.p.M, xplan, xtab);
-                    if (d_xtab) B.free_one(d_xtab);
-                    n_xtab = (uint32_t)xtab.size(); xtab_M = m.p.M; xtab_sb = sb;
-                    xtab.resize(xtab.size() + 64, 0u);                                // (sweep_lean_kernel reads up to 63 words past a pass's end, unused)
-                    d_xtab = B.alloc<uint32_t>(xtab.size());
-                    CK(cudaMemcpyAsync(d_xtab, xtab.data(), xtab.size() * 4, cudaMemcpyHostToDevice, s)); CK(cudaStreamSynchronize(s));
-                }
-                w.plan = xplan;
-                if (!d_queue) d_queue = B.alloc<SeedNode>(queue_cap);
-                w.st[0] = m.st[0]; w.st[1] = m.st[1]; w.gq = m.gq; w.skip = m.skip; w.n_guides = ng; w.xtab = d_xtab; w.n_xtab = n_xtab;
-                w.M = m.p.M; w.plen = m.plen; w.pampack = m.pampack; w.load_mode = (uint32_t)env_int("GSX_SWEEP_LOAD", 2);
-                w.parts = 1;                                                       // measured: cutting the units does not pay (profiles/r01r_*)
-                w.queue = d_queue; w.queue_cap = (uint32_t)queue_cap; w.queue_count = d_ctrs + 3; w.item_counter = d_ctrs + 4;
-                w.error_flag = d_ctrs + 2; w.stats = d_stats; w.fmask = m.fmask;
-                if (gtab_cap < ng) { if (d_gtab) B.free_one(d_gtab); d_gtab = B.alloc<uint32_t>((size_t)ng * 20); gtab_cap = ng; }
-                w.gtab = d_gtab;
-                CK(launch_sweep_guides(w, s)); n_launches++;
-                // sweep_lean_kernel (variants 10-12) where its compiled loops cover the batch: at most 4 mismatches, every guide length
-                // of the batch giving one of its plane layouts
-                // measured at 3.1 Gb (profiles/r02c_session_3100mb_sweep_lean3.jsonl): six CTAs per SM (variant 12) for plain batches of
-                // at most 3 mismatches -- 24.0 ms per 200 k guides against 36.6 for sweep_kernel --, five (variant 11) for 4 mismatches
-                // and for the edited guides of a bulge search
-                int sv = env_int("GSX_SWEEP_VARIANT", (m.p.M <= 3 && !m.fmask && !use_variants) ? 12 : 11);
-                if (sv >= 10) {
-                    bool lean_ok = m.p.M <= 4;
-                    for (uint32_t ql = lean_qmin; lean_ok && ql <= lean_qmax; ql++)
-                        lean_ok = sweep_shape_of(sweep_codes((uint64_t)ql << 58, ftab_L, m.plen, m.pampack)) >= 0;
-                    if (!lean_ok) sv = 2;
-                }
-                CK(launch_sweep(w, sv, di.sm_count, s)); n_launches++;
-                m.seeds = d_queue; m.n_seeds = d_ctrs + 3; m.seed_cap = (uint32_t)queue_cap; m.combos = nullptr; m.n_combos = 0;
-            }
-            if (ev_mid) CK(cudaEventRecord(ev_mid, s));
-            CK(launch_search_fast(m, variant_f, di.sm_count, s)); n_launches++;
-        };
-        // alternative PAMs (process.hpp:51-56): the searches of the PAMs are independent and their matches are collected in
-        // the same per-guide sets, so each PAM gets its own pass over the same arenas; only the work counters start over
-        // Default (GSX_FUSED_PAMS=0 keeps one pass per PAM; m = 4 with NGG + NAG at 3.1 Gb: 232 k against 142 k guides/s, same text): the PAMs in
-        // ONE pass -- search with the filter PAM, keep the alignments whose PAM characters spell a real PAM (gsx_core.h fused_pam_ok)
-        const bool fuse_pams = prep.n_fast_pams > 1 && variant_f == 1 && env_int("GSX_FUSED_PAMS", 1) != 0;
-        auto run_fast_all_pams = [&](SearchArgs& m, uint32_t ng, uint32_t sb, cudaEvent_t ev_mid) {
-            m.n_fused = 0;
-            if (fuse_pams && !m.p.counting) {
-                m.n_fused = prep.n_fast_pams;
-                for (uint32_t k = 0; k < prep.n_fast_pams; k++) m.fused_pams[k] = prep.pampacks[k];
-                m.plen = prep.plens[0]; m.pampack = fused_filter_pampack(prep.pampacks, prep.n_fast_pams, prep.plens[0]);
-                launch_fast(m, ng, sb, ev_mid);
-                return;
-            }
-            for (uint32_t k = 0; k < prep.n_fast_pams; k++) {
-                m.pampack = prep.pampacks[k]; m.plen = prep.plens[k];
-                if (k) { CK(cudaMemsetAsync(d_ctrs, 0, 4, s)); CK(cudaMemsetAsync(d_ctrs + 3, 0, 8, s)); }      // task / seed-queue / work-unit counters
-                launch_fast(m, ng, sb, k == 0 ? ev_mid : nullptr);
-            }
-        };
-        auto grow_queue = [&]() { B.free_one(d_queue); d_queue = nullptr; queue_cap *= 4; if (queue_cap >= (1ull << 32)) throw std::runtime_error("seed queue keeps overflowing"); };
-
-        // Calls from several host threads (the reference's own worker threads, or gsx_enumerate_start) take turns on a device from the
-        // first search launch to the last result copy (gsx::device_turn).
-        std::unique_lock<std::mutex> turn = gsx::device_turn(di.device);
-        CK(cudaEventRecord(ev[0], s));
-        // ---- threshold prefilter (process.hpp:66-76): mismatch-only counting search, guide dropped if > 1 site -----
-        if (p.threshold > 0) {
-            unsigned long long* d_gcount = B.alloc<unsigned long long>(n, true, s);
-            uint32_t spill_cap = 4096;
-            for (;;) {
-                int warps = use_fast ? search_fast_grid_warps(variant_f, di.sm_count) : search_grid_warps(false, variant_n, di.sm_count);
-                if (warps <= 0) throw std::runtime_error("unknown search kernel variant");
-                uint32_t* d_spill = B.alloc<uint32_t>((size_t)warps * spill_cap * 6);
-                CK(cudaMemsetAsync(d_ctrs, 0, 8 * sizeof(uint32_t), s));
-                CK(cudaMemsetAsync(d_gcount, 0, (size_t)n * 8, s));
-                SearchArgs c = a; c.p.M = (uint32_t)p.threshold; c.p.R = c.p.D = 0; c.p.counting = 1; c.p.match_cap = 0; c.p.spill_cap = spill_cap;
-                const uint32_t sb_thr = plan_sweep(n, prep.min_qlen, c.p.M);
-                if (use_fast && ftab_L && !sb_thr) {
-                    std::vector<uint64_t> cb = ftab_combos(ftab_L - 2, c.p.M);
-                    uint64_t* d_cb = B.alloc<uint64_t>(cb.size());
-                    CK(cudaMemcpyAsync(d_cb, cb.data(), cb.size() * 8, cudaMemcpyHostToDevice, s)); CK(cudaStreamSynchronize(s));
-                    c.combos = d_cb; c.n_combos = (uint32_t)cb.size();
-                }
-                c.guide_count = d_gcount; c.spill = d_spill; c.skip = nullptr; c.matches = nullptr;
-                if (use_fast) run_fast_all_pams(c, n, sb_thr, nullptr); else { CK(launch_search(c, false, variant_n, di.sm_count, s, nullptr)); n_launches++; }
-                upload_guides(s2);
-                uint32_t h[3]; read_ctrs(h, 3, d_ctrs); n_launches++;
-                B.free_one(d_spill);
-                if (h[2] & GSX_KERR_WATCHDOG) throw std::runtime_error("search kernel watchdog tripped");
-                if (h[2] & GSX_KERR_QUEUE_OVERFLOW) { grow_queue(); if (h[2] & GSX_KERR_SPILL_OVERFLOW) spill_cap *= 4; continue; }
-                if (h[2] & GSX_KERR_SPILL_OVERFLOW) { spill_cap *= 4; continue; }
-                break;
-            }
-            CK(launch_threshold(d_gcount, d_dropped, n, s)); n_launches++;
-            unsigned long long zero[8] = {0}; CK(cudaMemcpyAsync(d_stats, zero, sizeof zero, cudaMemcpyHostToDevice, s));
-        }
-        // ---- main search ---------------------------------------------------------------------------------------------
-        const bool wide = prep.wide;
-        const int variant = wide ? variant_w : variant_n;
-        // Match arena: an overflow costs a second run of the whole search, so the first size has to be right.  Expected matches per
-        // guide on a genome without structure = 2 strands x rows x (substitution patterns within the budget) / 4^length x the fraction
-        // of sites a PAM list accepts: 11 at 3 mismatches / NGG on 3.1 Gb, 300 at 4 mismatches with NGG + NAG (the size round 1 got
-        // wrong: n x 48 -- every such call searched twice).  What a call actually needed is remembered per index and option set and
-        // serves as the floor for the next call (real genomes have repeats that no formula knows).
-        const uint64_t learn_key = (uint64_t)p.mismatches | ((uint64_t)prep.n_fast_pams << 8) | ((uint64_t)p.rna_bulges << 16) | ((uint64_t)p.dna_bulges << 24) |
-                                   ((uint64_t)prep.min_qlen << 32) | ((uint64_t)(wide ? 1 : 0) << 40);
-        double per_guide = wide ? 2048.0 : 48.0;
-        if (!wide) {
-            const double ql = (double)std::max<uint32_t>(prep.min_qlen, 1);
-            double patterns = 0, c = 1;                                           // sum over j <= M of C(q, j) 3^j
-            for (uint32_t j = 0; j <= p.mismatches && j <= prep.min_qlen; j++) { patterns += c; c = c * 3.0 * (ql - j) / (j + 1.0); }
-            double pam_frac = 0;
-            for (int ps = 0; ps < kMaxPamSets; ps++) {
-                double f = 0;
-                for (int k = 0; k < prep.pamsets[ps].n_pams; k++) { double g1 = 1; for (int j = 0; j < prep.pamsets[ps].plen[k]; j++) if (prep.pamsets[ps].sym[k][j] != SYM_N) g1 *= 0.25; f += g1; }
-                pam_frac = std::max(pam_frac, std::min(1.0, f));
-            }
-            const double expect = 2.0 * (double)di.st[0].d.n * patterns / std::pow(4.0, ql) * pam_frac;
-            per_guide = std::max(per_guide, 1.5 * expect + 8.0);
-        }
-        {
-            std::lock_guard<std::mutex> lk(job->ix->learn_mu);
-            auto it = job->ix->learned_matches_per_guide.find(learn_key);
-            if (it != job->ix->learned_matches_per_guide.end()) per_guide = std::max(per_guide, 1.25 * it->second);
-        }
-        uint64_t match_cap = std::max<uint64_t>((uint64_t)((double)n * per_guide), 1u << 18);
-        match_cap = std::min<uint64_t>(match_cap, 1u << 27);
-        uint32_t spill_cap = wide ? 8192 : 2048;
-        if (env_int("GSX_MATCH_CAP", 0) > 0) match_cap = (uint64_t)env_int("GSX_MATCH_CAP", 0);      // tests: force the retry path
-        if (env_int("GSX_SPILL_CAP", 0) > 0) spill_cap = (uint32_t)env_int("GSX_SPILL_CAP", 0);
-        MatchRec* d_matches = nullptr; uint32_t* d_spill = nullptr; uint32_t n_matches = 0, n_seeds_used = 0;
-        if (use_fast && ftab_L && (!use_sweep || use_variants)) {
-            std::vector<uint64_t> cb = ftab_combos(ftab_L - 2, p.mismatches);
-            uint64_t* d_cb = B.alloc<uint64_t>(cb.size());
-            CK(cudaMemcpyAsync(d_cb, cb.data(), cb.size() * 8, cudaMemcpyHostToDevice, s)); CK(cudaStreamSynchronize(s));
-            a.combos = d_cb; a.n_combos = (uint32_t)cb.size();
-        }
-        if (use_variants) {
-            // ---- bulges as edited guides: chunks of guides whose edited forms fill one launch of the specialised kernels ----
-            const uint32_t R = p.rna_bulges, D = p.dna_bulges;
-            std::vector<uint32_t> descs, doff(kMaxQ + 2, 0), dcnt(kMaxQ + 2, 0);
-            for (uint32_t ql = prep.min_qlen; ql <= prep.max_qlen; ql++) {
-                const std::vector<uint32_t> v = bulge_variants(ql, R, D);
-                doff[ql] = (uint32_t)descs.size(); dcnt[ql] = (uint32_t)v.size(); descs.insert(descs.end(), v.begin(), v.end());
-            }
-            uint32_t* d_descs = B.alloc<uint32_t>(descs.size()); uint32_t* d_doff = B.alloc<uint32_t>(doff.size());
-            CK(cudaMemcpyAsync(d_descs, descs.data(), descs.size() * 4, cudaMemcpyHostToDevice, s));
-            CK(cudaMemcpyAsync(d_doff, doff.data(), doff.size() * 4, cudaMemcpyHostToDevice, s));
-            std::vector<uint8_t> h_dropped(n, 0);
-            if (p.threshold > 0) CK(cudaMemcpyAsync(h_dropped.data(), d_dropped, n, cudaMemcpyDeviceToHost, s));
-            CK(cudaStreamSynchronize(s));
-            const uint32_t chunk_v = (uint32_t)std::min<int64_t>(std::max<int64_t>(env_int("GSX_VARIANT_CHUNK", 262144), 1), (1 << 22));
-            const uint32_t vmin_qlen = prep.min_qlen > R ? prep.min_qlen - R : 0;
-            lean_qmin = vmin_qlen; lean_qmax = prep.max_qlen + D;
-            const int warps = search_fast_grid_warps(variant_f, di.sm_count);
-            if (warps <= 0) throw std::runtime_error("unknown search kernel variant");
-            if (d_queue) { B.free_one(d_queue); d_queue = nullptr; }               // (sized by the threshold pass)
-            queue_cap = std::max<uint64_t>((uint64_t)chunk_v * 256, 1u << 20);
-            if (env_int("GSX_QUEUE_CAP", 0) > 0) queue_cap = (uint64_t)env_int("GSX_QUEUE_CAP", 0);
-            uint64_t vmatch_cap = std::max<uint64_t>((uint64_t)chunk_v * 48, 1u << 18);
-            match_cap = std::max<uint64_t>(1u << 18, std::min<uint64_t>((uint64_t)n * dcnt[prep.max_qlen] * 12, 1u << 26));
-            if (env_int("GSX_MATCH_CAP", 0) > 0) vmatch_cap = match_cap = (uint64_t)env_int("GSX_MATCH_CAP", 0);
-            spill_cap = 2048; if (env_int("GSX_SPILL_CAP", 0) > 0) spill_cap = (uint32_t)env_int("GSX_SPILL_CAP", 0);
-            uint64_t* d_vq = B.alloc<uint64_t>(chunk_v + 1); uint32_t* d_vdesc = B.alloc<uint32_t>(chunk_v + 1); uint32_t* d_vguide = B.alloc<uint32_t>(chunk_v + 1);
-            uint32_t* d_vnmatch = B.alloc<uint32_t>(chunk_v + 1);
-            // the sweep skips patterns that substitute an inserted position (GSX_FORCED_SWEEP=0: it tests them and the rewrite drops their
-            // matches; 11 % fewer seeds, 1.4 % less search time at 3.1 Gb)
-            uint32_t* d_vfmask = env_int("GSX_FORCED_SWEEP", 1) ? B.alloc<uint32_t>(chunk_v + 1) : nullptr;
-            uint32_t* d_voff = nullptr; size_t voff_cap = 0;
-            MatchRec* d_vmatches = B.alloc<MatchRec>(vmatch_cap);
-            d_matches = B.alloc<MatchRec>(match_cap);
-            CK(cudaMemsetAsync(d_ctrs, 0, 8 * sizeof(uint32_t), s));             // [5]: matches in the final arena
-            CK(cudaMemsetAsync(d_nmatch, 0, (size_t)(n + 1) * 4, s));
-            CK(cudaMemsetAsync(d_stats, 0, 8 * sizeof(unsigned long long), s));
-            CK(cudaEventRecord(ev[6], s)); CK(cudaEventRecord(ev[7], s));
-            std::vector<uint32_t> seg;                                             // {first edited guide, guide, first op list} per segment
-            uint32_t n_final = 0;
-            uint32_t c0 = 0, f0 = 0;                                               // next guide, and how many of its op lists are done
-            while (c0 < n) {
-                // as many guides as fit the chunk; a guide with more edited forms than a chunk holds is cut into runs of op lists;
-                // guides dropped by the threshold pass have no edited forms
-                seg.clear(); uint32_t n_v = 0;
-                while (c0 < n && n_v < chunk_v) {
-                    const uint32_t cnt = h_dropped[c0] ? 0u : dcnt[prep.recs[job->g0 + c0].qlen];
-                    const uint32_t take = std::min<uint32_t>(cnt - f0, chunk_v - n_v);
-                    if (take) { seg.push_back(n_v); seg.push_back(c0); seg.push_back(f0); n_v += take; }
-                    f0 += take;
-                    if (f0 == cnt) { c0++; f0 = 0; } else break;                   // chunk full in the middle of a guide
-                }
-                const uint32_t n_seg = (uint32_t)(seg.size() / 3);
-                seg.push_back(n_v);
-                job->ctr.edited_guides += n_v;
-                if (n_v) {
-                    if (voff_cap < seg.size()) { if (d_voff) B.free_one(d_voff); voff_cap = std::max<size_t>(seg.size(), 4096); d_voff = B.alloc<uint32_t>(voff_cap); }
-                    CK(cudaMemcpyAsync(d_voff, seg.data(), seg.size() * 4, cudaMemcpyHostToDevice, s));
-                    CK(launch_variant_expand(d_guides, n_seg, n_v, d_voff, d_descs, d_doff, d_vq, d_vdesc, d_vguide, d_vfmask, s)); n_launches++;
-                    const uint32_t sb = plan_sweep(n_v, vmin_qlen, p.mismatches);
-                    if (sb) use_sweep = true;
-                    for (int attempt = 0;; attempt++) {
-                        if (attempt > 12) throw std::runtime_error("search arenas keep overflowing");
-                        d_spill = B.alloc<uint32_t>((size_t)warps * spill_cap * 6);
-                        CK(cudaMemsetAsync(d_ctrs, 0, 5 * sizeof(uint32_t), s));
-                        SearchArgs m = a; m.p.M = p.mismatches; m.p.R = m.p.D = 0; m.p.counting = 0; m.p.n_tasks = 2 * n_v;
-                        m.p.match_cap = (uint32_t)vmatch_cap; m.p.spill_cap = spill_cap; m.spill = d_spill; m.matches = d_vmatches;
-                        m.skip = nullptr; m.gq = d_vq; m.guide_nmatch = d_vnmatch; m.guides = nullptr; m.fmask = d_vfmask;
-                        run_fast_all_pams(m, n_v, sb, nullptr);
-                        uint32_t h[4]; read_ctrs(h, 4, d_ctrs); n_launches++;
-                        B.free_one(d_spill);
-                        if (h[2] & GSX_KERR_WATCHDOG) throw std::runtime_error("search kernel watchdog tripped");
-                        if (h[2] & (GSX_KERR_MATCH_OVERFLOW | GSX_KERR_SPILL_OVERFLOW | GSX_KERR_QUEUE_OVERFLOW)) {
-                            if (h[2] & GSX_KERR_QUEUE_OVERFLOW) grow_queue();
-                            if (h[2] & GSX_KERR_MATCH_OVERFLOW) {
-                                B.free_one(d_vmatches); vmatch_cap = std::max<uint64_t>(vmatch_cap * 2, (uint64_t)h[1] + (h[1] >> 2));
-                                if (vmatch_cap > (1ull << 31)) throw std::runtime_error("more than 2^31 matches in one chunk; lower GSX_VARIANT_CHUNK");
-                                d_vmatches = B.alloc<MatchRec>(vmatch_cap);
-                            }
-                            if (h[2] & GSX_KERR_SPILL_OVERFLOW) spill_cap *= 4;
-                            continue;
-                        }
-                        n_seeds_used += sb ? h[3] : 0;
-                        // room for every match of the chunk in the final arena, then rewrite (cannot overflow any more)
-                        if ((uint64_t)n_final + h[1] > match_cap) {
-                            const uint64_t cap2 = std::max<uint64_t>(match_cap * 2, ((uint64_t)n_final + h[1]) * 2);
-                            if (cap2 > (1ull << 31)) throw std::runtime_error("more than 2^31 matches in one batch; lower the batch size");
-                            MatchRec* bigger = B.alloc<MatchRec>(cap2);
-                            CK(cudaMemcpyAsync(bigger, d_matches, (size_t)n_final * sizeof(MatchRec), cudaMemcpyDeviceToDevice, s));
-                            CK(cudaStreamSynchronize(s));
-                            B.free_one(d_matches); d_matches = bigger; match_cap = cap2;
-                        }
-                        CK(launch_variant_rewrite(d_vmatches, h[1], d_guides, d_vdesc, d_vguide, d_matches, (uint32_t)match_cap, d_ctrs + 5, d_nmatch, d_ctrs + 2, s));
-                        n_launches++;
-                        read_ctrs(&n_final, 1, d_ctrs + 5); n_launches++;
-                        break;
-                    }
-                }
-            }
-            n_matches = n_final;
-        } else {
-        Node* d_gseeds = nullptr; uint32_t n_gseeds = 0;
-        if (!use_fast && env_int("GSX_EXPAND_ROOTS", 1)) {
-            const int gw = search_grid_warps(wide, variant, di.sm_count);
-            if (gw > 0 && (uint64_t)2 * n < (uint64_t)4 * gw) {                     // fewer tasks than the grid can keep busy
-                const std::vector<Node> gs = wide ? expand_roots<true>(job->ix, prep, job->g0, n, p.mismatches, p.rna_bulges, p.dna_bulges, (size_t)8 * gw, 6)
-                                                  : expand_roots<false>(job->ix, prep, job->g0, n, p.mismatches, p.rna_bulges, p.dna_bulges, (size_t)8 * gw, 6);
-                if (gs.size() > (size_t)2 * n) {
-                    d_gseeds = B.alloc<Node>(gs.size()); n_gseeds = (uint32_t)gs.size();
-                    CK(cudaMemcpyAsync(d_gseeds, gs.data(), gs.size() * sizeof(Node), cudaMemcpyHostToDevice, s)); CK(cudaStreamSynchronize(s));
-                }
-            }
-        }
+        if (plan.split) sp.ctrs2 = B.alloc<uint32_t>(4, true, s);
+        sw.queue_cap = plan.queue_cap; qmin = prep.min_qlen; qmax = prep.max_qlen; use_sweep = plan.search_sb != 0;
+        turn = gsx::device_turn(di.device);
+        CK(cudaEventRecord(js.ev[kSearchBegin], s));
+        return true;
+    }
+    // One search, run until its arenas hold everything it finds.  Each attempt gets a spill stack for the grid, runs `launch` (the
+    // caller's counter resets and launches) and reads d_ctrs[0..3] back into h.  On an overflow the arenas grow -- seed queue x4,
+    // match arena to max(2x, 1.25x what the search asked for), spill stack x4 -- and the search runs again, at most 12 times more.
+    // The grown sizes stay with the caller for its later searches.
+    template <class F> void search_until_fits(int warps, uint32_t spill_words, uint32_t& spill_cap, MatchArena* arena, uint32_t h[4], F&& launch) {
         for (int attempt = 0;; attempt++) {
             if (attempt > 12) throw std::runtime_error("search arenas keep overflowing");
-            int warps = use_fast ? search_fast_grid_warps(variant_f, di.sm_count) : search_grid_warps(wide, variant, di.sm_count);
             if (warps <= 0) throw std::runtime_error("unknown search kernel variant");
-            d_matches = B.alloc<MatchRec>(match_cap);
-            d_spill = B.alloc<uint32_t>((size_t)warps * spill_cap * (wide ? 8 : 6));
+            uint32_t* d_spill = B.alloc<uint32_t>((size_t)warps * spill_cap * spill_words);
+            launch(d_spill);
+            read_ctrs(h, 4, d_ctrs); n_launches++;
+            B.free_one(d_spill);
+            if (h[2] & GSX_KERR_WATCHDOG) throw std::runtime_error("search kernel watchdog tripped");
+            if (h[2] & GSX_KERR_REANCHOR) throw std::runtime_error("two-part search: a PAM-first match has no interval in the other index");
+            if (!(h[2] & (GSX_KERR_MATCH_OVERFLOW | GSX_KERR_SPILL_OVERFLOW | GSX_KERR_QUEUE_OVERFLOW))) return;
+            if (h[2] & GSX_KERR_QUEUE_OVERFLOW) { B.free_one(sw.queue); sw.queue = nullptr; sw.queue_cap *= 4; }
+            if (sw.queue_cap >= (1ull << 32)) throw std::runtime_error("seed queue keeps overflowing");
+            if ((h[2] & GSX_KERR_MATCH_OVERFLOW) && arena) {
+                B.free_one(arena->p); arena->cap = std::max<uint64_t>(arena->cap * 2, (uint64_t)h[1] + (h[1] >> 2));
+                if (arena->cap > (1ull << 31)) throw std::runtime_error(arena->too_many);
+                arena->p = B.alloc<MatchRec>(arena->cap);
+            }
+            if (h[2] & GSX_KERR_SPILL_OVERFLOW) spill_cap *= 4;
+        }
+    }
+    // threshold prefilter (process.hpp:66-76): mismatch-only counting search, guide dropped if > 1 site
+    void threshold_pass() {
+        unsigned long long* d_gcount = B.alloc<unsigned long long>(n, true, s);
+        SearchArgs base = a;
+        if (plan.threshold_combos) upload_combos(base, (uint32_t)p.threshold);
+        uint32_t spill_cap = 4096, h[4];
+        search_until_fits(plan.threshold_warps, 6, spill_cap, nullptr, h, [&](uint32_t* d_spill) {           // (counting: no match arena)
+            CK(cudaMemsetAsync(d_ctrs, 0, 8 * sizeof(uint32_t), s));
+            CK(cudaMemsetAsync(d_gcount, 0, (size_t)n * 8, s));
+            SearchArgs c = base; c.p.M = (uint32_t)p.threshold; c.p.R = c.p.D = 0; c.p.counting = 1; c.p.match_cap = 0; c.p.spill_cap = spill_cap;
+            c.guide_count = d_gcount; c.spill = d_spill; c.skip = nullptr; c.matches = nullptr;
+            if (plan.use_fast) run_fast_all_pams(c, n, plan.threshold_sb, nullptr);
+            else LAUNCH(launch_search(c, false, plan.variant_general[0], di.sm_count, s, nullptr));
+            upload_guides(s2);
+        });
+        LAUNCH(launch_threshold(d_gcount, d_dropped, n, s));
+        unsigned long long zero[8] = {0}; CK(cudaMemcpyAsync(d_stats, zero, sizeof zero, cudaMemcpyHostToDevice, s));
+    }
+    // the main search: the batch or its edited guides; then what it needed per guide is remembered for the next call
+    void search() {
+        if (plan.combos) upload_combos(a, p.mismatches);
+        if (plan.use_variants) search_edited(); else search_batch();
+        CK(cudaEventRecord(js.ev[kSearchEnd], s));
+        std::lock_guard<std::mutex> lk(job.ix->learn_mu);
+        double& v = job.ix->learned_matches_per_guide[learn_key];
+        v = std::max(v * 0.9, (double)n_matches / (double)n);                  // (decays, so that one odd batch does not inflate the arenas for good)
+    }
+    // all n guides in one search: sweep, two-part sweep, jump-table combos or the general kernel
+    void search_batch() {
+        const bool wide = prep.wide;
+        double per_guide = plan.match_per_guide;                             // raised to what earlier calls on the index needed
+        {
+            std::lock_guard<std::mutex> lk(job.ix->learn_mu);
+            auto it = job.ix->learned_matches_per_guide.find(learn_key);
+            if (it != job.ix->learned_matches_per_guide.end()) per_guide = std::max(per_guide, 1.25 * it->second);
+        }
+        const uint64_t cap = std::min<uint64_t>(std::max<uint64_t>((uint64_t)((double)n * per_guide), 1u << 18), 1u << 27);
+        MatchArena out{nullptr, plan.match_cap_set ? plan.match_cap_set : cap, "more than 2^31 matches in one batch; lower the batch size"};
+        uint32_t spill_cap = plan.spill_cap;
+        Node* d_gseeds = nullptr; uint32_t n_gseeds = 0;
+        if (plan.expand_roots) {
+            const std::vector<Node> gs = wide ? expand_roots<true>(job.ix, prep, job.g0, n, p.mismatches, p.rna_bulges, p.dna_bulges, plan.expand_roots, 6)
+                                              : expand_roots<false>(job.ix, prep, job.g0, n, p.mismatches, p.rna_bulges, p.dna_bulges, plan.expand_roots, 6);
+            if (gs.size() > (size_t)2 * n) {
+                d_gseeds = B.alloc<Node>(gs.size()); n_gseeds = (uint32_t)gs.size();
+                CK(cudaMemcpyAsync(d_gseeds, gs.data(), gs.size() * sizeof(Node), cudaMemcpyHostToDevice, s)); CK(cudaStreamSynchronize(s));
+            }
+        }
+        out.p = B.alloc<MatchRec>(out.cap);
+        uint32_t h[4];
+        search_until_fits(plan.search_warps, wide ? 8 : 6, spill_cap, &out, h, [&](uint32_t* d_spill) {
             CK(cudaMemsetAsync(d_ctrs, 0, 8 * sizeof(uint32_t), s));
             CK(cudaMemsetAsync(d_nmatch, 0, (size_t)(n + 1) * 4, s));
             CK(cudaMemsetAsync(d_stats, 0, 8 * sizeof(unsigned long long), s));
             SearchArgs m = a; m.p.M = p.mismatches; m.p.R = p.rna_bulges; m.p.D = p.dna_bulges; m.p.counting = 0;
-            m.p.match_cap = (uint32_t)match_cap; m.p.spill_cap = spill_cap; m.spill = d_spill; m.matches = d_matches;
+            m.p.match_cap = (uint32_t)out.cap; m.p.spill_cap = spill_cap; m.spill = d_spill; m.matches = out.p;
             m.skip = p.threshold > 0 ? d_dropped : nullptr;
             m.gseeds = d_gseeds; m.n_gseeds = n_gseeds;
-            CK(cudaEventRecord(ev[6], s));
-            if (use_fast) run_fast_all_pams(m, n, sweep_sb, ev[7]); else { CK(cudaEventRecord(ev[7], s)); CK(launch_search(m, wide, variant, di.sm_count, s, nullptr)); n_launches++; }
+            CK(cudaEventRecord(js.ev[kSweepBegin], s));
+            if (plan.use_fast) run_fast_all_pams(m, n, plan.search_sb, js.ev[kSweepEnd]);
+            else { CK(cudaEventRecord(js.ev[kSweepEnd], s)); LAUNCH(launch_search(m, wide, plan.variant_general[wide], di.sm_count, s, nullptr)); }
             upload_guides(s2);
-            uint32_t h[4]; read_ctrs(h, 4, d_ctrs); n_launches++;
-            B.free_one(d_spill);
-            if (h[2] & GSX_KERR_WATCHDOG) throw std::runtime_error("search kernel watchdog tripped");
-            if (h[2] & GSX_KERR_REANCHOR) throw std::runtime_error("two-part search: a PAM-first match has no interval in the other index");
-            if (h[2] & (GSX_KERR_MATCH_OVERFLOW | GSX_KERR_SPILL_OVERFLOW | GSX_KERR_QUEUE_OVERFLOW)) {
-                B.free_one(d_matches);
-                if (h[2] & GSX_KERR_QUEUE_OVERFLOW) grow_queue();
-                if (h[2] & GSX_KERR_MATCH_OVERFLOW) match_cap = std::max<uint64_t>(match_cap * 2, (uint64_t)h[1] + (h[1] >> 2));
-                if (h[2] & GSX_KERR_SPILL_OVERFLOW) spill_cap *= 4;
-                if (match_cap > (1ull << 31)) throw std::runtime_error("more than 2^31 matches in one batch; lower the batch size");
-                continue;
+        });
+        d_matches = out.p; n_matches = h[1]; n_seeds = use_sweep ? h[3] : 0;
+        if (sp.ran) { uint32_t h1; read_ctrs(&h1, 1, sp.ctrs2); n_seeds += h1; n_launches++; }
+    }
+    // bulges as edited guides: chunks of guides whose edited forms fill one launch of the specialised kernels.  Each chunk's matches
+    // are rewritten into the batch's arena; d_nmatch and d_stats add up over the chunks.
+    void search_edited() {
+        const uint32_t R = p.rna_bulges, D = p.dna_bulges;
+        std::vector<uint32_t> descs, doff(kMaxQ + 2, 0), dcnt(kMaxQ + 2, 0);
+        for (uint32_t ql = prep.min_qlen; ql <= prep.max_qlen; ql++) {
+            const std::vector<uint32_t> v = bulge_variants(ql, R, D);
+            doff[ql] = (uint32_t)descs.size(); dcnt[ql] = (uint32_t)v.size(); descs.insert(descs.end(), v.begin(), v.end());
+        }
+        uint32_t* d_descs = B.alloc<uint32_t>(descs.size()); uint32_t* d_doff = B.alloc<uint32_t>(doff.size());
+        CK(cudaMemcpyAsync(d_descs, descs.data(), descs.size() * 4, cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(d_doff, doff.data(), doff.size() * 4, cudaMemcpyHostToDevice, s));
+        std::vector<uint8_t> h_dropped(n, 0);
+        if (p.threshold > 0) CK(cudaMemcpyAsync(h_dropped.data(), d_dropped, n, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        const uint32_t chunk_v = plan.chunk;
+        qmin = plan.edited_qmin; qmax = plan.edited_qmax;
+        if (sw.queue) { B.free_one(sw.queue); sw.queue = nullptr; }               // (sized by the threshold pass)
+        sw.queue_cap = plan.chunk_queue_cap;
+        uint64_t match_cap = plan.edited_match_cap;
+        uint32_t spill_cap = plan.spill_cap;
+        uint64_t* d_vq = B.alloc<uint64_t>(chunk_v + 1); uint32_t* d_vdesc = B.alloc<uint32_t>(chunk_v + 1); uint32_t* d_vguide = B.alloc<uint32_t>(chunk_v + 1);
+        uint32_t* d_vnmatch = B.alloc<uint32_t>(chunk_v + 1);
+        uint32_t* d_vfmask = plan.fmask ? B.alloc<uint32_t>(chunk_v + 1) : nullptr;
+        uint32_t* d_voff = nullptr; size_t voff_cap = 0;
+        MatchArena chunk{B.alloc<MatchRec>(plan.chunk_match_cap), plan.chunk_match_cap, "more than 2^31 matches in one chunk; lower GSX_VARIANT_CHUNK"};
+        d_matches = B.alloc<MatchRec>(match_cap);
+        CK(cudaMemsetAsync(d_ctrs, 0, 8 * sizeof(uint32_t), s));
+        CK(cudaMemsetAsync(d_nmatch, 0, (size_t)(n + 1) * 4, s));
+        CK(cudaMemsetAsync(d_stats, 0, 8 * sizeof(unsigned long long), s));
+        CK(cudaEventRecord(js.ev[kSweepBegin], s)); CK(cudaEventRecord(js.ev[kSweepEnd], s));
+        std::vector<uint32_t> seg;                                             // {first edited guide, guide, first op list} per segment
+        uint32_t n_final = 0;
+        uint32_t c0 = 0, f0 = 0;                                               // next guide, and how many of its op lists are done
+        while (c0 < n) {
+            // as many guides as fit the chunk; a guide with more edited forms than a chunk holds is cut into runs of op lists;
+            // guides dropped by the threshold pass have no edited forms
+            seg.clear(); uint32_t n_v = 0;
+            while (c0 < n && n_v < chunk_v) {
+                const uint32_t cnt = h_dropped[c0] ? 0u : dcnt[prep.recs[job.g0 + c0].qlen];
+                const uint32_t take = std::min<uint32_t>(cnt - f0, chunk_v - n_v);
+                if (take) { seg.push_back(n_v); seg.push_back(c0); seg.push_back(f0); n_v += take; }
+                f0 += take;
+                if (f0 == cnt) { c0++; f0 = 0; } else break;                   // chunk full in the middle of a guide
             }
-            n_matches = h[1]; n_seeds_used = use_sweep ? h[3] : 0;
-            if (split_ran) { uint32_t h1; read_ctrs(&h1, 1, d_ctrs2); n_seeds_used += h1; n_launches++; }
-            break;
+            const uint32_t n_seg = (uint32_t)(seg.size() / 3);
+            seg.push_back(n_v);
+            job.ctr.edited_guides += n_v;
+            if (!n_v) continue;
+            if (voff_cap < seg.size()) { if (d_voff) B.free_one(d_voff); voff_cap = std::max<size_t>(seg.size(), 4096); d_voff = B.alloc<uint32_t>(voff_cap); }
+            CK(cudaMemcpyAsync(d_voff, seg.data(), seg.size() * 4, cudaMemcpyHostToDevice, s));
+            LAUNCH(launch_variant_expand(d_guides, n_seg, n_v, d_voff, d_descs, d_doff, d_vq, d_vdesc, d_vguide, d_vfmask, s));
+            const uint32_t sb = plan.sweep_sb(n_v, plan.edited_qmin, p.mismatches);
+            if (sb) use_sweep = true;
+            uint32_t h[4];
+            search_until_fits(plan.search_warps, 6, spill_cap, &chunk, h, [&](uint32_t* d_spill) {
+                CK(cudaMemsetAsync(d_ctrs, 0, 5 * sizeof(uint32_t), s));       // ([5], the final arena's count, stays)
+                SearchArgs m = a; m.p.M = p.mismatches; m.p.R = m.p.D = 0; m.p.counting = 0; m.p.n_tasks = 2 * n_v;
+                m.p.match_cap = (uint32_t)chunk.cap; m.p.spill_cap = spill_cap; m.spill = d_spill; m.matches = chunk.p;
+                m.skip = nullptr; m.gq = d_vq; m.guide_nmatch = d_vnmatch; m.guides = nullptr; m.fmask = d_vfmask;
+                run_fast_all_pams(m, n_v, sb, nullptr);
+            });
+            n_seeds += sb ? h[3] : 0;
+            // room for every match of the chunk in the final arena, then rewrite (cannot overflow any more)
+            if ((uint64_t)n_final + h[1] > match_cap) {
+                const uint64_t cap2 = std::max<uint64_t>(match_cap * 2, ((uint64_t)n_final + h[1]) * 2);
+                if (cap2 > (1ull << 31)) throw std::runtime_error("more than 2^31 matches in one batch; lower the batch size");
+                MatchRec* bigger = B.alloc<MatchRec>(cap2);
+                CK(cudaMemcpyAsync(bigger, d_matches, (size_t)n_final * sizeof(MatchRec), cudaMemcpyDeviceToDevice, s));
+                CK(cudaStreamSynchronize(s));
+                B.free_one(d_matches); d_matches = bigger; match_cap = cap2;
+            }
+            LAUNCH(launch_variant_rewrite(chunk.p, h[1], d_guides, d_vdesc, d_vguide, d_matches, (uint32_t)match_cap, d_ctrs + 5, d_nmatch, d_ctrs + 2, s));
+            read_ctrs(&n_final, 1, d_ctrs + 5); n_launches++;
         }
+        n_matches = n_final;
+    }
+    // every PAM of the batch over the guides of m: in one fused pass, or one pass per PAM over the same arenas (only the work
+    // counters start over)
+    void run_fast_all_pams(SearchArgs& m, uint32_t ng, uint32_t sb, cudaEvent_t ev_mid) {
+        m.n_fused = 0;
+        if (plan.fuse_pams && !m.p.counting) {
+            m.n_fused = prep.n_fast_pams;
+            for (uint32_t k = 0; k < prep.n_fast_pams; k++) m.fused_pams[k] = prep.pampacks[k];
+            m.plen = prep.plens[0]; m.pampack = fused_filter_pampack(prep.pampacks, prep.n_fast_pams, prep.plens[0]);
+            launch_fast(m, ng, sb, ev_mid);
+            return;
         }
-        CK(cudaEventRecord(ev[1], s));
-        if (n) {
-            std::lock_guard<std::mutex> lk(job->ix->learn_mu);
-            double& v = job->ix->learned_matches_per_guide[learn_key];
-            v = std::max(v * 0.9, (double)n_matches / (double)n);                  // (decays, so that one odd batch does not inflate the arenas for good)
+        for (uint32_t k = 0; k < prep.n_fast_pams; k++) {
+            m.pampack = prep.pampacks[k]; m.plen = prep.plens[k];
+            if (k) { CK(cudaMemsetAsync(d_ctrs, 0, 4, s)); CK(cudaMemsetAsync(d_ctrs + 3, 0, 8, s)); }      // task / seed-queue / work-unit counters
+            launch_fast(m, ng, sb, k == 0 ? ev_mid : nullptr);
         }
-        // ---- arrange --------------------------------------------------------------------------------------------------
-        uint32_t* d_moff = B.alloc<uint32_t>(n + 1);
+    }
+    // fast path launch over ng guides (m.gq): [sweep ->] search_fast_kernel [-> the two-part sweep's PAM-first search].
+    // d_ctrs: [3] seed queue count, [4] sweep work-unit counter
+    void launch_fast(SearchArgs& m, uint32_t ng, uint32_t sb, cudaEvent_t ev_mid) {
+        const bool split = sb && plan.split;                               // (never a counting pass or edited guides: plan_search)
+        if (split) sweep_split(m, ng); else if (sb) sweep_plain(m, ng, sb);
+        if (sb) { m.seeds = sw.queue; m.n_seeds = d_ctrs + 3; m.seed_cap = (uint32_t)sw.queue_cap; m.combos = nullptr; m.n_combos = 0; }
+        if (ev_mid) CK(cudaEventRecord(ev_mid, s));
+        LAUNCH(launch_search_fast(m, plan.variant_fast, di.sm_count, s));
+        if (split) finish_split(m);
+    }
+    // the sweep's arguments for the ng guides of m: its seed queue, gtab_rows rows of per-guide filter masks
+    SweepArgs sweep_args(const SearchArgs& m, uint32_t ng, size_t gtab_rows) {
+        if (!sw.queue) sw.queue = B.alloc<SeedNode>(sw.queue_cap);
+        if (sw.gtab_cap < gtab_rows) { if (sw.gtab) B.free_one(sw.gtab); sw.gtab = B.alloc<uint32_t>(gtab_rows * 20); sw.gtab_cap = gtab_rows; }
+        SweepArgs w{};
+        w.st[0] = m.st[0]; w.st[1] = m.st[1]; w.gq = m.gq; w.skip = m.skip; w.n_guides = ng; w.M = m.p.M; w.plen = m.plen; w.pampack = m.pampack;
+        w.queue = sw.queue; w.queue_cap = (uint32_t)sw.queue_cap; w.queue_count = d_ctrs + 3; w.item_counter = d_ctrs + 4;
+        w.error_flag = d_ctrs + 2; w.stats = d_stats; w.gtab = sw.gtab;
+        return w;
+    }
+    void sweep_plain(const SearchArgs& m, uint32_t ng, uint32_t sb) {
+        if (sw.xtab_M != m.p.M || sw.xtab_sb != sb) {
+            std::vector<uint32_t> xtab;
+            sweep_make_plan(plan.ftab_L, sb, m.p.M, sw.plan, xtab);
+            if (sw.xtab) B.free_one(sw.xtab);
+            sw.n_xtab = (uint32_t)xtab.size(); sw.xtab_M = m.p.M; sw.xtab_sb = sb;
+            xtab.resize(xtab.size() + 64, 0u);                                // (sweep_lean_kernel reads up to 63 words past a pass's end, unused)
+            sw.xtab = B.alloc<uint32_t>(xtab.size());
+            CK(cudaMemcpyAsync(sw.xtab, xtab.data(), xtab.size() * 4, cudaMemcpyHostToDevice, s)); CK(cudaStreamSynchronize(s));
+        }
+        SweepArgs w = sweep_args(m, ng, ng);
+        w.plan = sw.plan; w.xtab = sw.xtab; w.n_xtab = sw.n_xtab; w.load_mode = plan.load_mode; w.fmask = m.fmask;
+        w.parts = 1;                                                       // measured: cutting the units does not pay (profiles/r01r_*)
+        LAUNCH(launch_sweep_guides(w, s));
+        LAUNCH(launch_sweep(w, plan.sweep_variant(m.p.M, qmin, qmax, m.plen, m.pampack), di.sm_count, s));
+    }
+    // the two-part sweep: the distal-first form (filter-mask rows 0 .. ng-1) and the PAM-first form (rows ng .. 2ng-1) in one
+    // sweep, each into its own seed queue
+    void sweep_split(const SearchArgs& m, uint32_t ng) {
+        if (!sp.xtab) {
+            std::vector<uint32_t> xtab;
+            split_make_plan(plan.ftab_L, plan.split_sb, m.p.M, 2 * kSplitHalf, prep.plen, prep.pampack, kSplitHalf, sp.plan, xtab);
+            if (xtab.size() > (size_t)kSplitXtabShared) throw std::runtime_error("two-part enumeration: xor table too long for this slice width");
+            sp.n_xtab = (uint32_t)xtab.size();
+            sp.xtab = B.alloc<uint32_t>(xtab.size());
+            CK(cudaMemcpyAsync(sp.xtab, xtab.data(), xtab.size() * 4, cudaMemcpyHostToDevice, s)); CK(cudaStreamSynchronize(s));
+            sp.gq2 = B.alloc<uint64_t>(ng); sp.nmatch2 = B.alloc<uint32_t>(ng + 1);
+            LAUNCH(launch_split_queries(m.gq, ng, prep.pampack, prep.plen, sp.gq2, s));
+        }
+        if (sp.queue2_cap != sw.queue_cap) { if (sp.queue2) B.free_one(sp.queue2); sp.queue2 = B.alloc<SeedNode>(sw.queue_cap); sp.queue2_cap = sw.queue_cap; }
+        if (sp.matches2_cap < m.p.match_cap) { if (sp.matches2) B.free_one(sp.matches2); sp.matches2 = B.alloc<MatchRec>(m.p.match_cap); sp.matches2_cap = m.p.match_cap; }
+        CK(cudaMemsetAsync(sp.ctrs2, 0, 4 * sizeof(uint32_t), s));
+        SweepArgs w = sweep_args(m, ng, 2 * (size_t)ng);
+        w.plan.L = plan.ftab_L; w.plan.sb = plan.split_sb; w.plan.M = m.p.M; w.split = sp.plan; w.gq2 = sp.gq2; w.xtab = sp.xtab; w.n_xtab = sp.n_xtab;
+        w.queue2 = sp.queue2; w.queue2_count = sp.ctrs2 + 0;
+        LAUNCH(launch_sweep_guides(w, s));                                 // rows 0 .. ng-1: form 0
+        SweepArgs w1 = w; w1.gq = sp.gq2; w1.plen = 0; w1.pampack = 0; w1.gtab = sw.gtab + (size_t)ng * 20;
+        LAUNCH(launch_sweep_guides(w1, s));                                // rows ng .. 2ng-1: form 1
+        LAUNCH(launch_sweep_split(w, plan.split_ctas, di.sm_count, s));
+    }
+    // form 1 after form 0's tree search: the tree search of its seeds with the PAM-first query (all of it protospacer), into an
+    // arena of its own, then the re-anchoring of those matches into m's arena
+    void finish_split(const SearchArgs& m) {
+        SearchArgs m1 = m;
+        m1.gq = sp.gq2; m1.plen = 0; m1.pampack = 0; m1.seeds = sp.queue2; m1.n_seeds = sp.ctrs2 + 0;
+        m1.task_counter = sp.ctrs2 + 1; m1.match_count = sp.ctrs2 + 2; m1.matches = sp.matches2; m1.guide_nmatch = sp.nmatch2;
+        LAUNCH(launch_search_fast(m1, plan.variant_fast, di.sm_count, s));
+        ReanchorArgs r{};
+        r.st[0] = m.st[0]; r.st[1] = m.st[1]; r.in = sp.matches2; r.n_in = sp.ctrs2 + 2; r.in_cap = m.p.match_cap;
+        r.gq = m.gq; r.gq2 = sp.gq2; r.pampack = prep.pampack; r.plen = prep.plen;
+        r.out = m.matches; r.out_count = m.match_count; r.out_cap = m.p.match_cap; r.guide_nmatch = m.guide_nmatch; r.error_flag = m.error_flag;
+        r.stats = d_stats;
+        LAUNCH(launch_reanchor(r, s));
+        sp.ran = true;
+    }
+    // matches -> per-guide hit lists in the reference's order
+    void arrange() {
+        HostArrays& H = job.out;
+        d_moff = B.alloc<uint32_t>(n + 1);
         uint32_t* d_cursor = B.alloc<uint32_t>(n, true, s);
         uint32_t* d_by_guide = B.alloc<uint32_t>(n_matches);
-        uint32_t* d_sorted = B.alloc<uint32_t>(n_matches);
-        uint32_t* d_sorted_off = B.alloc<uint32_t>(n_matches);
-        uint32_t* d_nhits = B.alloc<uint32_t>(n + 1, true, s);
-        uint32_t* d_hoff = B.alloc<uint32_t>(n + 1);
-        uint32_t* d_cbd = B.alloc<uint32_t>((size_t)n * n_dist, true, s);
+        d_sorted = B.alloc<uint32_t>(n_matches);
+        d_sorted_off = B.alloc<uint32_t>(n_matches);
+        d_nhits = B.alloc<uint32_t>(n + 1, true, s);
+        d_hoff = B.alloc<uint32_t>(n + 1);
+        d_cbd = B.alloc<uint32_t>((size_t)n * n_dist, true, s);
         CK(launch_scan(d_nmatch, d_moff, n, s)); n_launches += 2 + (n_matches ? 1 : 0);
         // thousands of matches per guide (bulges): global radix sort (gsx_arrange.cu); otherwise the per-guide rank sort
-        // (GSX_ORDER: 0 warp per guide, 1 CTA per guide, 2 radix sort)
         // ... and whenever SOME guide has thousands (repeat families, low-complexity guides: the rank sort is quadratic per guide -- 457 ms
         // per 200 k guides on the skew stressor of SURVEY 8(d), profiles/r02d_session_3100mb_files_cfg4_skew.jsonl)
         uint64_t max_per_guide = 0;
-        if (n_matches && (uint64_t)n_matches <= (uint64_t)n * 256 && !env_int("GSX_ORDER", 0) && !env_int("GSX_ORDER_CTA", 0)) {
+        if (n_matches && (uint64_t)n_matches <= (uint64_t)n * 256 && plan.order_probe) {
             unsigned long long* d_tm = B.alloc<unsigned long long>(3, true, s);
-            CK(launch_total_u32(d_nmatch, n, d_tm, reinterpret_cast<unsigned int*>(d_tm + 2), reinterpret_cast<unsigned long long*>(mbox.p + 32), s)); n_launches++;
+            LAUNCH(launch_total_u32(d_nmatch, n, d_tm, reinterpret_cast<unsigned int*>(d_tm + 2), reinterpret_cast<unsigned long long*>(mbox.p + 32), s));
             CK(cudaStreamSynchronize(s));
             max_per_guide = reinterpret_cast<volatile unsigned long long*>(mbox.p + 32)[1];
         }
-        const int order_mode = env_int("GSX_ORDER", env_int("GSX_ORDER_CTA", 0) ? 1 : (((uint64_t)n_matches > (uint64_t)n * 256 || max_per_guide > 2048) ? 2 : 0));
+        const int order_mode = plan.order_mode != kUnset ? plan.order_mode : (((uint64_t)n_matches > (uint64_t)n * 256 || max_per_guide > 2048) ? 2 : 0);
         if (order_mode == 2) {
             const size_t sb_bytes = order_sorted_scratch_bytes(n_matches);
             void* scratch = B.alloc<unsigned char>(sb_bytes);
@@ -1181,47 +1213,49 @@ static void run_device_job(DeviceJob* job) {
         {   // total hits can exceed 2^32 only for absurd inputs; the scan is 32-bit, so the total is a 64-bit sum (device-side, stored
             // into the mailbox: the per-guide counts themselves travel with the other result arrays at the end)
             unsigned long long* d_tot = B.alloc<unsigned long long>(3, true, s);
-            CK(launch_total_u32(d_nhits, n, d_tot, reinterpret_cast<unsigned int*>(d_tot + 2), reinterpret_cast<unsigned long long*>(mbox.p + 32), s)); n_launches++;
+            LAUNCH(launch_total_u32(d_nhits, n, d_tot, reinterpret_cast<unsigned int*>(d_tot + 2), reinterpret_cast<unsigned long long*>(mbox.p + 32), s));
             CK(cudaStreamSynchronize(s));
             const uint64_t tot = *reinterpret_cast<volatile unsigned long long*>(mbox.p + 32);
             if (tot >= (1ull << 32)) throw std::runtime_error("more than 2^32 hits in one batch; lower the batch size");
             H.n_hits = (size_t)tot;
         }
         CK(launch_scan(d_nhits, d_hoff, n, s));
-        const uint32_t nh = (uint32_t)H.n_hits;
-        uint32_t* d_hit_match = B.alloc<uint32_t>(nh); uint32_t* d_hit_row = B.alloc<uint32_t>(nh); uint32_t* d_hit_guide = B.alloc<uint32_t>(nh);
+        nh = (uint32_t)H.n_hits;
+        d_hit_match = B.alloc<uint32_t>(nh); d_hit_row = B.alloc<uint32_t>(nh); uint32_t* d_hit_guide = B.alloc<uint32_t>(nh);
         n_launches += (n_matches ? 1 : 0) + (H.n_hits ? 1 : 0) + 2;      // scan, expand, locate_score, specificity
         CK(launch_expand(d_matches, d_moff, d_sorted, d_sorted_off, d_hoff, n, n_matches, d_hit_match, d_hit_row, d_hit_guide, s));
-        CK(cudaEventRecord(ev[2], s));
-        // ---- locate + coordinates + CFD ------------------------------------------------------------------------------
-        CK(cudaStreamWaitEvent(s, ev_guides, 0));                                     // the guide records (uploaded under the search)
-        LocateArgs L{};
+        CK(cudaEventRecord(js.ev[kArrangeEnd], s));
+    }
+    // coordinates, strands, distances and CFD of every hit
+    void locate_score() {
+        CK(cudaStreamWaitEvent(s, js.ev_guides, 0));                                  // the guide records (uploaded under the search)
         L.st[0] = di.st[0].d; L.st[1] = di.st[1].d; L.matches = d_matches; L.guides = d_guides; L.pamsets = d_pamsets; L.chroms = di.chroms;
-        L.hit_match = d_hit_match; L.hit_row = d_hit_row; L.n_hits = nh; L.n_chr = (uint32_t)job->ix->chroms.size(); L.wide = wide;
-        L.genome_length = job->ix->host.genome_length;
+        L.hit_match = d_hit_match; L.hit_row = d_hit_row; L.n_hits = nh; L.n_chr = (uint32_t)job.ix->chroms.size(); L.wide = prep.wide;
+        L.genome_length = job.ix->host.genome_length;
         L.abs_pos = B.alloc<int64_t>(nh); L.chr = B.alloc<int32_t>(nh); L.pos1 = B.alloc<uint32_t>(nh); L.strand = B.alloc<uint8_t>(nh);
         L.distance = B.alloc<uint8_t>(nh); L.dna = B.alloc<uint8_t>(nh); L.rna = B.alloc<uint8_t>(nh); L.index_id = B.alloc<uint8_t>(nh);
         L.cfd = B.alloc<float>(nh); L.flags = B.alloc<uint8_t>(nh); L.stats = d_stats;
-        L.key_lo = B.alloc<uint64_t>(nh); L.key_hi = wide ? B.alloc<uint64_t>(nh) : nullptr; L.mlen = B.alloc<uint8_t>(nh);
+        L.key_lo = B.alloc<uint64_t>(nh); L.key_hi = prep.wide ? B.alloc<uint64_t>(nh) : nullptr; L.mlen = B.alloc<uint8_t>(nh);
         CK(launch_locate_score(L, s));
-        CK(cudaEventRecord(ev[3], s));
-        // ---- specificity ------------------------------------------------------------------------------------------------
-        SpecArgs S{};
+        CK(cudaEventRecord(js.ev[kLocateEnd], s));
+    }
+    void specificity() {
         S.guide_hoff = d_hoff; S.count_by_distance = d_cbd; S.chr = L.chr; S.cfd = L.cfd; S.flags = L.flags;
         S.counted = B.alloc<uint8_t>(nh, true, s); S.specificity = B.alloc<float>(n); S.perfect = B.alloc<uint8_t>(n);
         S.n_guides = n; S.n_dist = n_dist; S.sam_rule = p.sam_scoring ? 1 : 0; S.max_off_targets = p.max_off_targets;
-        S.warp_per_guide = (uint32_t)env_int("GSX_SPEC_WARP", (uint64_t)nh > (uint64_t)n * 64 ? 1 : 0);
+        S.warp_per_guide = plan.spec_warp != kUnset ? (uint32_t)plan.spec_warp : ((uint64_t)nh > (uint64_t)n * 64 ? 1u : 0u);
         CK(launch_specificity(S, s));
-        CK(cudaEventRecord(ev[4], s));
-        // ---- results to host ---------------------------------------------------------------------------------------------
+        CK(cudaEventRecord(js.ev[kScoreEnd], s));
+    }
+    // the per-guide arrays and the per-hit arrays the caller reads (all of them for the public calls); the device's turn ends here
+    void copy_results() {
+        HostArrays& H = job.out;
         auto d2h = [&](void* dst, const void* src, size_t bytes) { if (bytes) CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s)); };
         d2h(H.dropped, d_dropped, n); d2h(H.hoff, d_hoff, (size_t)(n + 1) * 4); d2h(H.n_hits_of, d_nhits, (size_t)n * 4); d2h(H.specificity, S.specificity, (size_t)n * 4);
         d2h(H.perfect, S.perfect, n); d2h(H.cbd, d_cbd, (size_t)n * n_dist * 4);
-        // the per-hit arrays: those the caller reads (all of them for the public calls)
-        const uint32_t want = job->want;
         auto hit_array = [&](uint32_t bit, auto*& dst, const auto* src) {
             using T = std::remove_pointer_t<std::remove_reference_t<decltype(dst)>>;
-            if (!(want & bit)) { dst = nullptr; return; }
+            if (!(job.want & bit)) { dst = nullptr; return; }
             dst = H.alloc<T>(nh); d2h(dst, src, (size_t)nh * sizeof(T));
         };
         hit_array(kWantAbsPos, H.abs_pos, L.abs_pos); hit_array(kWantSaRow, H.sa_row, d_hit_row); hit_array(kWantChr, H.chr, L.chr);
@@ -1229,29 +1263,45 @@ static void run_device_job(DeviceJob* job) {
         hit_array(kWantBulges, H.rna, L.rna); hit_array(kWantBulges, H.dna, L.dna); hit_array(kWantIndexId, H.index_id, L.index_id);
         hit_array(kWantCfd, H.cfd, L.cfd); hit_array(kWantCounted, H.counted, S.counted);
         hit_array(kWantMatchString, H.key_lo, L.key_lo); hit_array(kWantMatchString, H.mlen, L.mlen);
-        H.key_hi = nullptr; if (wide) hit_array(kWantMatchString, H.key_hi, L.key_hi);
-        unsigned long long st[8]; d2h(st, d_stats, sizeof st);
-        CK(cudaEventRecord(ev[5], s));
+        H.key_hi = nullptr; if (prep.wide) hit_array(kWantMatchString, H.key_hi, L.key_hi);
+        d2h(stats, d_stats, sizeof stats);
+        CK(cudaEventRecord(js.ev[kCopyEnd], s));
         CK(cudaStreamSynchronize(s)); CK(cudaStreamSynchronize(s2));
         // the turn on the device ends with the copies: a result transfer running under the NEXT call's sweep slows both several
         // times over (170 MB streaming through the L2 that holds the sweep's slices: profiles/r02b_session_3100mb_sweep_lean.jsonl,
         // m3_lean_v11_pipe2); what overlaps between pipelined calls is the host work -- guide packing before, result assembly after
         if (turn.owns_lock()) turn.unlock();
-        float ms;
-        CK(cudaEventElapsedTime(&ms, ev[0], ev[1])); job->ctr.ms_search = ms;
-        CK(cudaEventElapsedTime(&ms, ev[1], ev[2])); job->ctr.ms_arrange = ms;
-        CK(cudaEventElapsedTime(&ms, ev[2], ev[3])); job->ctr.ms_locate = ms;
-        CK(cudaEventElapsedTime(&ms, ev[3], ev[4])); job->ctr.ms_score = ms;
-        CK(cudaEventElapsedTime(&ms, ev[0], ev[4])); job->ctr.ms_total_device = ms;
-        CK(cudaEventElapsedTime(&ms, ev[4], ev[5])); job->ctr.ms_d2h = ms;
-        CK(cudaEventElapsedTime(&ms, ev[6], ev[7])); job->ctr.ms_sweep = ms; job->ctr.seeds = n_seeds_used;
-        job->ctr.sectors = use_sweep ? st[5] + st[7] : st[1];
-        job->ctr.nodes = st[0]; job->ctr.lookups = st[1]; job->ctr.spills = st[2]; job->ctr.lf_steps = st[3];
-        job->ctr.matches = n_matches; job->ctr.hits = nh; job->ctr.launches = n_launches;
+    }
+    void counters() {
+        gsx_counters& c = job.ctr;
+        auto ms = [&](JobEvent a0, JobEvent a1) { float t; CK(cudaEventElapsedTime(&t, js.ev[a0], js.ev[a1])); return (double)t; };
+        c.ms_search = ms(kSearchBegin, kSearchEnd); c.ms_arrange = ms(kSearchEnd, kArrangeEnd); c.ms_locate = ms(kArrangeEnd, kLocateEnd);
+        c.ms_score = ms(kLocateEnd, kScoreEnd); c.ms_total_device = ms(kSearchBegin, kScoreEnd); c.ms_d2h = ms(kScoreEnd, kCopyEnd);
+        c.ms_sweep = ms(kSweepBegin, kSweepEnd); c.seeds = n_seeds;
+        c.sectors = use_sweep ? stats[5] + stats[7] : stats[1];
+        c.nodes = stats[0]; c.lookups = stats[1]; c.spills = stats[2]; c.lf_steps = stats[3];
+        c.matches = n_matches; c.hits = nh; c.launches = n_launches;
+    }
+};
+
+
+static void run_device_job(DeviceJob* job) {
+    try {
+        CK(cudaSetDevice(job->ix->dev[job->slot].device));
+        DeviceRun r(*job);
+        if (!r.setup()) return;
+        if (job->p->threshold > 0) r.threshold_pass();
+        r.search();
+        r.arrange();
+        r.locate_score();
+        r.specificity();
+        r.copy_results();
+        r.counters();
     } catch (const CudaError& e) { job->status = GSX_ERR_CUDA; job->err = e.what(); }
     catch (const std::bad_alloc&) { job->status = GSX_ERR_NOMEM; job->err = "out of host memory"; }
     catch (const std::exception& e) { job->status = GSX_ERR_INTERNAL; job->err = e.what(); }
 }
+#undef LAUNCH
 
 // The public view.  One part: its arrays as they are.  Several parts (one per device): the per-guide and per-hit arrays are
 // concatenated -- lazily, when gsx_result_view_get is first called; the library's own formatter reads the parts in place.

@@ -138,6 +138,54 @@ struct Prepared {
     uint32_t max_qlen = 0;
 };
 
+// what the search plan reads from a device index (DeviceIndex)
+struct IndexShape {
+    bool plain = true;              // no BWT row outside A/C/G/T but the sentinel, on either strand (n_exc == 1, n_nrows == 0)
+    bool lines = false;             // look-ahead lines
+    bool exc_map = false;           // exception-block bitmaps on both strands
+    uint32_t ftab_L[2] = {0, 0};    // jump-table depth per strand
+    bool sum0 = false;              // pattern summaries on both strands
+    uint64_t rows = 0;              // rows of the forward strand
+    int sm_count = 0;
+};
+
+// How a device job searches its n guides (gsx_api.cpp plan_search): the path, the kernel variants, the slice widths, the first
+// arena sizes and every GSX_* knob of the search.  A pure function of the batch, the parameters, the index's shape and the
+// environment.
+struct SearchPlan {
+    bool use_fast = false;          // search_fast_kernel; otherwise the general search_kernel
+    bool exc = false;               // ... over an index with N (search_fast_kernel<..., EXC>)
+    bool use_variants = false;      // bulges as edited guides, `chunk` edited guides per launch
+    bool late_guides = false;       // the guide records go up on the second stream under the first search
+    int variant_general[2] = {0, 0}, variant_fast = 1;     // occupancy variants of the tree search: general narrow / wide, fast
+    int search_warps = 0, threshold_warps = 0;              // grids of the main search and of the threshold pass (<= 0: unknown variant)
+    bool fuse_pams = false;         // every alternative PAM in one pass
+    uint32_t search_sb = 0, threshold_sb = 0;               // slice characters of the sweep, 0 = no sweep
+    bool combos = false, threshold_combos = false;          // jump-table combos (search_fast_kernel without a sweep)
+    bool split = false; uint32_t split_sb = 0; int split_ctas = 6;       // two-part sweep (sweep_split_kernel)
+    uint32_t load_mode = 2, pin_width = 0;
+    size_t expand_roots = 0;        // general kernel with fewer tasks than its grid keeps busy: roots expanded to this many nodes
+    uint32_t chunk = 0; bool fmask = false;                 // edited guides per launch; the sweep skips substituted insertions
+    uint32_t edited_qmin = 0, edited_qmax = 0;              // lengths of the edited guides
+    uint64_t queue_cap = 0, chunk_queue_cap = 0;            // seed queue: batch (and threshold pass), edited-guide chunk
+    double match_per_guide = 0;     // main search's match arena per guide, before what earlier calls needed
+    uint64_t match_cap_set = 0;     // GSX_MATCH_CAP
+    uint64_t chunk_match_cap = 0, edited_match_cap = 0;     // match arenas of one edited-guide chunk and of the whole batch
+    uint32_t spill_cap = 0;         // spill stack entries per warp of the main search
+    // GSX_ORDER (0 warp per guide, 1 CTA per guide, 2 radix sort), GSX_SPEC_WARP, GSX_SWEEP_VARIANT; INT_MIN when not set: by
+    // matches per guide, hits per guide, and mismatches and guide lengths
+    int order_mode = 0, spec_warp = 0, sweep_variant_set = 0;
+    bool order_probe = true;        // measure the largest matches per guide for the automatic ordering
+    // the sweep's slice characters where a batch is large enough (0 = no sweep), for launches whose batch is known per chunk
+    uint32_t ftab_L = 0, sweep_width = 0, sweep_min = 0;
+
+    // slice characters of a sweep over ng guides no shorter than min_qlen with M mismatches, 0 = no sweep
+    uint32_t sweep_sb(uint32_t ng, uint32_t min_qlen, uint32_t M) const;
+    // sweep kernel variant for guide lengths qmin .. qmax, M mismatches and this PAM (2 where sweep_lean_kernel has no layout)
+    int sweep_variant(uint32_t M, uint32_t qmin, uint32_t qmax, uint32_t plen, uint32_t pampack) const;
+};
+SearchPlan plan_search(const Prepared& prep, const gsx_params& p, const IndexShape& ix, uint32_t n);
+
 // every way to substitute at most M of the first n_pos characters (k-mer jump table enumeration, gsx_core.h)
 std::vector<uint64_t> ftab_combos(uint32_t n_pos, uint32_t M);
 // slice-major enumeration plan (gsx_core.h sweep_pattern): the xor table of every way to substitute at most M of the
