@@ -5,7 +5,9 @@
 #include "gsx_host.h"
 #include "gsx_core.h"
 #include "gsx_sites.h"
+#include "gsx_decode.h"
 #include <algorithm>
+#include <atomic>
 #include <cstdio>
 #include <cstdlib>
 #include <chrono>
@@ -313,17 +315,21 @@ bool read_guides_csv(const char* path, GuideTable& t, std::string& err) {
 }
 }  // namespace
 
+namespace {
+std::string csv_header(bool complete) {                                                     // printer.hpp:181-187
+    std::string s = "id,sequence,match_chrm,match_position,match_strand,match_distance";
+    if (complete) s += ",match_sequence,rna_bulges,dna_bulges";
+    return s + ",specificity\n";
+}
+}  // namespace
+
 extern "C" int gsx_format_header(const gsx_index* ix, int format_sam, int complete, char** buf, size_t* len) {
     if (!ix || !buf || !len) return GSX_ERR_ARG;
     std::string s;
     if (format_sam) {                                                                        // printer.hpp:173-179
         s += "@HD\tVN:1.0\tSO:unknown\n@PG\tID:Guidescan\tVN:2.0.0\n";
         for (size_t i = 0; i < ix->host.chr_names.size(); i++) { s += "@SQ\tSN:" + ix->host.chr_names[i] + "\tLN:"; put_u64(s, ix->host.chr_lens[i]); s += "\n"; }
-    } else {                                                                                 // printer.hpp:181-187
-        s += "id,sequence,match_chrm,match_position,match_strand,match_distance";
-        if (complete) s += ",match_sequence,rna_bulges,dna_bulges";
-        s += ",specificity\n";
-    }
+    } else s = csv_header(complete != 0);
     return ret_buf(s, buf, len);
 }
 
@@ -848,4 +854,419 @@ extern "C" int gsx_enumerate_genome(const gsx_index* ix, const char* fasta_path,
     catch (const std::bad_alloc&) { rc = gsx_set_error(GSX_ERR_NOMEM, "out of host memory"); }
     fclose(in);
     return rc;
+}
+
+// ---- SAM complete database in, off-target rows out (gsx_decode_database) -------------------------------------------------------
+// A host thread reads the SAM in batches of whole lines and splits the records; the of:H: lists go to the device inside the batch's
+// own text (gsx_decode.cu), the rows come back as arrays, and a formatter and a writer thread turn them into CSV behind the reader,
+// in record order -- the structure of run_file_job.
+namespace {
+struct DecodeRec {
+    const char* id; const char* sp; uint32_t id_len, sp_len;
+    uint32_t seq_at, seq_len;              // the guide's sequence in the batch's `seqs`
+    uint64_t at;                           // byte offset of the record in the file
+};
+struct DecodeBatch {
+    gsx::PinnedBuf text_buf; const char* text = nullptr; size_t len = 0; uint64_t file_off = 0;
+    std::vector<DecodeRec> recs; std::string seqs;
+    std::vector<uint64_t> rec_hex; std::vector<uint32_t> rec_entry; std::vector<gsx::DecodeGuide> guides;
+    gsx::DecodeRows rows;
+    void clear() { recs.clear(); seqs.clear(); rec_hex.clear(); rec_entry.assign(1, 0); guides.clear(); len = 0; }
+};
+
+gsx::SiteError decode_error(const std::string& msg) { return gsx::SiteError{GSX_ERR_ARG, msg}; }
+std::string quoted(const char* p, size_t n) { return "\"" + std::string(p, std::min<size_t>(n, 200)) + "\""; }
+
+// the SAM in batches of whole lines, about `bytes` each (a longer line makes its batch longer)
+struct SamReader {
+    FILE* f; uint64_t off = 0; std::string carry; bool eof = false;
+    explicit SamReader(FILE* ff) : f(ff) {}
+    bool next(size_t bytes, DecodeBatch& b) {
+        b.clear(); b.file_off = off;
+        size_t cap = std::max(bytes, 2 * carry.size() + 1);
+        char* t = (char*)b.text_buf.need(cap); cap = b.text_buf.cap;
+        memcpy(t, carry.data(), carry.size());
+        size_t have = carry.size(); carry.clear();
+        for (;;) {
+            while (!eof && have < cap) { const size_t got = fread(t + have, 1, cap - have, f); if (!got) eof = true; have += got; }
+            const char* nl = have ? (const char*)memrchr(t, '\n', have) : nullptr;
+            if (nl || eof) {
+                const size_t keep = nl && !eof ? (size_t)(nl - t) + 1 : have;
+                carry.assign(t + keep, have - keep); b.len = keep;
+                break;
+            }
+            std::string whole(t, have);                                                     // one line longer than the batch
+            t = (char*)b.text_buf.need(2 * cap); cap = b.text_buf.cap; memcpy(t, whole.data(), have);
+        }
+        b.text = t; off += b.len;
+        return b.len > 0;
+    }
+};
+
+// one record's fields: QNAME, FLAG, RNAME, POS, SEQ and the two tags the decode reads
+struct SamFields {
+    const char* f[11]; uint32_t n[11]; int nf = 0;
+    const char* of = nullptr; size_t of_len = 0; const char* sp = nullptr; size_t sp_len = 0;
+    void split(const char* p, const char* end) {
+        nf = 0; of = sp = nullptr;
+        for (;;) {
+            const char* tab = (const char*)memchr(p, '\t', (size_t)(end - p));
+            const char* e = tab ? tab : end;
+            if (nf < 11) { f[nf] = p; n[nf] = (uint32_t)(e - p); }
+            else if (e - p >= 5 && !memcmp(p, "of:H:", 5)) { of = p + 5; of_len = (size_t)(e - p) - 5; }
+            else if (e - p >= 5 && !memcmp(p, "sp:f:", 5)) { sp = p + 5; sp_len = (size_t)(e - p) - 5; }
+            nf++;
+            if (!tab) break;
+            p = tab + 1;
+        }
+    }
+    bool number(int i, uint64_t& v) const {
+        if (!n[i] || n[i] > 19) return false;
+        v = 0; for (uint32_t k = 0; k < n[i]; k++) { const char c = f[i][k]; if (c < '0' || c > '9') return false; v = v * 10 + (uint64_t)(c - '0'); }
+        return true;
+    }
+};
+
+int64_t hex_le64(const char* p) {                                                           // 16 digits, low byte first (printer.hpp:18-88)
+    uint64_t v = 0;
+    for (int b = 0; b < 8; b++) {
+        int d[2];
+        for (int k = 0; k < 2; k++) { const char c = p[2 * b + k], l = (char)(c | 32); d[k] = c >= '0' && c <= '9' ? c - '0' : (l >= 'a' && l <= 'f' ? l - 'a' + 10 : -1); }
+        if (d[0] < 0 || d[1] < 0) return 0;
+        v |= (uint64_t)(d[0] * 16 + d[1]) << (8 * b);
+    }
+    return (int64_t)v;
+}
+
+// Records of a batch: which are decoded, with their guides.  Consecutive records of one QNAME are one guide: the first is decoded, the
+// others must carry the same list.
+struct DecodeSplitter {
+    uint32_t pam_len; const std::map<std::string, std::vector<std::pair<uint64_t, uint64_t>>>* regions;
+    std::map<std::string, std::vector<gsx::StartRange>> ranges; uint32_t ranges_k = 0;      // the regions as site starts for sites of ranges_k bases
+    std::string prev_id, prev_of; const char* pid = nullptr; size_t pid_len = 0; const char* pof = nullptr; size_t pof_len = 0; bool have_prev = false;
+    size_t records = 0;
+
+    bool selected(const SamFields& F, uint32_t L) {
+        if (!regions) return true;
+        uint64_t pos = 0;
+        if (!F.number(3, pos) || pos == 0) return false;                                     // (a sentinel record, or POS 0)
+        if (L != ranges_k) {
+            ranges.clear(); ranges_k = L;
+            for (const auto& kv : *regions) ranges[kv.first] = gsx::merge_regions(kv.second, L);
+        }
+        const auto it = ranges.find(std::string(F.f[2], F.n[2]));
+        if (it == ranges.end()) return false;
+        const uint64_t a = pos - 1;                                                          // the site is [POS - 1, POS - 1 + L)
+        const std::vector<gsx::StartRange>& v = it->second;
+        const auto r = std::upper_bound(v.begin(), v.end(), a, [](uint64_t x, const gsx::StartRange& s) { return x < s.first; });
+        return r != v.begin() && a <= (r - 1)->second;
+    }
+
+    void split(DecodeBatch& b) {
+        SamFields F;
+        for (size_t at = 0; at < b.len;) {
+            const char* line = b.text + at;
+            const char* nl = (const char*)memchr(line, '\n', b.len - at);
+            const char* end = nl ? nl : b.text + b.len;
+            const uint64_t where = b.file_off + at;
+            at = (size_t)(end - b.text) + (nl ? 1 : 0);
+            if (end > line && end[-1] == '\r') end--;
+            if (end == line || line[0] == '@') continue;
+            records++;
+            F.split(line, end);
+            auto rec = [&] { return "record " + quoted(F.f[0], F.n[0]) + " at byte " + std::to_string(where); };
+            if (F.nf < 11) throw decode_error(rec() + " has " + std::to_string(F.nf) + " tab-separated fields, a SAM record at least 11");
+            if (!F.of) throw decode_error(rec() + " has no of:H: tag: a database written with --mode succinct lists no off-targets; write it with --mode complete");
+            if (!F.sp) throw decode_error(rec() + " has no sp:f: tag");
+            if (F.of_len < 32 || F.of_len % 16) throw decode_error(rec() + ": its of:H: value has " + std::to_string(F.of_len) + " hex digits, not a whole list of 16-digit values (truncated?)");
+            if (have_prev && F.n[0] == pid_len && !memcmp(F.f[0], pid, pid_len)) {           // another perfect match of the same guide
+                if (F.of_len != pof_len || memcmp(F.of, pof, pof_len)) throw decode_error(rec() + ": its of:H: list differs from the previous record of the same QNAME");
+                continue;
+            }
+            have_prev = true; pid = F.f[0]; pid_len = F.n[0]; pof = F.of; pof_len = F.of_len;
+            uint64_t flag = 0;
+            if (!F.number(1, flag)) throw decode_error(rec() + ": FLAG " + quoted(F.f[1], F.n[1]) + " is not a number");
+            const uint32_t L = F.n[9];
+            if (L <= pam_len || L - pam_len > (uint32_t)kMaxQ)
+                throw decode_error(rec() + ": SEQ has " + std::to_string(L) + " bases; with a PAM column of " + std::to_string(pam_len) + " the protospacer must have 1.." + std::to_string(kMaxQ));
+            if (!selected(F, L)) continue;
+            gsx::DecodeGuide g{};
+            const char* s = F.f[9];
+            for (uint32_t i = 0; i < L; i++) g.seq[i] = (flag & 16) ? complement_char(s[L - 1 - i]) : s[i];
+            g.qlen = (uint8_t)(L - pam_len); g.plen = (uint8_t)pam_len;
+            b.recs.push_back({F.f[0], F.sp, F.n[0], (uint32_t)F.sp_len, (uint32_t)b.seqs.size(), L, where});
+            b.seqs.append(g.seq, L);
+            b.guides.push_back(g);
+            b.rec_hex.push_back((uint64_t)(F.of - b.text));
+            b.rec_entry.push_back(b.rec_entry.back() + (uint32_t)(F.of_len / 16));
+        }
+        if (have_prev) {                                                                     // the next batch compares with a copy
+            prev_id.assign(pid, pid_len); prev_of.assign(pof, pof_len);
+            pid = prev_id.data(); pof = prev_of.data();
+        }
+    }
+};
+
+// the rows of records [r0, r1) of a decoded batch, as format_csv_guide prints them (+ the CFD column)
+void format_decoded(const DecodeBatch& b, size_t r0, size_t r1, const std::vector<std::string>& chr_names, bool complete, bool with_cfd, std::string& o) {
+    const gsx::DecodeRows& R = b.rows;
+    std::vector<char> line;
+    for (size_t r = r0; r < r1; r++) {
+        const DecodeRec& c = b.recs[r];
+        const uint32_t h0 = R.rec_row[r], h1 = R.rec_row[r + 1];
+        if (h0 == h1) continue;
+        const size_t need = c.id_len + c.seq_len + c.sp_len + 2 * (kMaxQ + kMaxPamLen) + 96;
+        size_t prefix = c.id_len + 1 + c.seq_len + 1;
+        if (line.size() < need) line.resize(need + 256);
+        char* l = line.data();
+        memcpy(l, c.id, c.id_len); l[c.id_len] = ','; memcpy(l + c.id_len + 1, b.seqs.data() + c.seq_at, c.seq_len); l[prefix - 1] = ',';
+        for (uint32_t h = h0; h < h1; h++) {
+            const std::string& chr = chr_names[R.chr[h]];
+            if (line.size() < need + chr.size()) { line.resize(need + chr.size() + 256); l = line.data(); }
+            char* w = l + prefix;
+            memcpy(w, chr.data(), chr.size()); w += chr.size(); *w++ = ',';
+            w = put_u64_at(w, R.pos1[h]); *w++ = ','; *w++ = (char)R.strand[h]; *w++ = ','; w = put_u64_at(w, R.distance[h]);
+            if (complete) {
+                *w++ = ','; memcpy(w, R.match + (size_t)h * R.stride, c.seq_len); w += c.seq_len;
+                memcpy(w, ",0,0", 4); w += 4;
+            }
+            *w++ = ','; memcpy(w, c.sp, c.sp_len); w += c.sp_len;
+            if (with_cfd) { *w++ = ','; w += snprintf(w, 32, "%.9g", (double)R.cfd[h]); }
+            *w++ = '\n';
+            o.append(l, (size_t)(w - l));
+        }
+    }
+}
+}  // namespace
+
+extern "C" int gsx_decode_database(const char* sam_path, const char* fasta_path, const char* out_path, uint32_t pam_length,
+                                   const char* const* alt_pams, uint32_t n_alt_pams, int complete, int with_cfd, const char* regions_bed,
+                                   int device, size_t* n_guides, size_t* n_rows) {
+    if (!sam_path || !fasta_path || !out_path || (n_alt_pams && !alt_pams)) return gsx_set_error(GSX_ERR_ARG, "null argument");
+    if (n_guides) *n_guides = 0;
+    if (n_rows) *n_rows = 0;
+    // everything is checked before the first device work: options, the SAM's header and first list against the FASTA, the regions
+    if (pam_length < 1 || pam_length > (uint32_t)kMaxPamLen) return gsx_set_error(GSX_ERR_ARG, "pam_length " + std::to_string(pam_length) + " is outside 1.." + std::to_string(kMaxPamLen));
+    if (n_alt_pams > (uint32_t)kMaxPams - 1) return gsx_set_error(GSX_ERR_ARG, std::to_string(n_alt_pams) + " alternative PAMs: at most " + std::to_string(kMaxPams - 1));
+    gsx::DecodePams pams{};
+    pams.n = n_alt_pams;
+    for (uint32_t i = 0; i < n_alt_pams; i++) {
+        const std::string a = alt_pams[i] ? alt_pams[i] : "";
+        if (a.size() != pam_length) return gsx_set_error(GSX_ERR_ARG, "alternative PAM \"" + a + "\" has " + std::to_string(a.size()) + " characters, the PAM column " + std::to_string(pam_length));
+        for (char c : a)
+            if (!(c == 'A' || c == 'C' || c == 'G' || c == 'T' || c == 'N'))
+                return gsx_set_error(GSX_ERR_ARG, "alternative PAM \"" + a + "\" has the character '" + std::string(1, c) + "': PAM characters must be A, C, G, T or N");
+        memcpy(pams.p[i], a.data(), a.size());
+    }
+    if (device < 0) return gsx_set_error(GSX_ERR_ARG, "device " + std::to_string(device) + " is not a device ordinal");
+    FILE* in = fopen(sam_path, "rb");
+    if (!in) return gsx_set_error(GSX_ERR_IO, std::string("cannot open ") + sam_path);
+    struct Closer { FILE* f; ~Closer() { fclose(f); } } closer{in};
+    // the header's @SQ lines and the first record
+    std::vector<std::pair<std::string, uint64_t>> sq;
+    std::string first; uint64_t first_at = 0;
+    {
+        char* lp = nullptr; size_t lcap = 0; ssize_t n; uint64_t at = 0;
+        while ((n = getline(&lp, &lcap, in)) > 0) {
+            std::string l(lp, (size_t)n);
+            while (!l.empty() && (l.back() == '\n' || l.back() == '\r')) l.pop_back();
+            if (l.empty()) { at += (uint64_t)n; continue; }
+            if (l[0] != '@') { first = l; first_at = at; break; }
+            if (l.compare(0, 4, "@SQ\t") == 0) {
+                std::string sn; uint64_t ln = 0; bool have_ln = false;
+                for (size_t b = 4; b <= l.size();) {
+                    size_t e = l.find('\t', b); if (e == std::string::npos) e = l.size();
+                    if (l.compare(b, 3, "SN:") == 0) sn = l.substr(b + 3, e - b - 3);
+                    if (l.compare(b, 3, "LN:") == 0) { ln = strtoull(l.c_str() + b + 3, nullptr, 10); have_ln = true; }
+                    b = e + 1;
+                }
+                if (sn.empty() || !have_ln) { free(lp); return gsx_set_error(GSX_ERR_ARG, "header line at byte " + std::to_string(at) + " of " + sam_path + " is an @SQ line without SN or LN"); }
+                sq.emplace_back(sn, ln);
+            }
+            at += (uint64_t)n;
+        }
+        free(lp);
+        rewind(in);
+    }
+    gsx::HostIndex gi; std::vector<uint8_t> genome; std::string err;
+    const auto t_fasta = std::chrono::steady_clock::now();
+    if (!gsx::read_fasta(fasta_path, genome, gi, err)) return gsx_set_error(GSX_ERR_IO, err);
+    const double s_fasta = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_fasta).count();
+    if (genome.size() != gi.genome_length) return gsx_set_error(GSX_ERR_ARG, std::string("FASTA ") + fasta_path + " has white space inside its sequence lines");
+    if (!sq.empty()) {
+        for (size_t i = 0; i < std::max(sq.size(), gi.chr_names.size()); i++) {
+            if (i < sq.size() && i < gi.chr_names.size() && sq[i].first == gi.chr_names[i] && sq[i].second == gi.chr_lens[i]) continue;
+            const std::string s = i < sq.size() ? "\"" + sq[i].first + "\" of " + std::to_string(sq[i].second) + " bases" : "nothing";
+            const std::string fa = i < gi.chr_names.size() ? "\"" + gi.chr_names[i] + "\" of " + std::to_string(gi.chr_lens[i]) + " bases" : "nothing";
+            return gsx_set_error(GSX_ERR_ARG, "@SQ line " + std::to_string(i + 1) + " of the database names " + s + ", FASTA record " + std::to_string(i + 1) +
+                                                  " is " + fa + ": the database was not computed on this assembly");
+        }
+    }
+    const int64_t delim = -((int64_t)gi.genome_length + 1);
+    if (!first.empty()) {
+        SamFields F; F.split(first.data(), first.data() + first.size());
+        const std::string rec = "record " + quoted(F.f[0], F.n[0]) + " at byte " + std::to_string(first_at);
+        if (!F.of) return gsx_set_error(GSX_ERR_ARG, rec + " has no of:H: tag: a database written with --mode succinct lists no off-targets; write it with --mode complete");
+        if (F.of_len < 32 || F.of_len % 16) return gsx_set_error(GSX_ERR_ARG, rec + ": its of:H: value has " + std::to_string(F.of_len) + " hex digits, not a whole list of 16-digit values (truncated?)");
+        const int64_t d = hex_le64(F.of + F.of_len - 16);
+        if (d != delim)
+            return gsx_set_error(GSX_ERR_ARG, rec + ": its of:H: list ends with " + std::to_string(d) + ", the delimiter of a genome of " + std::to_string(gi.genome_length) +
+                                                  " bases is " + std::to_string(delim) + ": the database was not computed on this assembly");
+    }
+    std::map<std::string, uint64_t> chr_len;
+    for (size_t i = 0; i < gi.chr_names.size(); i++) chr_len[gi.chr_names[i]] = gi.chr_lens[i];
+    std::map<std::string, std::vector<std::pair<uint64_t, uint64_t>>> regions;
+    if (regions_bed) {
+        int code = GSX_OK;
+        if (!read_bed(regions_bed, chr_len, regions, code, err)) return gsx_set_error(code, err);
+    }
+    const int have = gsx_device_count();
+    if (have <= 0) return gsx_set_error(GSX_ERR_NO_DEVICE, "no CUDA device available (this library has no CPU path)");
+    if (device >= have) return gsx_set_error(GSX_ERR_ARG, "device " + std::to_string(device) + " is out of range (" + std::to_string(have) + " device(s))");
+
+    OutFile out;
+    if (!out.open(out_path)) return gsx_set_error(GSX_ERR_IO, std::string("cannot write ") + out_path);
+    {
+        std::string h = csv_header(complete != 0);
+        if (with_cfd) { h.pop_back(); h += ",cfd\n"; }
+        if (!out.append(std::vector<std::string>(1, h))) { out.close_file(); return gsx_set_error(GSX_ERR_IO, std::string("cannot write ") + out_path); }
+    }
+    const char* eb = getenv("GSX_DECODE_BATCH_BYTES");                                      // (tests: batches of a few records)
+    const size_t batch_bytes = eb && *eb && atoll(eb) > 0 ? (size_t)atoll(eb) : ((size_t)128 << 20);
+    const bool timing = getenv("GSX_FILE_TIMING") != nullptr;
+    auto now = [] { return std::chrono::steady_clock::now(); };
+    auto since = [](std::chrono::steady_clock::time_point t) { return std::chrono::duration<double>(std::chrono::steady_clock::now() - t).count(); };
+    const auto t_job = now();
+    double s_upload = 0, s_read = 0, s_device = 0, ms_device = 0, s_format = 0, s_write = 0;
+    size_t n_batches = 0, guides = 0, rows = 0, sam_bytes = 0;
+
+    // reader (this thread) -> device (this thread) -> formatter -> writer; at most two batches wait between two stages
+    std::mutex mu; std::condition_variable cv;
+    std::deque<std::unique_ptr<DecodeBatch>> fqueue, spare; std::deque<std::vector<std::string>> wqueue;
+    bool rdone = false, fdone = false, failed = false; int wrc = GSX_OK;
+    std::atomic<bool> format_nomem{false};
+    std::thread writer([&] {
+        for (;;) {
+            std::vector<std::string> parts;
+            { std::unique_lock<std::mutex> lk(mu); cv.wait(lk, [&] { return !wqueue.empty() || fdone; }); if (wqueue.empty()) return; parts = std::move(wqueue.front()); }
+            const auto tw = now();
+            if (wrc == GSX_OK && !out.append(parts)) wrc = GSX_ERR_IO;
+            s_write += since(tw);
+            for (std::string& p : parts) string_pool().put(std::move(p));
+            { std::lock_guard<std::mutex> lk(mu); wqueue.pop_front(); }
+            cv.notify_all();
+        }
+    });
+    std::thread formatter([&] {
+        const unsigned hw = std::max(1u, std::thread::hardware_concurrency());
+        for (;;) {
+            std::unique_ptr<DecodeBatch> b; bool skip;
+            {
+                std::unique_lock<std::mutex> lk(mu);
+                cv.wait(lk, [&] { return !fqueue.empty() || rdone; });
+                if (fqueue.empty()) break;
+                b = std::move(fqueue.front()); fqueue.pop_front(); skip = failed;
+            }
+            cv.notify_all();
+            if (skip) { std::lock_guard<std::mutex> lk(mu); spare.push_back(std::move(b)); continue; }
+            const auto tf = now();
+            // slices of about equal numbers of rows, cut at records
+            const size_t nr = b->recs.size(), total = b->rows.n_rows;
+            const unsigned nt = (unsigned)std::max<size_t>(1, std::min<size_t>({(size_t)hw, nr, total / 32768 + 1}));
+            std::vector<size_t> cut(nt + 1, nr); cut[0] = 0;
+            for (unsigned t = 1; t < nt; t++) cut[t] = (size_t)(std::lower_bound(b->rows.rec_row, b->rows.rec_row + nr, (uint32_t)(total * t / nt)) - b->rows.rec_row);
+            std::vector<std::string> parts(nt);
+            auto work = [&](unsigned t) {
+                parts[t] = string_pool().get();
+                const size_t a = std::min(cut[t], nr), e = std::max(a, std::min(cut[t + 1], nr));
+                parts[t].reserve((size_t)(b->rows.rec_row[e] - b->rows.rec_row[a]) * 120);
+                try { format_decoded(*b, a, e, gi.chr_names, complete != 0, with_cfd != 0, parts[t]); }
+                catch (const std::bad_alloc&) { format_nomem = true; parts[t].clear(); }
+            };
+            if (nt == 1) work(0);
+            else { std::vector<std::thread> th; for (unsigned t = 0; t < nt; t++) th.emplace_back(work, t); for (auto& x : th) x.join(); }
+            s_format += since(tf);
+            std::unique_lock<std::mutex> lk(mu);
+            spare.push_back(std::move(b));
+            cv.wait(lk, [&] { return wqueue.size() < 2; });
+            wqueue.push_back(std::move(parts));
+            lk.unlock(); cv.notify_all();
+        }
+        { std::lock_guard<std::mutex> lk(mu); fdone = true; }
+        cv.notify_all();
+    });
+
+    int rc = GSX_OK; std::string rc_msg;
+    try {
+        const auto tu = now();
+        std::vector<gsx::Chrom> chroms; uint64_t start = 0;
+        for (uint64_t l : gi.chr_lens) { chroms.push_back({start, l}); start += l; }
+        gsx::DecodeDevice dev(device, genome.data(), gi.genome_length, chroms, pams);
+        s_upload = since(tu);
+        SamReader reader(in);
+        DecodeSplitter splitter{pam_length, regions_bed ? &regions : nullptr};
+        for (;;) {
+            std::unique_ptr<DecodeBatch> b;
+            {
+                std::unique_lock<std::mutex> lk(mu);
+                cv.wait(lk, [&] { return fqueue.size() < 2; });
+                if (!spare.empty()) { b = std::move(spare.front()); spare.pop_front(); }
+            }
+            if (!b) b.reset(new DecodeBatch());
+            const auto tr = now();
+            if (!reader.next(batch_bytes, *b)) break;
+            splitter.split(*b);
+            s_read += since(tr);
+            sam_bytes += b->len;
+            if (b->recs.empty()) { std::lock_guard<std::mutex> lk(mu); spare.push_back(std::move(b)); continue; }      // (keeps its pinned text)
+            const auto td = now();
+            dev.run({b->text, b->len, b->rec_hex.data(), b->rec_entry.data(), b->guides.data(), (uint32_t)b->recs.size()}, b->rows);
+            s_device += since(td); ms_device += b->rows.ms; n_batches++;
+            if (b->rows.err_code) {
+                const gsx::DecodeRows& R = b->rows;
+                const size_t r = (size_t)(std::upper_bound(b->rec_entry.begin(), b->rec_entry.end(), R.err_entry) - b->rec_entry.begin()) - 1;
+                const DecodeRec& c = b->recs[r];
+                const std::string rec = "record " + quoted(c.id, c.id_len) + " at byte " + std::to_string(c.at);
+                const uint32_t t = R.err_entry - b->rec_entry[r];
+                std::string what;
+                if (R.err_code == gsx::kDecodeBadHex) what = "value " + std::to_string(t) + " of its of:H: list is not 16 hex digits";
+                else if (R.err_code == gsx::kDecodeBadGroup) what = "its of:H: list is not a run of groups [positions] d " + std::to_string(delim) + " for d = 0, 1, ... (at value " + std::to_string(t) + ")";
+                else {
+                    const int64_t abs = R.err_value; const gsx::DecodeGuide& g = b->guides[r];
+                    uint32_t pos1 = 0; uint8_t sc = '+';
+                    const int chr = gsx::resolve_abs(chroms.data(), (uint32_t)chroms.size(), abs, g.qlen, g.plen, &pos1, &sc);
+                    const std::string site = "off-target " + std::to_string(abs) + (chr >= 0 ? " (" + gi.chr_names[chr] + ":" + std::to_string(pos1) + ":" + (char)sc + ")" : "");
+                    if (R.err_code == gsx::kDecodeOutside) what = site + " does not lie inside one chromosome of the genome";
+                    else if (R.err_code == gsx::kDecodeDistance)
+                        what = site + " has " + std::to_string(R.err_found) + " mismatches to the guide but is listed at distance " + std::to_string(R.err_listed) + ": the database was written with bulges, or "
+                               "on another genome";
+                    else what = site + " carries neither the guide's PAM column nor an alternative PAM: the database was written with bulges, with other PAMs (-a), or "
+                           "on another genome";
+                }
+                throw decode_error(rec + ": " + what);
+            }
+            guides += b->recs.size(); rows += b->rows.n_rows;
+            {
+                std::lock_guard<std::mutex> lk(mu);
+                fqueue.push_back(std::move(b));
+            }
+            cv.notify_all();
+        }
+    } catch (const gsx::SiteError& f) { rc = f.code; rc_msg = f.msg; }
+    catch (const std::bad_alloc&) { rc = GSX_ERR_NOMEM; rc_msg = "out of host memory"; }
+    catch (const std::exception& x) { rc = GSX_ERR_INTERNAL; rc_msg = std::string("decode: ") + x.what(); }
+    { std::lock_guard<std::mutex> lk(mu); rdone = true; failed = rc != GSX_OK; }
+    cv.notify_all();
+    formatter.join(); writer.join();
+    if (timing)
+        fprintf(stderr, "gsx decode: %.3f s wall, %zu SAM bytes, %zu guides decoded, %zu rows, %zu batch(es); FASTA read %.3f s (before the wall); genome upload %.3f s; read/split %.3f s; "
+                "device %.3f s (events %.3f ms, %.3f ms per batch); format %.3f s; write %.3f s\n",
+                since(t_job), sam_bytes, guides, rows, n_batches, s_fasta, s_upload, s_read, s_device, ms_device, n_batches ? ms_device / n_batches : 0.0, s_format, s_write);
+    if (!out.close_file() && wrc == GSX_OK) wrc = GSX_ERR_IO;
+    if (rc) return gsx_set_error(rc, rc_msg);
+    if (format_nomem) return gsx_set_error(GSX_ERR_NOMEM, "out of host memory formatting the rows");
+    if (wrc) return gsx_set_error(wrc, std::string("cannot write ") + out_path);
+    if (n_guides) *n_guides = guides;
+    if (n_rows) *n_rows = rows;
+    return GSX_OK;
 }

@@ -62,7 +62,7 @@ EXPORTS = ["gsx_params_default", "gsx_index_open", "gsx_index_build", "gsx_index
            "gsx_index_n_chromosomes", "gsx_index_chromosome_name", "gsx_index_chromosome_length", "gsx_index_device_bytes",
            "gsx_index_n_devices", "gsx_index_save_reference_format", "gsx_index_open_seconds", "gsx_index_device_checksum", "gsx_enumerate_start", "gsx_enumerate_wait", "gsx_index_rank", "gsx_index_locate", "gsx_index_export_bwt", "gsx_index_export_sa_samples", "gsx_enumerate", "gsx_result_view_get",
            "gsx_result_counters", "gsx_result_match_sequence", "gsx_result_free", "gsx_format_rows", "gsx_format_header",
-           "gsx_enumerate_file", "gsx_guides_csv_open", "gsx_guides_csv_row", "gsx_guides_csv_close", "gsx_generate_kmers", "gsx_enumerate_genome", "gsx_free", "gsx_last_error", "gsx_version", "gsx_device_count"]
+           "gsx_enumerate_file", "gsx_guides_csv_open", "gsx_guides_csv_row", "gsx_guides_csv_close", "gsx_generate_kmers", "gsx_enumerate_genome", "gsx_decode_database", "gsx_free", "gsx_last_error", "gsx_version", "gsx_device_count"]
 
 _L.gsx_last_error.restype = C.c_char_p
 _L.gsx_version.restype = C.c_char_p
@@ -111,6 +111,9 @@ _L.gsx_generate_kmers.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, C.c_uint32
 _L.gsx_enumerate_genome.argtypes = [C.c_void_p, C.c_char_p, C.c_char_p, C.c_uint32, C.c_uint64, C.c_char_p, C.c_char_p, C.c_char_p,
                                     C.POINTER(Params), C.c_int, C.c_int, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(Counters)]
 
+_L.gsx_decode_database.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, C.c_uint32, C.POINTER(C.c_char_p), C.c_uint32, C.c_int, C.c_int,
+                                   C.c_char_p, C.c_int, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]
+
 
 class GsxError(RuntimeError):
     def __init__(self, code, where):
@@ -133,6 +136,17 @@ def generate_kmers(fasta: str, out_csv: str, pam="NGG", kmer_length=20, min_chr_
     _ck(_L.gsx_generate_kmers(fasta.encode(), out_csv.encode(), pam.encode(), kmer_length, min_chr_length, prefix.encode(),
                               int(bool(start)), device, C.byref(n)), "gsx_generate_kmers")
     return n.value
+
+
+def decode_database(sam: str, fasta: str, out: str, pam_length=3, alt_pams=(), mode="complete", cfd=False, regions=None, device=0):
+    """The off-targets of a SAM complete database (`enumerate --format sam --mode complete`) back as enumerate's CSV rows, sites and
+    CFD from `fasta` on the GPU (include/gsx.h gsx_decode_database).  Returns (guides decoded, rows written)."""
+    arr = (C.c_char_p * max(1, len(alt_pams)))(*[a.encode() for a in alt_pams])
+    ng, nr = C.c_size_t(), C.c_size_t()
+    _ck(_L.gsx_decode_database(sam.encode(), fasta.encode(), out.encode(), pam_length, arr, len(alt_pams), int(mode == "complete"),
+                               int(bool(cfd)), regions.encode() if regions else None, device, C.byref(ng), C.byref(nr)),
+        "gsx_decode_database")
+    return ng.value, nr.value
 
 
 def make_params(mismatches=3, rna_bulges=0, dna_bulges=0, threshold=-1, start=False, max_off_targets=-1,

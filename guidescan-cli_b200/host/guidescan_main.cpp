@@ -53,7 +53,18 @@ static void usage() {
             "      --min-chr-length UINT=0     Skip FASTA records shorter than this.\n"
             "      --prefix TEXT               Prefix of every k-mer id.\n"
             "      --start                     The PAM precedes the k-mer.\n"
-            "      --device INT=0              GPU that runs the scan.\n");
+            "      --device INT=0              GPU that runs the scan.\n"
+            "  decode [OPTIONS] DATABASE.sam\n"
+            "      Turns the of:H: off-target lists of a database written with --format sam --mode complete back into enumerate's\n"
+            "      CSV rows (the original's scripts/decode_database.py; sites and CFD computed on the GPU).\n"
+            "      --genome GENOME.fa          REQUIRED  The assembly the database was computed on.\n"
+            "      -o,--output FILE            REQUIRED  Output CSV.\n"
+            "      --mode TEXT:{succinct,complete}  Columns, as enumerate's (default complete).\n"
+            "      --cfd                       Append a cfd column.\n"
+            "      --pam-length UINT=3         Characters of the PAM column at the end of each sequence.\n"
+            "      -a,--alt-pam TEXT ...       Alternative PAMs the database was written with.\n"
+            "      --regions BED               Only guides whose on-target site lies inside one BED interval (0-based, half-open).\n"
+            "      --device INT=0              GPU that decodes.\n");
 }
 
 static std::string lower(std::string s) { std::transform(s.begin(), s.end(), s.begin(), ::tolower); return s; }
@@ -101,6 +112,42 @@ static int do_kmers(int argc, char** argv) {
         fprintf(stderr, "ERROR: %s\n", gsx_last_error()); return 1;
     }
     printf("Wrote %llu kmer(s) to %s in %.3f s.\n", (unsigned long long)n, output.c_str(), std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count());
+    return 0;
+}
+
+static int do_decode(int argc, char** argv) {
+    std::string sam, genome, output, mode = "complete", regions;
+    std::vector<std::string> alts; unsigned long long pam_length = 3, device = 0; bool cfd = false;
+    for (int i = 0; i < argc; i++) {
+        std::string a = argv[i];
+        auto need = [&](const char* name) -> const char* { if (i + 1 >= argc) { fprintf(stderr, "%s: 1 required\n", name); exit(106); } return argv[++i]; };
+        if (a == "-o" || a == "--output") output = need("--output");
+        else if (a == "--genome") genome = need("--genome");
+        else if (a == "--mode") mode = lower(need("--mode"));
+        else if (a == "--cfd") cfd = true;
+        else if (a == "--pam-length") pam_length = uint_arg("--pam-length", need("--pam-length"));
+        else if (a == "-a" || a == "--alt-pam") { while (i + 1 < argc && argv[i + 1][0] != '-') alts.push_back(argv[++i]); }
+        else if (a == "--regions") regions = need("--regions");
+        else if (a == "--device") device = uint_arg("--device", need("--device"));
+        else if (a == "-h" || a == "--help") { usage(); return 0; }
+        else if (!a.empty() && a[0] == '-') { fprintf(stderr, "The following argument was not expected: %s\n", a.c_str()); return 109; }
+        else sam = a;
+    }
+    if (sam.empty()) { fprintf(stderr, "database is required\n"); return 106; }
+    if (genome.empty()) { fprintf(stderr, "--genome is required\n"); return 106; }
+    if (output.empty()) { fprintf(stderr, "--output is required\n"); return 106; }
+    if (mode != "succinct" && mode != "complete") { fprintf(stderr, "--mode: %s not in {succinct,complete}\n", mode.c_str()); return 105; }
+    if (pam_length < 1 || pam_length > 8) { fprintf(stderr, "--pam-length: %llu not in 1..8\n", pam_length); return 105; }
+    for (auto& x : alts)
+        if (!pam_ok(x) || x.size() != pam_length) { fprintf(stderr, "--alt-pam: %s must be %llu characters of A, C, G, T, N\n", x.c_str(), pam_length); return 105; }
+    std::vector<const char*> ap; for (auto& s : alts) ap.push_back(s.c_str());
+    size_t ng = 0, nr = 0;
+    const auto t0 = std::chrono::steady_clock::now();
+    if (gsx_decode_database(sam.c_str(), genome.c_str(), output.c_str(), (uint32_t)pam_length, ap.data(), (uint32_t)ap.size(), mode == "complete", cfd,
+                            regions.empty() ? nullptr : regions.c_str(), (int)device, &ng, &nr)) {
+        fprintf(stderr, "ERROR: %s\n", gsx_last_error()); return 1;
+    }
+    printf("Decoded %zu guide(s) into %zu row(s) in %s in %.3f s.\n", ng, nr, output.c_str(), std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count());
     return 0;
 }
 
@@ -213,6 +260,7 @@ int main(int argc, char** argv) {
     if (cmd == "index") return do_index(argc - 2, argv + 2);
     if (cmd == "enumerate") return do_enumerate(argc - 2, argv + 2);
     if (cmd == "kmers") return do_kmers(argc - 2, argv + 2);
+    if (cmd == "decode") return do_decode(argc - 2, argv + 2);
     if (cmd == "download") { fprintf(stderr, "download: not part of the GPU hot path (no network); use the reference binary\n"); return 1; }
     usage();
     return 106;

@@ -218,6 +218,24 @@ int gsx_enumerate_genome(const gsx_index*, const char* fasta_path, const char* p
                          const char* prefix, const char* regions_bed, const char* out_path, const gsx_params*, int format_sam,
                          int complete, size_t batch_guides, size_t* n_guides, gsx_counters* counters);
 
+/* ---- SAM database decode ------------------------------------------------------------------------------ */
+/* The off-targets of a database written by `enumerate --format sam --mode complete` (this library's or the original's), back as
+ * rows: what scripts/decode_database.py of the original does, as the CSV that enumerate writes.  Per record: QNAME = guide id, SEQ
+ * (reverse-complemented back when FLAG has 16) = protospacer + PAM column (its last pam_length characters), sp:f: = specificity
+ * (copied as text); every position of the of:H: list becomes one row with its chromosome, position and strand (resolve_absolute),
+ * the listed distance and the site's text from the genome, in record and list order.  Consecutive records of one QNAME are one guide:
+ * the first is decoded, the others must carry the same list.  Each site is checked against its list: its mismatches to the guide
+ * must be the listed distance, its PAM the guide's PAM column or one of alt_pams (of the column's length; N matches anything) --
+ * a database written with bulges, with other PAMs or on another assembly fails with GSX_ERR_ARG naming the record and the site.
+ * `fasta_path` is the assembly the database was computed on (its records must equal the SAM's @SQ lines); no index is needed.
+ * complete: the columns of --mode complete (bulge columns 0), else succinct; with_cfd != 0 appends a `cfd` column (%.9g of the
+ * float32 CFD the search computes).  regions_bed != NULL: only the records whose on-target site (RNAME:POS, len(SEQ) bases) lies
+ * inside one BED interval.  Options, header, FASTA and BED are checked before any device work.  Runs on `device`; host memory holds
+ * the genome and the batches in flight.  *n_guides = guides decoded, *n_rows = rows written (both may be NULL). */
+int gsx_decode_database(const char* sam_path, const char* fasta_path, const char* out_path, uint32_t pam_length,
+                        const char* const* alt_pams, uint32_t n_alt_pams, int complete, int with_cfd, const char* regions_bed,
+                        int device, size_t* n_guides, size_t* n_rows);
+
 void gsx_free(void*);
 
 const char* gsx_last_error(void);
