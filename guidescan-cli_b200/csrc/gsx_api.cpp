@@ -3,6 +3,7 @@
 #include "../../include/gsx.h"
 #include "gsx_host.h"
 #include "gsx_core.h"
+#include "gsx_iupac.h"
 #include <cuda_runtime.h>
 #include <algorithm>
 #include <chrono>
@@ -555,8 +556,13 @@ int gsx_prepare_guides(const gsx_guide* guides, size_t n, const gsx_params* p, g
                     if (s.size() > (size_t)kMaxPamLen) return fail(GSX_ERR_ARG, "alternative PAM longer than 8");
                     if (s.empty() && pams.size() > 1) return fail(GSX_ERR_ARG, "empty alternative PAM");
                     ps.plen[k] = (uint8_t)s.size();
-                    for (size_t j = 0; j < s.size(); j++)
-                        ps.sym[k][j] = p->start ? sym_of(s[s.size() - 1 - j]) : sym_of(complement_char(s[j]));
+                    for (size_t j = 0; j < s.size(); j++) {
+                        // under iupac_pams a class letter is one character of code SYM_CLS with its members in cmask (complemented in
+                        // the default orientation: iupac_complement, not complement_char, which keeps the reference's parity)
+                        const char c = p->start ? s[s.size() - 1 - j] : s[j];
+                        if (p->iupac_pams && iupac_is_class(c)) { ps.sym[k][j] = SYM_CLS; ps.cmask[k][j] = (uint8_t)iupac_mask(p->start ? c : iupac_complement(c)); }
+                        else ps.sym[k][j] = p->start ? sym_of(c) : sym_of(complement_char(c));
+                    }
                     set_mp[id] = std::max(set_mp[id], s.size());
                 }
                 out.max_pams = std::max<uint32_t>(out.max_pams, ps.n_pams);
@@ -620,10 +626,13 @@ int gsx_prepare_guides(const gsx_guide* guides, size_t n, const gsx_params* p, g
         const PamSet& ps = out.pamsets[0];
         out.n_fast_pams = ps.n_pams;
         for (uint32_t k = 0; k < ps.n_pams; k++) {
-            out.plens[k] = ps.plen[k]; out.pampacks[k] = 0;
-            for (uint32_t j = 0; j < ps.plen[k]; j++) out.pampacks[k] |= (uint32_t)ps.sym[k][j] << (3 * j);
+            out.plens[k] = ps.plen[k]; out.pampacks[k] = 0; out.pammasks[k] = 0;
+            for (uint32_t j = 0; j < ps.plen[k]; j++) {
+                out.pampacks[k] |= (uint32_t)ps.sym[k][j] << (3 * j);
+                out.pammasks[k] |= (uint32_t)ps.cmask[k][j] << (4 * j);
+            }
         }
-        out.plen = out.plens[0]; out.pampack = out.pampacks[0];
+        out.plen = out.plens[0]; out.pampack = out.pampacks[0]; out.pammask = out.pammasks[0];
     }
     return GSX_OK;
 }
@@ -706,7 +715,7 @@ SearchPlan gsx::plan_search(const Prepared& prep, const gsx_params& p, const Ind
     // characters, at most 3 mismatches, an index without N, no --start, no threshold pass, and a jump table deep enough to hold
     // both capped halves (13 characters: the PAM and the proximal half of the PAM-first form; with fewer, that form would hand the
     // tree search alignments with two proximal mismatches only for the re-anchoring to drop them).  Per guide and strand a quarter
-    // of the summary sectors of the plain sweep.
+    // of the summary sectors of the plain sweep.  A class PAM character (code 6) is not concrete, so class PAMs keep the plain sweep.
     pl.split = pl.search_sb != 0 && !pl.use_variants && p.threshold <= 0 && !p.start && prep.n_fast_pams == 1 && prep.plen == 3 &&
                (prep.pampack & 7u) == 4u && ((prep.pampack >> 3) & 7u) < 4u && ((prep.pampack >> 6) & 7u) < 4u &&
                prep.min_qlen == 2 * kSplitHalf && prep.max_qlen == 2 * kSplitHalf && p.mismatches <= kSplitMaxM && ix.plain &&
@@ -743,7 +752,12 @@ SearchPlan gsx::plan_search(const Prepared& prep, const gsx_params& p, const Ind
         double pam_frac = 0;
         for (int ps = 0; ps < kMaxPamSets; ps++) {
             double f = 0;
-            for (int k = 0; k < prep.pamsets[ps].n_pams; k++) { double g1 = 1; for (int j = 0; j < prep.pamsets[ps].plen[k]; j++) if (prep.pamsets[ps].sym[k][j] != SYM_N) g1 *= 0.25; f += g1; }
+            const PamSet& P = prep.pamsets[ps];
+            for (int k = 0; k < P.n_pams; k++) {
+                double g1 = 1;                                                // a class character passes |class| / 4 of the sites
+                for (int j = 0; j < P.plen[k]; j++) g1 *= P.sym[k][j] == SYM_CLS ? 0.25 * popc64(P.cmask[k][j]) : P.sym[k][j] != SYM_N ? 0.25 : 1.0;
+                f += g1;
+            }
             pam_frac = std::max(pam_frac, std::min(1.0, f));
         }
         const double expect = 2.0 * (double)ix.rows * patterns / std::pow(4.0, ql) * pam_frac;
@@ -908,7 +922,7 @@ struct DeviceRun {
             uint64_t* d_gq = B.alloc<uint64_t>(n);
             CK(cudaMemcpyAsync(d_gq, prep.gq.data() + job.g0, (size_t)n * 8, cudaMemcpyHostToDevice, s));
             if (plan.late_guides) job.ctr.ms_h2d += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_h2d0).count();
-            a.gq = d_gq; a.pampack = prep.pampack; a.plen = prep.plen;
+            a.gq = d_gq; a.pampack = prep.pampack; a.pammask = prep.pammask; a.plen = prep.plen;
             a.exc = plan.exc ? 1u : 0u; a.exc_map[0] = (const uint32_t*)di.st[0].exc_map; a.exc_map[1] = (const uint32_t*)di.st[1].exc_map;
             a.pin_width = plan.pin_width; a.combos = nullptr; a.n_combos = 0;
         }
@@ -1092,13 +1106,13 @@ struct DeviceRun {
         m.n_fused = 0;
         if (plan.fuse_pams && !m.p.counting) {
             m.n_fused = prep.n_fast_pams;
-            for (uint32_t k = 0; k < prep.n_fast_pams; k++) m.fused_pams[k] = prep.pampacks[k];
-            m.plen = prep.plens[0]; m.pampack = fused_filter_pampack(prep.pampacks, prep.n_fast_pams, prep.plens[0]);
+            for (uint32_t k = 0; k < prep.n_fast_pams; k++) { m.fused_pams[k] = prep.pampacks[k]; m.fused_masks[k] = prep.pammasks[k]; }
+            m.plen = prep.plens[0]; m.pampack = fused_filter_pampack(prep.pampacks, prep.n_fast_pams, prep.plens[0], prep.pammasks, &m.pammask);
             launch_fast(m, ng, sb, ev_mid);
             return;
         }
         for (uint32_t k = 0; k < prep.n_fast_pams; k++) {
-            m.pampack = prep.pampacks[k]; m.plen = prep.plens[k];
+            m.pampack = prep.pampacks[k]; m.pammask = prep.pammasks[k]; m.plen = prep.plens[k];
             if (k) { CK(cudaMemsetAsync(d_ctrs, 0, 4, s)); CK(cudaMemsetAsync(d_ctrs + 3, 0, 8, s)); }      // task / seed-queue / work-unit counters
             launch_fast(m, ng, sb, k == 0 ? ev_mid : nullptr);
         }

@@ -150,7 +150,8 @@ GSX_HD bool make_child(int cand, const Node& nd, const ExpandCtx& cx, const uint
             if (j >= cx.ps->plen[pam]) return false;
             uint32_t pc = cx.ps->sym[pam][j];
             if (cand == CAND_LITN) { if (pc != SYM_N) return false; }
-            else if (!(pc == s || pc == SYM_N)) return false;                       // index.hpp:151-168 with mismatches = 0
+            else if (!(pc == s || pc == SYM_N || (pc == SYM_CLS && ((cx.ps->cmask[pam][j] >> s) & 1u)))) return false;   // index.hpp:151-168 with mismatches = 0
+                                                                                    // (a class: its members only, never a literal N)
             digit = WIDE ? wide_upper_digit(s) : (s < 3 ? s : (s == 3 ? 4u : 3u));
         }
         uint32_t o_s, o_e;
@@ -446,7 +447,9 @@ GSX_HD void guide_specificity(const SpecArgs& a, uint32_t g) {
 // character matched.  A child whose bit is clear can never reach the final level, so it is not expanded: the set of
 // emitted matches is unchanged.  Planes hold arbitrary symbols where the true one is not A/C/G/T or lies before the
 // text start; that can only set bits spuriously (no pruning), never clear one that should be set, because such a
-// path cannot be continued by an A/C/G/T query character in the first place.
+// path cannot be continued by an A/C/G/T query character in the first place.  A class PAM character (code 6) counts as a wildcard
+// here: its members always survive, a non-member is only pruned later (the child itself is tested against the class), so the mask
+// stays a superset of the exact one at no extra registers on the tree search's hot loop.
 GSX_HD uint32_t viable_children(const uint64_t hi[7], const uint64_t lo[7], uint32_t sp, uint32_t ep, uint32_t lvl,
                                 uint32_t qlen, uint32_t total, uint64_t q, uint32_t pampack, uint32_t budget) {
     const uint32_t r0 = sp & 63u, r1 = ep & 63u;
@@ -461,7 +464,7 @@ GSX_HD uint32_t viable_children(const uint64_t hi[7], const uint64_t lo[7], uint
             const uint32_t L = lvl + j;
             uint32_t sym; bool proto = L < qlen, wild = false, kill = false;
             if (proto) sym = (uint32_t)(q >> (2u * L)) & 3u;
-            else { uint32_t pc = (pampack >> (3u * (L - qlen))) & 7u; sym = pc & 3u; wild = pc == 4u; kill = pc > 4u; }
+            else { uint32_t pc = (pampack >> (3u * (L - qlen))) & 7u; sym = pc & 3u; wild = pc == 4u || pc == 6u; kill = pc == 5u || pc == 7u; }
             const uint64_t eq = ~(hi[j] ^ ((sym & 2u) ? ~0ull : 0ull)) & ~(lo[j] ^ ((sym & 1u) ? ~0ull : 0ull));
             if (proto) {
                 const uint64_t mis = ~eq;
@@ -484,7 +487,9 @@ GSX_HD uint32_t viable_children(const uint64_t hi[7], const uint64_t lo[7], uint
 // like the jump table) -- the next seven characters of every row of the interval as bit planes -- and tests all rows at once.
 //   codes: per guide, 4 bits per plane j = 0..6 of what a row must show at level L + j: 0..3 = that symbol in the
 //          protospacer (anything else costs one mismatch), 8..11 = that symbol in the PAM (anything else kills the row),
-//          12 = PAM wildcard, 13 = kills every row, 7 = no such level.
+//          12 = PAM wildcard, 13 = kills every row, 7 = no such level.  A class PAM character (pampack code 6) is a wildcard here:
+//          the sweep only chooses seeds and the tree search behind it tests the class exactly, so this keeps a superset of the
+//          seeds and the compiled plane layouts (shape 0 covers NRG, NNGRRT and --start TTTV at 20 nt).
 //   u[r]:  rows with at most budget - r mismatches so far (r = 0 .. NB-1, NB > budget); u[0] = rows still alive.
 //   One 32-byte sector holds all seven levels for 16 rows (sum0: rows 0..15 of the interval, sum1: rows 16..31), so a single
 //          load settles nine nodes out of ten; lanes whose node has more than 16 rows and found nothing among the first 16
@@ -496,7 +501,7 @@ GSX_HD uint32_t sweep_codes(uint64_t q, uint32_t L, uint32_t plen, uint32_t pamp
         const uint32_t Lv = L + j;
         uint32_t c;
         if (Lv < qlen) c = (uint32_t)(q >> (2u * Lv)) & 3u;
-        else if (Lv < qlen + plen) { c = (pampack >> (3u * (Lv - qlen))) & 7u; if (c > 4u) c = 5u; c |= 8u; }     // bit 3: PAM level
+        else if (Lv < qlen + plen) { c = (pampack >> (3u * (Lv - qlen))) & 7u; c = c == 6u ? 4u : c > 4u ? 5u : c; c |= 8u; }     // bit 3: PAM level
         else c = 7u;
         codes |= c << (4u * j);
     }
@@ -510,7 +515,7 @@ GSX_HD uint32_t sweep_codes2(uint64_t q, uint32_t L, uint32_t plen, uint32_t pam
         const uint32_t Lv = L + 7u + j;
         uint32_t c;
         if (Lv < qlen) c = (uint32_t)(q >> (2u * Lv)) & 3u;
-        else if (Lv < qlen + plen) { c = (pampack >> (3u * (Lv - qlen))) & 7u; if (c > 4u) c = 5u; c |= 8u; }
+        else if (Lv < qlen + plen) { c = (pampack >> (3u * (Lv - qlen))) & 7u; c = c == 6u ? 4u : c > 4u ? 5u : c; c |= 8u; }
         else c = 7u;
         codes |= c << (4u * j);
     }
@@ -878,26 +883,34 @@ GSX_HD void split_classes(uint32_t form, uint32_t L, uint32_t qlen, uint32_t ple
 // common character where all PAMs agree, the wildcard where they differ -- and keep a finished alignment only if the PAM
 // characters it consumed spell one of the real PAMs.  (Counting passes keep one pass per PAM: the reference's threshold
 // counter counts a site once per PAM it satisfies.)
-//   packs[k]: 3 bits per PAM character in consumption order (0..3 symbol, 4 = N wildcard, 5 = never matches); equal lengths
-GSX_HD uint32_t fused_filter_pampack(const uint32_t* packs, uint32_t n, uint32_t plen) {
-    uint32_t out = 0;
+//   packs[k]: 3 bits per PAM character in consumption order (0..3 symbol, 4 = N wildcard, 5 = never matches, 6 = class); equal
+//   lengths.  masks[k] (nullptr: no class anywhere): 4 bits per character, the members of a class character.  Two classes at one
+//   position are the same character only with the same members (NRG + NYG filter on the wildcard); *out_mask = the filter's masks.
+GSX_HD uint32_t fused_filter_pampack(const uint32_t* packs, uint32_t n, uint32_t plen, const uint32_t* masks = nullptr,
+                                     uint32_t* out_mask = nullptr) {
+    uint32_t out = 0, omask = 0;
     for (uint32_t j = 0; j < plen; j++) {
-        const uint32_t c0 = (packs[0] >> (3u * j)) & 7u;
+        const uint32_t c0 = (packs[0] >> (3u * j)) & 7u, m0 = masks ? (masks[0] >> (4u * j)) & 15u : 0u;
         bool same = true;
-        for (uint32_t k = 1; k < n; k++) same = same && (((packs[k] >> (3u * j)) & 7u) == c0);
+        for (uint32_t k = 1; k < n; k++) same = same && (((packs[k] >> (3u * j)) & 7u) == c0) && (!masks || ((masks[k] >> (4u * j)) & 15u) == m0);
         out |= (same ? c0 : 4u) << (3u * j);
+        if (same) omask |= m0 << (4u * j);
     }
+    if (out_mask) *out_mask = omask;
     return out;
 }
 // key: narrow string key whose last plen digits are the consumed PAM characters (A,C,G,N,T = 0..4, gsx_core.h key_append)
-GSX_HD bool fused_pam_ok(uint64_t key, uint32_t plen, const uint32_t* packs, uint32_t n) {
+// (masks as in fused_filter_pampack: a class character accepts the digits of its members, never N's)
+GSX_HD bool fused_pam_ok(uint64_t key, uint32_t plen, const uint32_t* packs, uint32_t n, const uint32_t* masks = nullptr) {
     uint32_t dg[kMaxPamLen];
     for (uint32_t j = plen; j-- > 0;) { dg[j] = (uint32_t)(key % 5ull); key /= 5ull; }
     for (uint32_t k = 0; k < n; k++) {
         bool ok = true;
         for (uint32_t j = 0; j < plen; j++) {
             const uint32_t pc = (packs[k] >> (3u * j)) & 7u;
-            ok = ok && (pc == 4u || (pc < 4u && dg[j] == (pc < 3u ? pc : 4u)));
+            const uint32_t cm = (pc == 6u && masks) ? (masks[k] >> (4u * j)) & 15u : 0u;
+            const uint32_t sbit = dg[j] == 3u ? 0u : 1u << (dg[j] < 3u ? dg[j] : 3u);       // digit A,C,G,N,T -> member bit (N: none)
+            ok = ok && (pc == 4u || (pc < 4u && dg[j] == (pc < 3u ? pc : 4u)) || (cm & sbit) != 0u);
         }
         if (ok) return true;
     }

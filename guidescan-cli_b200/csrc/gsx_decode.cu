@@ -9,6 +9,7 @@
 #include "../../include/gsx.h"
 #include "gsx_core.h"
 #include "gsx_decode.h"
+#include "gsx_iupac.h"
 #include "gsx_host.h"
 #include "gsx_sites.h"
 #include "cfd_tables.h"
@@ -67,8 +68,9 @@ __global__ void decode_hex_kernel(const unsigned char* __restrict__ text, const 
     }
 }
 
+// N accepts any site character, a class letter (R, Y, ..., V) its member bases, any other letter itself (gsx_iupac.h)
 __device__ __forceinline__ bool pam_fits(const char* pam, const char* site, uint32_t plen) {
-    for (uint32_t i = 0; i < plen; i++) if (pam[i] != 'N' && pam[i] != site[i]) return false;
+    for (uint32_t i = 0; i < plen; i++) if (!iupac_pam_fits(pam[i], site[i])) return false;
     return true;
 }
 

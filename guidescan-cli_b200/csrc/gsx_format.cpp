@@ -6,6 +6,7 @@
 #include "gsx_core.h"
 #include "gsx_sites.h"
 #include "gsx_decode.h"
+#include "gsx_iupac.h"
 #include <algorithm>
 #include <atomic>
 #include <cstdio>
@@ -51,6 +52,10 @@ inline char* put_hex_le64_at(char* w, uint64_t v) {
     return w + 16;
 }
 std::string revcomp(const std::string& x) { std::string r(x.size(), 'N'); for (size_t i = 0; i < x.size(); i++) r[i] = complement_char(x[x.size() - 1 - i]); return r; }
+// complement of a SAM SEQ character: IUPAC class letters to their partners (R<->Y, K<->M, B<->V, D<->H; S, W kept), as
+// Bio.Seq.reverse_complement does; every other character as complement_char
+static char seq_complement(char c) { return iupac_is_class(c) ? iupac_complement(c) : complement_char(c); }
+static std::string seq_revcomp(const std::string& x) { std::string r(x.size(), 'N'); for (size_t i = 0; i < x.size(); i++) r[i] = seq_complement(x[x.size() - 1 - i]); return r; }
 
 // The results of a call lie in one part per device (gsx_host.h HostArrays), each with its own guide and hit numbering.  The
 // formatter reads the parts in place: the merged arrays of the public view are only built when a caller asks for them
@@ -172,7 +177,7 @@ void format_sam_guide(const gsx_index* ix, const gsx_result* r, const gsx_guide_
     for (uint64_t h = b; h < b + n && P.distance[h] == 0; h++) n0++;
     if (!n0) return;                                                                         // rows exist only for 0-mismatch alignments
     std::string sequence = p->start ? std::string(row.pam) + row.seq : std::string(row.seq) + row.pam;
-    std::string seq_out = row.sense_positive ? sequence : revcomp(sequence);
+    std::string seq_out = row.sense_positive ? sequence : seq_revcomp(sequence);
     const uint32_t* cbd = P.cbd + at.gl * n_dist;
     // the row up to the of:H: list, and behind it; the list itself (off_target_fields, printer.hpp:115-170) is written straight into
     // the output buffer: 16 hex digits per counted hit plus a (distance, delimiter) pair per distance -- kilobytes per guide at m = 4
@@ -812,9 +817,14 @@ extern "C" int gsx_enumerate_genome(const gsx_index* ix, const char* fasta_path,
     const std::string pam(pam_c), prefix(prefix_c ? prefix_c : "");
     if (k < 1 || k > 32) return gsx_set_error(GSX_ERR_ARG, "kmer_length " + std::to_string(k) + " is outside 1..32");
     if (pam.empty() || pam.size() > 8) return gsx_set_error(GSX_ERR_ARG, "PAM \"" + pam + "\" must have 1..8 characters");
-    for (char c : pam)
-        if (!(c == 'A' || c == 'C' || c == 'G' || c == 'T' || c == 'N'))
-            return gsx_set_error(GSX_ERR_ARG, "PAM \"" + pam + "\" has the character '" + std::string(1, c) + "': PAM characters must be A, C, G, T or N");
+    for (char c : pam) {
+        if (!iupac_pam_char(c))
+            return gsx_set_error(GSX_ERR_ARG, "PAM \"" + pam + "\" has the character '" + std::string(1, c) +
+                                                  "': PAM characters must be A, C, G, T, N or an IUPAC class letter (R, Y, S, W, K, M, B, D, H, V)");
+        // the generated guides carry the pattern as their PAM column: without class semantics they could never match
+        if (iupac_is_class(c) && !p->iupac_pams)
+            return gsx_set_error(GSX_ERR_ARG, "PAM \"" + pam + "\" has the class letter '" + std::string(1, c) + "': it needs iupac_pams (--iupac-pam)");
+    }
     std::string longest = pam;
     for (uint32_t i = 0; i < p->n_alt_pams; i++) if (p->alt_pams && p->alt_pams[i] && strlen(p->alt_pams[i]) > longest.size()) longest = p->alt_pams[i];
     if (k + longest.size() + p->dna_bulges > 32)
@@ -992,7 +1002,7 @@ struct DecodeSplitter {
             if (!selected(F, L)) continue;
             gsx::DecodeGuide g{};
             const char* s = F.f[9];
-            for (uint32_t i = 0; i < L; i++) g.seq[i] = (flag & 16) ? complement_char(s[L - 1 - i]) : s[i];
+            for (uint32_t i = 0; i < L; i++) g.seq[i] = (flag & 16) ? seq_complement(s[L - 1 - i]) : s[i];
             g.qlen = (uint8_t)(L - pam_len); g.plen = (uint8_t)pam_len;
             b.recs.push_back({F.f[0], F.sp, F.n[0], (uint32_t)F.sp_len, (uint32_t)b.seqs.size(), L, where});
             b.seqs.append(g.seq, L);
@@ -1054,8 +1064,9 @@ extern "C" int gsx_decode_database(const char* sam_path, const char* fasta_path,
         const std::string a = alt_pams[i] ? alt_pams[i] : "";
         if (a.size() != pam_length) return gsx_set_error(GSX_ERR_ARG, "alternative PAM \"" + a + "\" has " + std::to_string(a.size()) + " characters, the PAM column " + std::to_string(pam_length));
         for (char c : a)
-            if (!(c == 'A' || c == 'C' || c == 'G' || c == 'T' || c == 'N'))
-                return gsx_set_error(GSX_ERR_ARG, "alternative PAM \"" + a + "\" has the character '" + std::string(1, c) + "': PAM characters must be A, C, G, T or N");
+            if (!iupac_pam_char(c))
+                return gsx_set_error(GSX_ERR_ARG, "alternative PAM \"" + a + "\" has the character '" + std::string(1, c) +
+                                                      "': PAM characters must be A, C, G, T, N or an IUPAC class letter (R, Y, S, W, K, M, B, D, H, V)");
         memcpy(pams.p[i], a.data(), a.size());
     }
     if (device < 0) return gsx_set_error(GSX_ERR_ARG, "device " + std::to_string(device) + " is not a device ordinal");

@@ -132,6 +132,7 @@ struct Prepared {
     std::vector<uint64_t> gq;      // per guide: 2-bit symbols in consumption order | qlen << 58
     uint32_t pampack = 0, plen = 0, min_qlen = 0;      // (first PAM of the list)
     uint32_t n_fast_pams = 0, pampacks[kMaxPams] = {0}, plens[kMaxPams] = {0};      // every PAM of the (single) PAM set: one search pass each
+    uint32_t pammask = 0, pammasks[kMaxPams] = {0};    // members of the class characters of pampack / pampacks (0: A/C/G/T/N only)
     // bulges on the specialised kernels: every guide is replaced by its edited guides (gsx_core.h variant_rewrite); valid when
     // the batch would be a fast-path batch without its bulges and the edited guides are few enough
     bool variant_ok = false;

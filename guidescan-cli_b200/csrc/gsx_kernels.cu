@@ -641,11 +641,13 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) search_fast_kernel(SearchArg
         // ---- children (branch-free) ---------------------------------------------------------------------------
         const bool in_proto = lvl < qlen;
         const uint32_t c = in_proto ? ((uint32_t)(q >> (2u * lvl)) & 3u) : ((a.pampack >> (3u * (lvl - qlen))) & 7u);
-        const bool allow = in_proto ? (mm < M) : (c == 4u);
+        // symbols other than c that may be consumed: all four within the mismatch budget or under a PAM wildcard, the members of a
+        // class PAM character (code 6, whose members are in pammask), none otherwise
+        const uint32_t allow = in_proto ? (mm < M ? 15u : 0u) : (c == 4u ? 15u : ((a.pammask >> (4u * (lvl - qlen))) & 15u));
         const bool final_lvl = (lvl + 1u == qlen + plen);
         const uint32_t w0 = oe0 - os0, w1 = oe1 - os1, w2 = oe2 - os2, w3 = oe3 - os3;
-        bool v0 = has && w0 && (c == 0u || allow), v1 = has && w1 && (c == 1u || allow);
-        bool v2 = has && w2 && (c == 2u || allow), v3 = has && w3 && (c == 3u || allow);
+        bool v0 = has && w0 && (c == 0u || (allow & 1u)), v1 = has && w1 && (c == 1u || (allow & 2u));
+        bool v2 = has && w2 && (c == 2u || (allow & 4u)), v3 = has && w3 && (c == 3u || (allow & 8u));
         if (LOOK && narrow) {        // drop children that cannot survive the next (up to) seven characters
             v0 = v0 && (vm & 1u); v1 = v1 && (vm & 2u); v2 = v2 && (vm & 4u); v3 = v3 && (vm & 8u);
         }
@@ -662,7 +664,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) search_fast_kernel(SearchArg
         if (__any_sync(FULL, final_lvl && (v0 || v1 || v2 || v3))) {
 #define GSX_EMIT(s)                                                                                                   \
             {                                                                                                         \
-                const bool e = final_lvl && v##s && (!FUSED || fused_pam_ok(key5 + GSX_CH_DIGIT(s), plen, a.fused_pams, a.n_fused)); \
+                const bool e = final_lvl && v##s && (!FUSED || fused_pam_ok(key5 + GSX_CH_DIGIT(s), plen, a.fused_pams, a.n_fused, a.fused_masks)); \
                 const uint32_t emask = __ballot_sync(FULL, e);                                                         \
                 if (emask) {                                                                                          \
                     if (a.p.counting) {                                                                               \
@@ -700,7 +702,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) search_fast_kernel(SearchArg
                 }
                 const bool vN = litn && wN != 0u;
                 const uint32_t spN = (s1 ? a.st[1].C[4] : a.st[0].C[4]) + o_s;
-                const bool eN = vN && final_lvl && (!FUSED || fused_pam_ok(key5 + 3u, plen, a.fused_pams, a.n_fused));
+                const bool eN = vN && final_lvl && (!FUSED || fused_pam_ok(key5 + 3u, plen, a.fused_pams, a.n_fused, a.fused_masks));
                 const uint32_t emask = __ballot_sync(FULL, eN);
                 if (emask) {
                     if (a.p.counting) { if (eN) atomicAdd(a.guide_count + ((tlm & 0xFFFFFFu) >> 1), (unsigned long long)wN); }

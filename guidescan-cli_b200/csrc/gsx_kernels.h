@@ -35,7 +35,7 @@ struct SearchArgs {
     uint32_t max_pams;
     // fast path only (search_fast_kernel): one PAM for all guides, ACGT-only guides, sentinel-only exception tables
     const uint64_t* gq;                // per guide: 2-bit symbol codes in consumption order | qlen << 58
-    uint32_t pampack;                  // 3 bits per PAM character in consumption order (4 = N wildcard, 5 = never matches)
+    uint32_t pampack;                  // 3 bits per PAM character in consumption order (4 = N wildcard, 5 = never matches, 6 = class)
     uint32_t plen;
     uint32_t pin_width;                // packed-block loads of intervals at least this wide ask L2 to keep the line (evict_last)
     const uint64_t* combos;            // k-mer jump table enumeration: substitution combos over characters 2 .. ftab_L - 1
@@ -55,6 +55,10 @@ struct SearchArgs {
     // edited guides (bulges): per guide, the must-match positions as an index mask (gsx_core.h variant_forced_mask); the sweep
     // skips the patterns that substitute them; nullptr = off
     const uint32_t* fmask;
+    // IUPAC class characters (code 6 of pampack / fused_pams): 4 bits per PAM character, the members (A=1, C=2, G=4, T=8) of a class
+    // character and 0 for every other one -- all zero for an A/C/G/T/N PAM list
+    uint32_t pammask;
+    uint32_t fused_masks[kMaxPams];
 };
 
 constexpr int kSweepXtabShared = 4352;          // words of shared memory the sweep kernels keep for the xor table (17 KB)

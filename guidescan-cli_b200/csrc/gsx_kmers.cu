@@ -7,7 +7,8 @@
 // Semantics restated (not copied) from the script:
 //   * chromosome = first word of the FASTA header; sequence upper-cased; records shorter than min_chr_length are skipped
 //   * the PAM pattern's N's are expanded one at a time, first N first, in the order A,C,T,G, breadth first -- e.g. NGG gives
-//     AGG, CGG, TGG, GGG (generate_kmers.py:55-68); the "-" strand uses the reverse complements of the same list
+//     AGG, CGG, TGG, GGG (generate_kmers.py:55-68); the "-" strand uses the reverse complements of the same list.  IUPAC class
+//     letters (R, Y, ..., V) expand the same way into their members, in the same order (NRG: AAG, AGG, CAG, CGG, TAG, ...)
 //   * for each concrete PAM, every (overlapping) occurrence i: PAM at the end (default): "+" k-mer = chr[i-k, i), position
 //     i-k; "-" k-mer = revcomp(chr[i+|pam|, i+|pam|+k)), position i.  PAM at the start (--start): "+" k-mer =
 //     chr[i+|pam|, i+|pam|+k), position i; "-" k-mer = revcomp(chr[i-k, i)), position i-k (generate_kmers.py:70-100)
@@ -17,6 +18,7 @@
 #include "../../include/gsx.h"
 #include "gsx_host.h"
 #include "gsx_sites.h"
+#include "gsx_iupac.h"
 #include <cub/cub.cuh>
 #include <thrust/iterator/counting_iterator.h>
 #include <cuda_runtime.h>
@@ -63,17 +65,8 @@ __global__ void upper_kernel(unsigned char* s, uint32_t len) {
 
 #define KCK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) throw gsx::SiteError{GSX_ERR_CUDA, std::string(#x ": ") + cudaGetErrorString(e_)}; } while (0)
 
-std::vector<std::string> expand_pam(const std::string& pam) {
-    std::deque<std::string> q{pam};
-    auto any_n = [&]() { for (auto& s : q) if (s.find('N') != std::string::npos) return true; return false; };
-    while (any_n()) {
-        std::string s = q.front(); q.pop_front();
-        const size_t at = s.find('N');
-        if (at == std::string::npos) { q.push_back(s); continue; }
-        for (char c : {'A', 'C', 'T', 'G'}) { std::string t = s; t[at] = c; q.push_back(t); }
-    }
-    return std::vector<std::string>(q.begin(), q.end());
-}
+// (IUPAC class letters expand into their members the same way: gsx_iupac.h)
+std::vector<std::string> expand_pam(const std::string& pam) { return gsx::iupac_expand(pam); }
 
 struct DeviceScratch {
     unsigned char* chr = nullptr; unsigned char* flags = nullptr; uint32_t* pos = nullptr; uint32_t* count = nullptr; void* tmp = nullptr;
@@ -207,7 +200,7 @@ extern "C" int gsx_generate_kmers(const char* fasta_path, const char* out_csv_pa
     if (!fasta_path || !out_csv_path || !pam_c) return gsx_set_error(GSX_ERR_ARG, "null argument");
     const std::string pam(pam_c), prefix(prefix_c ? prefix_c : "");
     if (pam.empty() || pam.size() > 8 || k == 0 || k > 64) return gsx_set_error(GSX_ERR_ARG, "PAM must have 1..8 characters and the k-mer 1..64");
-    for (char c : pam) if (!(c == 'A' || c == 'C' || c == 'G' || c == 'T' || c == 'N')) return gsx_set_error(GSX_ERR_ARG, "PAM characters must be A, C, G, T or N");
+    for (char c : pam) if (!gsx::iupac_pam_char(c)) return gsx_set_error(GSX_ERR_ARG, "PAM characters must be A, C, G, T, N or an IUPAC class letter (R, Y, S, W, K, M, B, D, H, V)");
     int have = 0;
     if (cudaGetDeviceCount(&have) != cudaSuccess || have <= 0) return gsx_set_error(GSX_ERR_NO_DEVICE, "no CUDA device available (this library has no CPU path)");
     if (device < 0 || device >= have) return gsx_set_error(GSX_ERR_ARG, "device ordinal out of range");

@@ -33,8 +33,9 @@ constexpr int kMaxPams = 8;        // alt PAMs + the guide's own
 constexpr int kMaxPamSets = 16;    // distinct (pam column value) groups per call
 constexpr int kMaxDist = 8;        // mismatches <= 7
 
-// symbol codes: 0..3 = A,C,G,T ; 4 = N ; 5 = anything else (never matches)
-enum : uint8_t { SYM_A = 0, SYM_C = 1, SYM_G = 2, SYM_T = 3, SYM_N = 4, SYM_X = 5 };
+// symbol codes: 0..3 = A,C,G,T ; 4 = N ; 5 = anything else (never matches) ; 6 = an IUPAC class letter of a PAM (R, Y, ..., V:
+// gsx_iupac.h), whose members come from a parallel mask (PamSet::cmask, the pammask words of the kernels)
+enum : uint8_t { SYM_A = 0, SYM_C = 1, SYM_G = 2, SYM_T = 3, SYM_N = 4, SYM_X = 5, SYM_CLS = 6 };
 
 struct alignas(32) OccBlock {
     uint32_t cnt[4];   // occurrences of A,C,G,T in BWT[0, 64*b)
@@ -88,6 +89,7 @@ struct PamSet {
     uint8_t sym[kMaxPams][kMaxPamLen];   // consumption order; SYM_N = wildcard
     uint8_t kpam_len;                    // length of the guide's own pam column (coordinates use it: structures.cxx:36,41)
     uint8_t pad[6];
+    uint8_t cmask[kMaxPams][kMaxPamLen]; // members of a SYM_CLS character (A=1, C=2, G=4, T=8); 0 for every other character
 };
 
 struct SearchParams {

@@ -27,7 +27,7 @@ class Params(C.Structure):
     _fields_ = [("mismatches", C.c_uint32), ("rna_bulges", C.c_uint32), ("dna_bulges", C.c_uint32),
                 ("max_bulge_size", C.c_uint32), ("threshold", C.c_int32), ("start", C.c_uint32),
                 ("max_off_targets", C.c_int64), ("alt_pams", C.POINTER(C.c_char_p)), ("n_alt_pams", C.c_uint32),
-                ("sam_scoring", C.c_uint32)]
+                ("sam_scoring", C.c_uint32), ("iupac_pams", C.c_uint32)]
 
 
 class ResultView(C.Structure):
@@ -150,7 +150,9 @@ def decode_database(sam: str, fasta: str, out: str, pam_length=3, alt_pams=(), m
 
 
 def make_params(mismatches=3, rna_bulges=0, dna_bulges=0, threshold=-1, start=False, max_off_targets=-1,
-                alt_pams=(), sam_scoring=False):
+                alt_pams=(), sam_scoring=False, iupac_pams=False):
+    """iupac_pams: read the guides' PAM column and alt_pams with IUPAC class letters (R, Y, S, W, K, M, B, D, H, V), each matching
+    its member bases and never a genome N; off, any letter but A, C, G, T, N never matches."""
     p = Params()
     _L.gsx_params_default(C.byref(p))
     p.mismatches, p.rna_bulges, p.dna_bulges = mismatches, rna_bulges, dna_bulges
@@ -159,6 +161,7 @@ def make_params(mismatches=3, rna_bulges=0, dna_bulges=0, threshold=-1, start=Fa
     p.alt_pams = C.cast(arr, C.POINTER(C.c_char_p))
     p.n_alt_pams = len(alt_pams)
     p.sam_scoring = int(bool(sam_scoring))
+    p.iupac_pams = int(bool(iupac_pams))
     p._keep = arr
     return p
 

@@ -26,6 +26,9 @@ static void usage() {
             "      --max-off-targets INT=-1    Maximum number of off-targets to store for each number of mismatches.\n"
             "      -n,--threads UINT           Host worker threads that format the output (default: all cores); the search runs on the GPU(s).\n"
             "      -a,--alt-pam TEXT ...       Alternative PAMs used to find off-targets\n"
+            "      --iupac-pam                 Read the kmers file's PAM column and -a with IUPAC class letters (R, Y, S, W, K, M,\n"
+            "                                  B, D, H, V: a class matches its member bases, never a genome N); without it any\n"
+            "                                  letter but A, C, G, T, N never matches (extension; set by itself for a --pam with one).\n"
             "      -m,--mismatches UINT=3      Number of mismatches to allow when finding off-targets\n"
             "      --rna-bulges UINT=0         Max number of RNA bulges to allow when finding off-targets\n"
             "      --dna-bulges UINT=0         Number of DNA bulges to allow when finding off-targets\n"
@@ -39,7 +42,7 @@ static void usage() {
             "      --devices LIST              The same with explicit device ordinals, e.g. 0,2,3 (extension).\n"
             "      --genome GENOME.fa          Generate the guides from this FASTA (as `kmers` does, PAM position from --start) and\n"
             "                                  enumerate them in one pass, without a kmers file (extension).  With --genome:\n"
-            "        --pam TEXT=NGG            PAM pattern (A, C, G, T, N).\n"
+            "        --pam TEXT=NGG            PAM pattern (A, C, G, T, N and IUPAC class letters, e.g. NRG, NNGRRT, TTTV).\n"
             "        --kmer-length UINT=20     Guide length, 1..32 (with the PAM and DNA bulges at most 32).\n"
             "        --min-chr-length UINT=0   Skip FASTA records shorter than this.\n"
             "        --prefix TEXT             Prefix of every guide id.\n"
@@ -48,7 +51,7 @@ static void usage() {
             "      Writes the kmers file `enumerate -f` reads: every k-mer next to a PAM on either strand (the original's\n"
             "      scripts/generate_kmers.py; the PAM scan runs on the GPU).\n"
             "      -o,--output FILE            REQUIRED  Output CSV.\n"
-            "      --pam TEXT=NGG              PAM pattern (A, C, G, T, N).\n"
+            "      --pam TEXT=NGG              PAM pattern (A, C, G, T, N and IUPAC class letters, expanded like N).\n"
             "      --kmer-length UINT=20       Length of the k-mers.\n"
             "      --min-chr-length UINT=0     Skip FASTA records shorter than this.\n"
             "      --prefix TEXT               Prefix of every k-mer id.\n"
@@ -62,7 +65,7 @@ static void usage() {
             "      --mode TEXT:{succinct,complete}  Columns, as enumerate's (default complete).\n"
             "      --cfd                       Append a cfd column.\n"
             "      --pam-length UINT=3         Characters of the PAM column at the end of each sequence.\n"
-            "      -a,--alt-pam TEXT ...       Alternative PAMs the database was written with.\n"
+            "      -a,--alt-pam TEXT ...       Alternative PAMs the database was written with (IUPAC class letters allowed).\n"
             "      --regions BED               Only guides whose on-target site lies inside one BED interval (0-based, half-open).\n"
             "      --device INT=0              GPU that decodes.\n");
 }
@@ -78,12 +81,14 @@ static unsigned long long uint_arg(const char* name, const char* v) {
     return x;
 }
 
-// PAM characters of the generator (scripts/generate_kmers.py expands N only)
+// PAM characters of the generator and the decoder: A, C, G, T, N and the upper-case IUPAC class letters
+static bool is_class(char c) { return c && strchr("RYSWKMBDHV", c) != nullptr; }
 static bool pam_ok(const std::string& pam) {
     if (pam.empty() || pam.size() > 8) return false;
-    for (char c : pam) if (!(c == 'A' || c == 'C' || c == 'G' || c == 'T' || c == 'N')) return false;
+    for (char c : pam) if (!(c == 'A' || c == 'C' || c == 'G' || c == 'T' || c == 'N' || is_class(c))) return false;
     return true;
 }
+static const char* kPamLetters = "A, C, G, T, N or IUPAC class letters (R, Y, S, W, K, M, B, D, H, V)";
 
 static int do_kmers(int argc, char** argv) {
     std::string fasta, output, pam = "NGG", prefix;
@@ -105,7 +110,7 @@ static int do_kmers(int argc, char** argv) {
     if (fasta.empty()) { fprintf(stderr, "genome is required\n"); return 106; }
     if (output.empty()) { fprintf(stderr, "--output is required\n"); return 106; }
     if (k < 1 || k > 64) { fprintf(stderr, "--kmer-length: %llu not in 1..64\n", k); return 105; }
-    if (!pam_ok(pam)) { fprintf(stderr, "--pam: %s must be 1..8 characters of A, C, G, T, N\n", pam.c_str()); return 105; }
+    if (!pam_ok(pam)) { fprintf(stderr, "--pam: %s must be 1..8 characters of %s\n", pam.c_str(), kPamLetters); return 105; }
     uint64_t n = 0;
     const auto t0 = std::chrono::steady_clock::now();
     if (gsx_generate_kmers(fasta.c_str(), output.c_str(), pam.c_str(), (uint32_t)k, min_len, prefix.c_str(), start, (int)device, &n)) {
@@ -139,7 +144,7 @@ static int do_decode(int argc, char** argv) {
     if (mode != "succinct" && mode != "complete") { fprintf(stderr, "--mode: %s not in {succinct,complete}\n", mode.c_str()); return 105; }
     if (pam_length < 1 || pam_length > 8) { fprintf(stderr, "--pam-length: %llu not in 1..8\n", pam_length); return 105; }
     for (auto& x : alts)
-        if (!pam_ok(x) || x.size() != pam_length) { fprintf(stderr, "--alt-pam: %s must be %llu characters of A, C, G, T, N\n", x.c_str(), pam_length); return 105; }
+        if (!pam_ok(x) || x.size() != pam_length) { fprintf(stderr, "--alt-pam: %s must be %llu characters of %s\n", x.c_str(), pam_length, kPamLetters); return 105; }
     std::vector<const char*> ap; for (auto& s : alts) ap.push_back(s.c_str());
     size_t ng = 0, nr = 0;
     const auto t0 = std::chrono::steady_clock::now();
@@ -186,6 +191,7 @@ static int do_enumerate(int argc, char** argv) {
         std::string a = argv[i];
         auto need = [&](const char* name) -> const char* { if (i + 1 >= argc) { fprintf(stderr, "%s: 1 required\n", name); exit(106); } return argv[++i]; };
         if (a == "--start") p.start = 1;
+        else if (a == "--iupac-pam") p.iupac_pams = 1;
         else if (a == "--max-off-targets") p.max_off_targets = atoll(need("--max-off-targets"));
         else if (a == "-n" || a == "--threads") { const int t = atoi(need("--threads")); if (t > 0) setenv("GSX_FORMAT_THREADS", std::to_string(t).c_str(), 1); }
         else if (a == "-a" || a == "--alt-pam") {          // greedy multi-value, as CLI11 parses it (SURVEY.md App. E.7)
@@ -223,7 +229,8 @@ static int do_enumerate(int argc, char** argv) {
     if (mode != "succinct" && mode != "complete") { fprintf(stderr, "--mode: %s not in {succinct,complete}\n", mode.c_str()); return 105; }
     if (!genome.empty()) {                                    // (the library checks these too; here they fail before the index is opened)
         if (k < 1 || k > 32) { fprintf(stderr, "--kmer-length: %llu not in 1..32\n", k); return 105; }
-        if (!pam_ok(pam)) { fprintf(stderr, "--pam: %s must be 1..8 characters of A, C, G, T, N\n", pam.c_str()); return 105; }
+        if (!pam_ok(pam)) { fprintf(stderr, "--pam: %s must be 1..8 characters of %s\n", pam.c_str(), kPamLetters); return 105; }
+        for (char c : pam) if (is_class(c)) p.iupac_pams = 1;      // the generated guides carry the pattern as their PAM column
         size_t longest = pam.size(); for (auto& x : alts) longest = std::max(longest, x.size());
         if (k + longest + p.dna_bulges > 32) { fprintf(stderr, "--kmer-length %llu + PAM %zu + --dna-bulges %u is longer than 32\n", k, longest, p.dna_bulges); return 105; }
     }

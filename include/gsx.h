@@ -56,6 +56,9 @@ typedef struct {
     const char* const* alt_pams;  /* -a */
     uint32_t n_alt_pams;
     uint32_t sam_scoring;         /* 0: specificity by the CSV rule (printer.hpp:244-300); 1: by the SAM rule (printer.hpp:115-170) */
+    uint32_t iupac_pams;          /* --iupac-pam: read the pam column and alt_pams with IUPAC class letters (R, Y, S, W, K, M, B, D, H, V):
+                                     a class matches its member bases, never a genome N.  0 (default): any letter but A, C, G, T, N never
+                                     matches, as before.  (Appended field: callers built against the earlier, shorter struct must be rebuilt.) */
 } gsx_params;
 
 void gsx_params_default(gsx_params* p);
