@@ -674,6 +674,30 @@ GSX_HD void summary_eval_masks(const uint32_t w[8], const uint32_t gm[15], uint3
         }
     }
 }
+// The same for guides whose seven planes are all protospacer levels or wildcards / absent levels (no concrete PAM character among them:
+// sweep_shape_of 0 or 1): every plane is stepped as a protospacer level.  A wildcard plane has A = X = 0, so every row matches it and
+// the step u[r] = u[r] | u[r+1] leaves the nested masks (u[r+1] within u[r]) as they are.  No per-plane flag: about half the
+// instructions of summary_eval_masks.  Equal to it for every such guide (tests/sweep_proto_check.cpp).
+template <int NB>
+GSX_HD void summary_eval_proto(const uint32_t w[8], const uint32_t gm[15], uint32_t budget, uint32_t u[NB]) {
+    const uint32_t valid = w[0] & 0xFFFFu;
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for (int r = 0; r < NB; r++) u[r] = budget >= (uint32_t)r ? valid : 0u;
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for (uint32_t j = 0; j < 7u; j++) {
+        const uint32_t y = (w[1u + j] & gm[j]) ^ gm[7u + j];
+        const uint32_t eq = ~(y | (y >> 16));
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+        for (int r = 0; r + 1 < NB; r++) u[r] = (u[r] & eq) | u[r + 1];
+        u[NB - 1] &= eq;
+    }
+}
 
 // levels L + 7 and L + 8 for the rows that survived the first seven: t = sum2[e] = {hi7, lo7, hi8, lo8} over rows 0..31,
 // half = which 16 of them the masks u[] describe

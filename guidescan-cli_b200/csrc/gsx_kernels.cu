@@ -1173,8 +1173,9 @@ __device__ __forceinline__ void lean_settle(const SweepArgs& a, ParkBuf& pk, uin
     lean_park(pk, lane, park, idx | (budget << 28), tl);
 }
 // one pattern of one guide -- its row of the guide table, any plane layout -- against one summary sector: rows still alive after
-// the seven planes and, where the guide has them, the two levels behind (sum2).  EXACT: no budget left.
-template <int NBX, bool EXACT>
+// the seven planes and, where the guide has them, the two levels behind (sum2).  EXACT: no budget left.  PROTO: the guide's planes
+// are all protospacer levels or wildcards (gsx_core.h summary_eval_proto).
+template <int NBX, bool EXACT, bool PROTO = false>
 __device__ __forceinline__ uint32_t lean_row_eval(const uint32_t* __restrict__ row, const unsigned char* sum, const unsigned char* sum2, uint32_t idx,
                                                   uint32_t budget, uint32_t half, bool live, uint32_t& w0) {
     const uint4* gp = reinterpret_cast<const uint4*>(row);
@@ -1191,7 +1192,7 @@ __device__ __forceinline__ uint32_t lean_row_eval(const uint32_t* __restrict__ r
         return v[0];
     }
     uint32_t u[NBX];
-    summary_eval_masks<NBX>(w, gm, budget, u);
+    if (PROTO) summary_eval_proto<NBX>(w, gm, budget, u); else summary_eval_masks<NBX>(w, gm, budget, u);
     if (u[0] && tail) { uint32_t t[4]; load_tail(sum2, idx, t); summary_tail<NBX>(t, half, codes2, u); }
     return u[0];
 }
@@ -1443,7 +1444,7 @@ __device__ __forceinline__ void split_emit(const SweepArgs& a, uint32_t lane, bo
     }
 }
 // up to 32 parked nodes of either form: rows 16..31 of their intervals (as lean_drain)
-template <int NB>
+template <int NB, bool PROTO>
 __device__ __forceinline__ void split_drain(const SweepArgs& a, ParkBuf& pk, uint32_t lane, LeanStats& st) {
     const uint32_t n = pk.count < 32u ? pk.count : 32u;
     const bool mine = lane < n;
@@ -1454,14 +1455,16 @@ __device__ __forceinline__ void split_drain(const SweepArgs& a, ParkBuf& pk, uin
     const uint32_t idx = word & 0x0FFFFFFFu, budget = word >> 28, row = tl >> 1;
     const bool s1 = (tl & 1u) != 0u, form1 = row >= a.n_guides;
     uint32_t alive = 0, w0;
-    if (mine) alive = lean_row_eval<NB, false>(a.gtab + (size_t)row * GT_WORDS, s1 ? a.st[1].sum1 : a.st[0].sum1, s1 ? a.st[1].sum2 : a.st[0].sum2,
-                                               idx, budget, 1u, true, w0);
+    if (mine) alive = lean_row_eval<NB, false, PROTO>(a.gtab + (size_t)row * GT_WORDS, s1 ? a.st[1].sum1 : a.st[0].sum1,
+                                                      s1 ? a.st[1].sum2 : a.st[0].sum2, idx, budget, 1u, true, w0);
     const uint32_t g = row - (form1 ? a.n_guides : 0u);
     split_emit(a, lane, alive != 0u, form1, idx, ((g << 1) | (tl & 1u)) | ((a.M - budget) << 24) | (budget << 27),
                reinterpret_cast<const FtabEntry*>(s1 ? a.st[1].ftab : a.st[0].ftab));
 }
 
-template <int WARPS, int MINB, int NB>
+// PROTO: the rows of both forms have only protospacer and wildcard planes (20-nt guides at jump-table depth 13 or 14): judged with
+// summary_eval_proto, half the instructions of the general filter
+template <int WARPS, int MINB, int NB, bool PROTO>
 __global__ void __launch_bounds__(WARPS * 32, MINB) sweep_split_kernel(SweepArgs a) {
     __shared__ SplitPlan s_sp;
     __shared__ uint32_t s_park[WARPS][2][PK_SLOTS];
@@ -1518,7 +1521,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) sweep_split_kernel(SweepArgs
         const FtabEntry* tab = reinterpret_cast<const FtabEntry*>(strand ? a.st[1].ftab : a.st[0].ftab);
         const uint32_t hi_bits = beta << low;
         for (uint32_t f0 = 0; f0 < total; f0 += 32u) {
-            while (pk.count >= 32u) split_drain<NB>(a, pk, lane, st);
+            while (pk.count >= 32u) split_drain<NB, PROTO>(a, pk, lane, st);
             const uint32_t fi = f0 + lane;
             const bool live = fi < total;
             uint32_t k = 0;                                                           // the lane whose list holds pattern fi: last k with off[k] <= fi
@@ -1536,7 +1539,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) sweep_split_kernel(SweepArgs
             const uint32_t budget = live ? (lw >> 16) - (xw >> 28) : 0u;
             st.lines += __popc(__ballot_sync(FULL, live && (xw & 15u) == 0u));
             uint32_t w0;
-            const uint32_t alive = lean_row_eval<NB, false>(rowp, sum0, sum2, idx, budget, 0u, live, w0);
+            const uint32_t alive = lean_row_eval<NB, false, PROTO>(rowp, sum0, sum2, idx, budget, 0u, live, w0);
             // (w0 == 0 for lanes without a pattern and for empty table entries; the flags are only ever set on non-empty ones)
             const bool emit = (alive | (w0 & SUM_WIDE32)) != 0u;                     // (more than 32 rows: not summarised, the tree search takes it)
             const bool park = !emit && (w0 & SUM_WIDE16) != 0u;
@@ -1546,7 +1549,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) sweep_split_kernel(SweepArgs
             lean_park(pk, lane, park, idx | (budget << 28), (row << 1) | strand);
         }
     }
-    while (pk.count) split_drain<NB>(a, pk, lane, st);
+    while (pk.count) split_drain<NB, PROTO>(a, pk, lane, st);
     unsigned long long n_nodes = st.nodes, n_two = st.two;
     for (int o = 16; o; o >>= 1) { n_nodes += __shfl_xor_sync(FULL, n_nodes, o); n_two += __shfl_xor_sync(FULL, n_two, o); }
     if (lane == 0) { atomicAdd(a.stats + 0, n_nodes); atomicAdd(a.stats + 1, n_nodes + n_two + st.lines); atomicAdd(a.stats + 5, (unsigned long long)st.sectors); }
@@ -1602,13 +1605,18 @@ cudaError_t launch_split_queries(const uint64_t* gq, uint32_t n, uint32_t pampac
 cudaError_t launch_sweep_split(const SweepArgs& a, int ctas_per_sm, int sm_count, cudaStream_t s) {
     if (a.M > kSplitMaxM || a.n_xtab > (uint32_t)kSplitXtabShared) return cudaErrorInvalidValue;
     const dim3 block(8 * 32);
+    // both forms' plane layouts (20-nt guides; form 1 reads all 23 characters as protospacer): protospacer and wildcard planes only?
+    const int shape0 = sweep_shape_of(sweep_codes((uint64_t)20 << 58, a.plan.L, a.plen, a.pampack));
+    const int shape1 = sweep_shape_of(sweep_codes((uint64_t)(20 + a.plen) << 58, a.plan.L, 0, 0));
+    const bool proto = (shape0 == 0 || shape0 == 1) && (shape1 == 0 || shape1 == 1);
+#define GSX_SPLIT_LAUNCH(C)                                                                                      \
+    case C: if (proto) sweep_split_kernel<8, C, 4, true><<<sm_count * C, block, 0, s>>>(a);                   \
+            else sweep_split_kernel<8, C, 4, false><<<sm_count * C, block, 0, s>>>(a); break;
     switch (ctas_per_sm) {
-    case 4: sweep_split_kernel<8, 4, 4><<<sm_count * 4, block, 0, s>>>(a); break;
-    case 5: sweep_split_kernel<8, 5, 4><<<sm_count * 5, block, 0, s>>>(a); break;
-    case 6: sweep_split_kernel<8, 6, 4><<<sm_count * 6, block, 0, s>>>(a); break;
-    case 8: sweep_split_kernel<8, 8, 4><<<sm_count * 8, block, 0, s>>>(a); break;
+    GSX_SPLIT_LAUNCH(4) GSX_SPLIT_LAUNCH(5) GSX_SPLIT_LAUNCH(6) GSX_SPLIT_LAUNCH(8)
     default: return cudaErrorInvalidValue;
     }
+#undef GSX_SPLIT_LAUNCH
     return cudaGetLastError();
 }
 cudaError_t launch_reanchor(const ReanchorArgs& r, cudaStream_t s) {
